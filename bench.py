@@ -2,7 +2,7 @@
 """
 bench.py -- measures the FP8 hot path on B200 and prints ONE JSON line (rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-sub] [--no-cpu]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-sub] [--no-cpu] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline at every N (BASELINE.json `metric` names "_scaled_mm TFLOPS" first; configs[3], "C4", is the config that
@@ -33,6 +33,11 @@ sweeps) and the un-patched torch._scaled_mm (cuBLASLt FP8) time on C4 as a libra
 
 --impl reference: the reference's CPU implementation of the same workload (oracle port, all host threads), same
 `config`, same JSON shape with "impl": "reference".
+
+--dump-outputs DIR (N = 1): after the timed steps, the results of the last step -- the C of each of the SETS calls --
+are written as DIR/c4_out_set<i>.npy, float32, restricted to a fixed set of DUMP_ROWS rows (every column of those
+rows; see dump_outputs).  The inputs come from fixed seeds, so two builds run with the same arguments can be
+compared output for output.
 """
 
 from __future__ import annotations
@@ -47,6 +52,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True             # the benchmark writes nothing into the tree it runs from (it may be read-only)
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "fp8-mps-metal_b200")
 for _p in (PKG, os.path.join(ROOT, "tests")):
@@ -69,6 +75,7 @@ SQ_BYTES = 14336 * 14336 + 14336 + 2 * 14336 + 8
 ROTATION = 16
 PASSES = 8
 SETS = 4                                   # C4 rotation: 4 x (12.6 + 37.7 + 100.7) MB > 126 MB L2
+DUMP_ROWS = 128                            # --dump-outputs: 128 of 4096 rows of each C, 4 x 6.3 MB of float32
 NVLINK_GBS = 770.0                         # peer-copy rate per direction per GPU quoted by B200_PROFILING.md
 NVLINK_MEASURED_GBS = 690.0                # what a peer accepts on these boxes with both directions busy: copy engine 708,
                                            # st.global / cp.async.bulk from 148 SMs 687 GB/s (profiles/r2_peer_bw_w2.log)
@@ -236,6 +243,19 @@ def time_graph(torch, step_fn, steps, warmup, dist=None):
     if dist is not None:
         dist.barrier()
     return e0.elapsed_time(e1), launches, t0, t1
+
+
+def dump_outputs(torch, out_dir, outputs):
+    """{name: (M, N) device tensor} -> out_dir/<name>.npy as float32 (exact for bf16), DUMP_ROWS full rows of each:
+    one row from every block of M / DUMP_ROWS rows, at an offset that walks through the block, so that every
+    row tile of the kernel and many row positions inside a tile are covered."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, c in outputs.items():
+        block = c.shape[0] // DUMP_ROWS
+        j = torch.arange(DUMP_ROWS, device=c.device)
+        rows = j * block + (5 * j) % block
+        np.save(os.path.join(out_dir, name + ".npy"), c[rows].float().cpu().numpy())
 
 
 def max_over_ranks(torch, dist, ms):
@@ -752,7 +772,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-sub", action="store_true", help="headline only")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a fixed row sample of the last timed step's results to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs is implemented for the single-GPU run of --impl ours")
     # stdout carries exactly ONE line: the JSON.  Libraries chat on fd 1 (NCCL prints its version there, the
     # patch prints like the reference), so fd 1 is pointed at stderr for the run and the line goes to the saved fd.
     global _JSON_OUT
@@ -808,6 +832,8 @@ def main():
     sampler.start()
     if n_gpus == 1:
         ms, launches_per_step, t0, t1 = time_graph(torch, step_single, steps, warmup)
+        if args.dump_outputs:                      # the graph's last replay wrote every `out`; nothing has run since
+            dump_outputs(torch, args.dump_outputs, {f"c4_out_set{i}": b[4] for i, b in enumerate(bufs)})
         clocks = sampler.summary(t0, t1)
         kernel_us = ms / steps * 1e3 / SETS
         kernel_name = "fp8b::fp8_gemm_tcgen05_kernel<256,2,2> (CTA pairs, 256x256 tiles, TMA-store epilogue)"

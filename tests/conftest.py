@@ -34,8 +34,23 @@ def _ensure_built():
     c_oracle.build()
 
 
+class _RootIsNotATestPackage:
+    """The repository root has an __init__.py because ComfyUI loads a clone of it as a custom node.  pytest would
+    collect the root as a package and, before every test, import that __init__.py as a module named after the
+    clone's directory, found through the directory above it.  Every test then errors when that directory cannot
+    be listed, and otherwise the import installs the patches for the whole session.  The root is collected as a
+    plain directory instead."""
+
+    @pytest.hookimpl(tryfirst=True)
+    def pytest_collect_directory(self, path, parent):
+        if os.path.samefile(path, ROOT):
+            return pytest.Dir.from_parent(parent, path=path)
+        return None
+
+
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (B200); run with -m gpu")
+    config.pluginmanager.register(_RootIsNotATestPackage(), "fp8b-root-is-not-a-test-package")
     _ensure_built()
 
 
