@@ -31,7 +31,7 @@ PROFILE = os.environ.get("FP8B_BUILD_PROFILE") == "1"
 OBJ = os.path.join(ROOT, "profiles", "tools", "bin", "obj") if PROFILE else os.path.join(HERE, "build")
 LIB = os.path.join(ROOT, "profiles", "tools", "bin", "libfp8_b200_profile.so") if PROFILE else os.path.join(HERE, "libfp8_b200.so")
 
-CU_SOURCES = ["fp8_cast.cu", "fp8_gemv.cu", "fp8_gemv_mma.cu", "fp8_gemv_rows.cu", "fp8_gemv_batch.cu", "fp8_gemv_ring.cu", "fp8_gemm_simt.cu", "fp8_gemm_tcgen05.cu", "fp8_capi.cu"]
+CU_SOURCES = ["fp8_cast.cu", "fp8_gemv.cu", "fp8_gemv_mma.cu", "fp8_gemv_batch.cu", "fp8_gemm_simt.cu", "fp8_gemm_tcgen05.cu", "fp8_capi.cu"]
 HEADERS = ["fp8_codec.cuh", "fp8_common.cuh", "fp8_mm.cuh", "fp8_async.cuh"]
 # -DFP8B_PROFILE adds the GEMM's profiling knobs (per-tile clock stamps, store/TMA suppression); never in a shipped build
 EXTRA_NVCC_FLAGS = (["-DFP8B_PROFILE"] + os.environ.get("FP8B_PROFILE_DEFINES", "").split()) if os.environ.get("FP8B_BUILD_PROFILE") == "1" else []

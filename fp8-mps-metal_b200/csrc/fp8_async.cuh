@@ -1,5 +1,5 @@
-// mbarrier / async-proxy PTX wrappers shared by the kernels that move data with the TMA unit
-// (fp8_gemm_tcgen05.cu: tensor-map tiles; fp8_gemv_ring.cu: 1-D bulk copies).
+// mbarrier / async-proxy PTX wrappers for the kernels that move data with the TMA unit
+// (fp8_gemm_tcgen05.cu: tensor-map tiles).
 #pragma once
 #include <cstdint>
 
@@ -43,13 +43,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
             if (t1 - t0 > 4000000000ull) __trap();      // 4 s
         }
     }
-}
-
-// 1-D bulk copy global -> shared (SASS UBLKCP), completion counted in bytes on an mbarrier.  16-byte aligned
-// addresses, size a multiple of 16.
-__device__ __forceinline__ void bulk_load_1d(uint32_t smem_dst, const void* gsrc, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 :: "r"(smem_dst), "l"(gsrc), "r"(bytes), "r"(bar) : "memory");
 }
 
 }  // namespace fp8b

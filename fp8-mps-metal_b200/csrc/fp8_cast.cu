@@ -15,7 +15,6 @@
 // The tile kernels run under programmatic dependent launch: coherent loads only.
 #include "fp8_codec.cuh"
 #include "fp8_common.cuh"
-#include "fp8_async.cuh"
 
 namespace fp8b {
 
@@ -178,136 +177,6 @@ fp8_to_wide_kernel(const uint8_t* __restrict__ in, void* __restrict__ out, size_
         decode_tile<OUT, SCALED, THREADS, UNROLL, FMT>(in, o8, (r * gridDim.x + blockIdx.x) * (size_t)(THREADS * UNROLL), nvec, s2);
     if (walk.rem_begin < walk.rem_end) decode_tile<OUT, SCALED, THREADS, UNROLL, FMT>(in, o8, walk.rem_begin, walk.rem_end, s2);
     if (blockIdx.x == 0 && threadIdx.x == 0) decode_tail<OUT, SCALED, FMT>(in, out, nvec * EPV, n, scale);
-}
-
-// ------------------------------------------------------------------------------------------
-// FP8 -> wide through the TMA unit.  The LDG/STG kernel above is limited by what its threads can keep in flight: two
-// thirds of its traffic are stores, each thread holds its loads in registers until it has stored them, and one
-// launch never got past 6.1 TB/s while four concurrent launches reach 6.5 (DESIGN.md 3.1).  Here no thread ever
-// touches global memory:
-//   warp 8 (producer)   cp.async.bulk global -> shared of 8 KB (f16/bf16 out) or 4 KB (f32 out) input tiles into a
-//                       4-deep ring, completion on an mbarrier;
-//   warps 0..7          convert shared -> shared: LDS.64 of 8 codes -> F2FP -> one conflict-free STS.128 into a
-//                       3-deep ring of 16 KB output tiles;
-//   thread 0            after the tile barrier: cp.async.bulk shared -> global of the 16 KB tile (full lines, no
-//                       partial-sector writes), up to two stores still READING shared memory while the next tile
-//                       is converted, all of them in flight until the CTA ends.
-// Each CTA owns one contiguous 1/gridDim share of the tensor (equal to within 16 bytes of input), so all SMs finish
-// together.  Needs 16-byte aligned in / out; the < 16-element ragged tail is the usual scalar tail.
-constexpr int kTmaCvtWarps = 8;
-constexpr int kTmaCvtThreads = 32 * kTmaCvtWarps;
-constexpr int kTmaInStages = 4;
-constexpr int kTmaOutStages = 3;
-constexpr int kTmaOutTile = 16384;
-constexpr bool kCastTmaDefault = false;        // measured choice (DESIGN.md 3.1)
-
-__device__ __forceinline__ void bulk_store_1d(void* gdst, uint32_t smem_src, uint32_t bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" :: "l"(gdst), "r"(smem_src), "r"(bytes) : "memory");
-}
-
-template <int OUT, bool SCALED, int FMT = 0>
-__global__ void __launch_bounds__(kTmaCvtThreads + 32)
-fp8_to_wide_tma_kernel(const uint8_t* __restrict__ in, void* __restrict__ out, size_t n, const float* __restrict__ scale)
-{
-    constexpr int ESZ = (OUT == FP8B_F32) ? 4 : 2;
-    constexpr int IN_TILE = kTmaOutTile / ESZ;                 // input bytes (= elements) per tile
-    constexpr int EPT = 16 / ESZ;                              // elements per thread-step: one 16-byte output vector
-    extern __shared__ __align__(128) uint8_t cvt_smem[];
-    uint8_t* in_ring = cvt_smem;
-    uint8_t* out_ring = cvt_smem + kTmaInStages * IN_TILE;
-    uint8_t* bar_mem = out_ring + kTmaOutStages * kTmaOutTile;
-    const uint32_t bar_base = smem_u32(bar_mem);
-    auto full_bar = [&](int s) { return bar_base + 8u * s; };
-    auto empty_bar = [&](int s) { return bar_base + 8u * (kTmaInStages + s); };
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    // this CTA's share: 16-element granules [g_begin, g_end)
-    const size_t granules = n / 16;
-    const size_t per = (granules + gridDim.x - 1) / gridDim.x;
-    const size_t g_begin = min(granules, (size_t)blockIdx.x * per);
-    const size_t g_end = min(granules, g_begin + per);
-    const size_t e_begin = g_begin * 16, e_end = g_end * 16;   // element range, multiples of 16
-    const int ntiles = (int)((e_end - e_begin + IN_TILE - 1) / IN_TILE);
-
-    pdl_launch_dependents();
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < kTmaInStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-        fence_mbar_init();
-    }
-    __syncthreads();
-    pdl_wait();
-
-    if (warp == kTmaCvtWarps) {
-        if (lane == 0) {
-            for (int i = 0; i < ntiles; ++i) {
-                const int s = i % kTmaInStages;
-                const size_t e0 = e_begin + (size_t)i * IN_TILE;
-                const uint32_t bytes = (uint32_t)min((size_t)IN_TILE, e_end - e0);
-                mbar_wait(empty_bar(s), ((i / kTmaInStages) & 1) ^ 1);
-                mbar_arrive_expect_tx(full_bar(s), bytes);
-                bulk_load_1d(smem_u32(in_ring + s * IN_TILE), in + e0, bytes, full_bar(s));
-            }
-        }
-    } else {
-        uint32_t s2 = 0;
-        if (SCALED) {
-            __half2 sc = __float2half2_rn(ld_scalar_f32(scale));   // RN16(scale), native.py:121
-            s2 = *reinterpret_cast<uint32_t*>(&sc);
-        }
-        uint8_t* o8 = reinterpret_cast<uint8_t*>(out);
-        for (int i = 0; i < ntiles; ++i) {
-            const int s = i % kTmaInStages, so = i % kTmaOutStages;
-            const size_t e0 = e_begin + (size_t)i * IN_TILE;
-            const int elems = (int)min((size_t)IN_TILE, e_end - e0);
-            // the store issued kTmaOutStages tiles ago must have finished reading its shared-memory tile
-            if (threadIdx.x == 0 && i >= kTmaOutStages) asm volatile("cp.async.bulk.wait_group.read %0;" :: "n"(kTmaOutStages - 1) : "memory");
-            mbar_wait(full_bar(s), (i / kTmaInStages) & 1);
-            asm volatile("bar.sync 1, %0;" :: "n"(kTmaCvtThreads) : "memory");
-            const uint8_t* src = in_ring + s * IN_TILE;
-            uint8_t* dst = out_ring + so * kTmaOutTile;
-#pragma unroll 4
-            for (int v = threadIdx.x; v * EPT < elems; v += kTmaCvtThreads) {
-                uint4 o;
-                if (OUT == FP8B_F32) {
-                    const uint32_t w = *reinterpret_cast<const uint32_t*>(src + v * 4);
-                    uint32_t lo, hi;
-                    dec4_fmt_f16x2<FMT>(w, lo, hi);
-                    const float2 a = __half22float2(*reinterpret_cast<__half2*>(&lo));
-                    const float2 c = __half22float2(*reinterpret_cast<__half2*>(&hi));
-                    o = make_uint4(__float_as_uint(a.x), __float_as_uint(a.y), __float_as_uint(c.x), __float_as_uint(c.y));
-                } else {
-                    const uint2 w = *reinterpret_cast<const uint2*>(src + v * 8);
-                    dec4_fmt_f16x2<FMT>(w.x, o.x, o.y);
-                    dec4_fmt_f16x2<FMT>(w.y, o.z, o.w);
-                    if (SCALED) {                               // fp16 multiply, native.py:122
-                        const __half2 sc = *reinterpret_cast<const __half2*>(&s2);
-                        uint32_t* q = &o.x;
-#pragma unroll
-                        for (int j = 0; j < 4; ++j) {
-                            __half2 r = __hmul2(*reinterpret_cast<__half2*>(&q[j]), sc);
-                            q[j] = *reinterpret_cast<uint32_t*>(&r);
-                        }
-                    }
-                    if (OUT == FP8B_BF16) {
-                        o.x = f16x2_to_bf16x2(o.x); o.y = f16x2_to_bf16x2(o.y);
-                        o.z = f16x2_to_bf16x2(o.z); o.w = f16x2_to_bf16x2(o.w);
-                    }
-                }
-                *reinterpret_cast<uint4*>(dst + v * 16) = o;
-            }
-            fence_proxy_async_smem();                           // generic-proxy writes -> visible to the bulk store
-            asm volatile("bar.sync 1, %0;" :: "n"(kTmaCvtThreads) : "memory");
-            if (threadIdx.x == 0) {
-                bulk_store_1d(o8 + e0 * ESZ, smem_u32(dst), (uint32_t)(elems * ESZ));
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                mbar_arrive(empty_bar(s));                      // every converter is past its reads of the input tile
-            }
-        }
-        if (threadIdx.x == 0) {
-            asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-            if (blockIdx.x == 0) decode_tail<OUT, SCALED, FMT>(in, out, granules * 16, n, scale);
-        }
-    }
 }
 
 template <int OUT, bool SCALED, int FMT = 0>
@@ -754,25 +623,11 @@ static int launch_decode_vec(const uint8_t* in, void* out, size_t n, const float
     constexpr int EPV = (OUT == FP8B_F32) ? 4 : 8;
     const CastShape c = cast_shape(n / EPV);
     const bool pdl = g_opt_pdl.load(std::memory_order_relaxed) != 0;
-    // TMA-pipelined kernel for tensors that give every SM several tiles (CAST_SHAPE 3 / 4 force it with 1 / 2 CTAs per SM)
-    const int mode = tune(kTuneCastShape, 0);
-    const bool tma_fit = aligned(in, 16) && aligned(out, 16) && n >= 64;
-    if (tma_fit && (mode == 3 || mode == 4 || (mode == 0 && kCastTmaDefault && n >= (size_t)device_info().sm_count * 65536))) {
-        constexpr int ESZ = (OUT == FP8B_F32) ? 4 : 2;
-        constexpr int kSmem = kTmaInStages * (kTmaOutTile / ESZ) + kTmaOutStages * kTmaOutTile + 2 * kTmaInStages * 8;
-        static std::atomic<int> attr_done[64];
-        if (int rc = ensure_max_smem(fp8_to_wide_tma_kernel<OUT, SCALED, FMT>, kSmem, attr_done)) return rc;
-        const size_t tiles = (n + (kTmaOutTile / ESZ) - 1) / (kTmaOutTile / ESZ);
-        size_t grid = (size_t)device_info().sm_count * (mode == 3 ? 1 : 2);
-        if (grid > tiles) grid = tiles;
-        return launch_ex(fp8_to_wide_tma_kernel<OUT, SCALED, FMT>, dim3((unsigned)grid), dim3(kTmaCvtThreads + 32), (size_t)kSmem, st, 1, 1,
-                         pdl, in, out, n, scale);
-    }
 #ifdef FP8B_PROFILE
     // launch-shape sweep for the write-heavy direction (profiling builds only): CAST_SHAPE 11.. = threads x unroll x CTAs/SM
     if constexpr (OUT == FP8B_F16 && !SCALED && FMT == 0) {
         const int sms = device_info().sm_count;
-        switch (mode) {
+        switch (tune(kTuneCastShape, 0)) {
             case 11: return launch_ex(fp8_to_wide_kernel<OUT, SCALED, 256, 8, FMT>, dim3(sms * 2), dim3(256), 0, st, 1, 1, pdl, in, out, n, scale);
             case 12: return launch_ex(fp8_to_wide_kernel<OUT, SCALED, 256, 8, FMT>, dim3(sms * 4), dim3(256), 0, st, 1, 1, pdl, in, out, n, scale);
             case 13: return launch_ex(fp8_to_wide_kernel<OUT, SCALED, 512, 4, FMT>, dim3(sms * 2), dim3(512), 0, st, 1, 1, pdl, in, out, n, scale);

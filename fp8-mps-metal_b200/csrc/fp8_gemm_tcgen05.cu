@@ -49,15 +49,8 @@ constexpr int kEpiColSplits = kNumEpiWarps / 4;
 //              128-row x 128-byte box with cp.async.bulk.tensor (TMA store) to 1..8 destinations -- this rank's
 //              buffer and, over NVLink, the same place in every peer's buffer.  The epilogue warps never wait on
 //              the memory system, so the accumulator goes back to the MMA warp as soon as TMEM is drained.
-//   kStWide    kStTma with ONE box per tile and CTA: 128 rows x the whole tile width (16-bit outputs), linear in shared
-//              memory (SWIZZLE_NONE tensor map over 16-bit elements), so every row leaves as one 256- or 512-byte
-//              write instead of the 128 bytes a 128B-swizzled box allows.  NVLink moves 128-byte row segments at
-//              595 GB/s of the ~690 GB/s a peer accepts for contiguous writes (profiles/r2_scaling.md).  The epilogue's
-//              st.shared are then 8-way bank-conflicted -- ~256 cycles per tile, irrelevant next to a 9 000-cycle tile.
-//              (Also tried: one 1-D cp.async.bulk per 256-byte row -- 118 us against 98 us at w = 2: the TMA unit
-//              retires only about one bulk copy per 230 cycles.)
-enum { kStDirect = 0, kStPeers = 1, kStTma = 2, kStWide = 3 };
-template <int MODE> constexpr bool is_push() { return MODE == kStTma || MODE == kStWide; }
+enum { kStDirect = 0, kStPeers = 1, kStTma = 2 };
+template <int MODE> constexpr bool is_push() { return MODE == kStTma; }
 constexpr int kMaxDst = 8;
 template <int MODE> constexpr int gemm_threads() { return 64 + 32 * kNumEpiWarps + (is_push<MODE>() ? 32 : 0); }
 
@@ -90,10 +83,8 @@ template <int BN, int CG, int MODE = kStDirect> struct GemmCfg {
     static constexpr int kBRows = BN / CG;                         // B rows staged by one CTA
     static constexpr int kBBytes = kBRows * kBK;
     static constexpr int kStageBytes = kABytes + kBBytes;
-    static constexpr int kSlotBytes = MODE == kStWide ? kBM * BN * 2 : kStoreBoxBytes;     // kStWide: 128 rows x BN 16-bit columns
-    static constexpr int kStoreSlots = MODE == kStWide ? (kSlotBytes <= 32768 ? 3 : 2) : FP8B_TMA_SLOTS; // ring of store boxes
     // epilogue staging: per epilogue warp 32 rows x 256 B, XOR-swizzled -- or the store ring
-    static constexpr int kEpiStageBytes = is_push<MODE>() ? kStoreSlots * kSlotBytes : kNumEpiWarps * 8192;
+    static constexpr int kEpiStageBytes = is_push<MODE>() ? FP8B_TMA_SLOTS * kStoreBoxBytes : kNumEpiWarps * 8192;
     static constexpr int kStagesFit = (232448 - 1024 - 256 - kEpiStageBytes) / kStageBytes;
     static constexpr int kStages = kStagesFit > 8 ? 8 : kStagesFit;
     static constexpr int kTmemCols = (2 * BN > 256) ? 512 : 256;   // two accumulators; a power of two >= 32
@@ -103,10 +94,10 @@ template <int BN, int CG, int MODE = kStDirect> struct GemmCfg {
     static constexpr int kOffBar = kOffStaging + kEpiStageBytes;
     static constexpr int kSmemBytes = kOffBar + kBarBytes + 1024;   // +1024: manual alignment
     static_assert(kStageBytes % 1024 == 0, "operand stages must keep the 1024-byte swizzle alignment");
-    static_assert((2 * kStages + 4 + 2 * kStoreSlots) * 8 + 8 <= kBarBytes, "barrier block too small");
+    static_assert((2 * kStages + 4 + 2 * FP8B_TMA_SLOTS) * 8 + 8 <= kBarBytes, "barrier block too small");
 };
 
-// kStTma / kStWide: one tensor map per destination buffer, plus the optional completion signal: when the last CTA of
+// kStTma: one tensor map per destination buffer, plus the optional completion signal: when the last CTA of
 // the grid has pushed its last box, it stores `epoch` into sig[d] for every peer d (a flag in the PEER's memory).
 struct StoreMaps {
     CUtensorMap m[kMaxDst];
@@ -118,7 +109,6 @@ struct StoreMaps {
 struct NoStoreMaps { int unused; };
 template <int MODE> struct StoreMapsOf { using type = NoStoreMaps; };
 template <> struct StoreMapsOf<kStTma> { using type = StoreMaps; };
-template <> struct StoreMapsOf<kStWide> { using type = StoreMaps; };
 
 struct GemmParams {
     const uint8_t* A; const uint8_t* B;      // for the NaN fix-up only
@@ -462,9 +452,9 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
     auto tfull_bar = [&](int a) { return bar_base + 8u * (2 * Cfg::kStages + a); };
     auto tempty_bar = [&](int a) { return bar_base + 8u * (2 * Cfg::kStages + 2 + a); };
     auto sfull_bar = [&](int s) { return bar_base + 8u * (2 * Cfg::kStages + 4 + s); };
-    auto sfree_bar = [&](int s) { return bar_base + 8u * (2 * Cfg::kStages + 4 + Cfg::kStoreSlots + s); };
+    auto sfree_bar = [&](int s) { return bar_base + 8u * (2 * Cfg::kStages + 4 + FP8B_TMA_SLOTS + s); };
     volatile uint32_t* tmem_slot =
-        reinterpret_cast<volatile uint32_t*>(bar_mem + 8 * (2 * Cfg::kStages + 4 + 2 * Cfg::kStoreSlots));
+        reinterpret_cast<volatile uint32_t*>(bar_mem + 8 * (2 * Cfg::kStages + 4 + 2 * FP8B_TMA_SLOTS));
     const uint32_t stage_base = smem_base + Cfg::kOffStaging;      // epilogue staging (1024-byte aligned)
 
     const int warp = __shfl_sync(0xFFFFFFFFu, (int)(threadIdx.x >> 5), 0);
@@ -487,7 +477,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
         for (int s = 0; s < Cfg::kStages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
         for (int a = 0; a < 2; ++a) { mbar_init(tfull_bar(a), 1); mbar_init(tempty_bar(a), kNumEpiWarps * CG); }
         if (is_push<MODE>())
-            for (int s = 0; s < Cfg::kStoreSlots; ++s) { mbar_init(sfull_bar(s), kNumEpiWarps); mbar_init(sfree_bar(s), 1); }
+            for (int s = 0; s < FP8B_TMA_SLOTS; ++s) { mbar_init(sfull_bar(s), kNumEpiWarps); mbar_init(sfree_bar(s), 1); }
         fence_mbar_init();
         fence_proxy_async_smem();
     }
@@ -606,7 +596,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
             }
         }
     } else if (is_push<MODE>() && warp == kWarpStore) {
-        // ===================== store issuer (kStTma / kStWide) =====================
+        // ===================== store issuer (kStTma) =====================
         // Walks the same (tile, box) sequence as the epilogue warps.  Per box: wait until the four epilogue warps
         // have filled the slot, issue the stores to every destination, commit; then recycle the slot whose stores have
         // finished READING shared memory (the writes themselves stay in flight).
@@ -622,8 +612,8 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                 for (int c = 0; c < tc.width; c += cols_per_box) {
                     const int n_box = tc.n0 + c;
                     if (n_box >= p.N) break;                      // warp-uniform; the epilogue skips the same boxes
-                    const uint32_t slot = seq % Cfg::kStoreSlots;
-                    mbar_wait(sfull_bar(slot), (seq / Cfg::kStoreSlots) & 1);
+                    const uint32_t slot = seq % FP8B_TMA_SLOTS;
+                    mbar_wait(sfull_bar(slot), (seq / FP8B_TMA_SLOTS) & 1);
                     if (elected) {
                         if (m_idx < p.M) {
                             const uint32_t src = stage_base + slot * kStoreBoxBytes;
@@ -631,7 +621,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                         }
                         bulk_commit_group();
                         bulk_wait_group_read<kStoreInflight>();
-                        if (seq >= (uint32_t)kStoreInflight) mbar_arrive(sfree_bar((seq - kStoreInflight) % Cfg::kStoreSlots));
+                        if (seq >= (uint32_t)kStoreInflight) mbar_arrive(sfree_bar((seq - kStoreInflight) % FP8B_TMA_SLOTS));
                     }
                     __syncwarp();
                     ++seq;
@@ -642,279 +632,158 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
 #ifdef FP8B_PROFILE
             if (dbg && blockIdx.x == 0 && lane == 0) dbg[15] = clock64();         // stores complete
 #endif
-        } else if constexpr (MODE == kStWide) {
-            // one box per tile: 128 rows x the tile width, coordinates in 16-bit elements
-            const bool elected = elect_one();
-            const int n_dst = p.store_mc >> 8;
-            constexpr int kInflight = 1;
-            uint32_t seq = 0;
-            for (int tile = worker; tile < num_tiles; tile += num_workers) {
-                const TileCoord tc = decode_tile(p, tile, BN);
-                const int m_idx = tc.m_blk * kTileM + (int)cta_rank * kBM;
-                if (tc.n0 >= p.N) continue;
-                const uint32_t slot = seq % Cfg::kStoreSlots;
-                mbar_wait(sfull_bar(slot), (seq / Cfg::kStoreSlots) & 1);
-                if (elected) {
-                    if (m_idx < p.M) {
-                        const uint32_t src = stage_base + slot * Cfg::kSlotBytes;
-                        for (int d = 0; d < n_dst; ++d) tma_store_2d(&smaps.m[d], src, tc.n0, m_idx);
-                    }
-                    bulk_commit_group();
-                    bulk_wait_group_read<kInflight>();
-                    if (seq >= (uint32_t)kInflight) mbar_arrive(sfree_bar((seq - kInflight) % Cfg::kStoreSlots));
-                }
-                __syncwarp();
-                ++seq;
-            }
-            if (elected) bulk_wait_group_all();
-            __syncwarp();
         }
     } else if (is_push<MODE>()) {
         // ===================== epilogue, store-ring flavour (warps 0..3) =====================
-        // tcgen05.ld -> scale/bias -> out dtype -> a box in shared memory.  Lane = row.  kStTma: 128 bytes per row,
+        // tcgen05.ld -> scale/bias -> out dtype -> a box in shared memory.  Lane = row, 128 bytes per row,
         // 16-byte piece j of row r at r*128 + ((j ^ (r & 7)) * 16) -- conflict-free st.shared.v4 and exactly the layout the
-        // SWIZZLE_128B tensor map of the store expects.  kStWide: BN 16-bit columns per row, linear.  Column/row edges
-        // need no code in either form: TMA clips the box.
+        // SWIZZLE_128B tensor map of the store expects.  Column/row edges need no code: TMA clips the box.
         if constexpr (is_push<MODE>()) {
-            constexpr bool kWide = MODE == kStWide;
             const int q = warp & 3;
             const int row_in_tile = q * 32 + lane;
             const Epi& e = p.epi;
             const float sr = e.sr ? *e.sr : 1.0f;
             const float sb0 = e.sb[0];
             const bool is_f32 = e.out_dtype == FP8B_F32;
-            const int cols_per_box = kWide ? BN : 128 / (is_f32 ? 4 : 2);      // kStWide: one box per tile (16-bit outputs only)
-            const uint32_t row_off = (uint32_t)row_in_tile * (kWide ? (uint32_t)(BN * 2) : 128u);
+            const int cols_per_box = 128 / (is_f32 ? 4 : 2);
+            const uint32_t row_off = (uint32_t)row_in_tile * 128u;
             uint32_t seq = 0;
             int acc = 0; uint32_t acc_phase = 0;
-            if constexpr (!kWide) {
-                // kStTma.  Software-pipelined: the tcgen05.ld of chunk c+1 is in flight while chunk c is scaled, packed and
-                // staged (two register sets).  Which optional epilogue terms exist (KIND) is a compile-time constant of the
-                // whole tile loop -- one of eight copies runs -- and the cold paths (NaN fix-up, ragged column edge) are out
-                // of line, so the hot loop is short and contiguous: a 128 x 256 accumulator is drained in 4 900 cycles
-                // instead of 8 100-12 000.  That matters where the epilogue is exposed: the last tile of every CTA, i.e.
-                // all of a small problem.
-                auto run_tiles = [&](auto kind_c) {
-                    constexpr int KIND = decltype(kind_c)::value;
-                    constexpr bool SBV = (KIND & 1) != 0, BIAS = (KIND & 2) != 0, SR = (KIND & 4) != 0;
-                    for (int tile = worker; tile < num_tiles; tile += num_workers) {
-                        const TileCoord tc = decode_tile(p, tile, BN);
-                        const int m_idx = tc.m_blk * kTileM + (int)cta_rank * kBM;
-                        const int n_idx = tc.n0;
-                        const int m = m_idx + row_in_tile;
-                        const bool m_ok = m < p.M;
-                        const float sa = e.sa[(size_t)(m_ok ? m : 0) * e.sa_stride];
-                        const int nch = tc.width >> 5;                    // 32-column chunks in this tile (2..8), warp-uniform
+            // Software-pipelined: the tcgen05.ld of chunk c+1 is in flight while chunk c is scaled, packed and
+            // staged (two register sets).  Which optional epilogue terms exist (KIND) is a compile-time constant of the
+            // whole tile loop -- one of eight copies runs -- and the cold paths (NaN fix-up, ragged column edge) are out
+            // of line, so the hot loop is short and contiguous: a 128 x 256 accumulator is drained in 4 900 cycles
+            // instead of 8 100-12 000.  That matters where the epilogue is exposed: the last tile of every CTA, i.e.
+            // all of a small problem.
+            auto run_tiles = [&](auto kind_c) {
+                constexpr int KIND = decltype(kind_c)::value;
+                constexpr bool SBV = (KIND & 1) != 0, BIAS = (KIND & 2) != 0, SR = (KIND & 4) != 0;
+                for (int tile = worker; tile < num_tiles; tile += num_workers) {
+                    const TileCoord tc = decode_tile(p, tile, BN);
+                    const int m_idx = tc.m_blk * kTileM + (int)cta_rank * kBM;
+                    const int n_idx = tc.n0;
+                    const int m = m_idx + row_in_tile;
+                    const bool m_ok = m < p.M;
+                    const float sa = e.sa[(size_t)(m_ok ? m : 0) * e.sa_stride];
+                    const int nch = tc.width >> 5;                    // 32-column chunks in this tile (2..8), warp-uniform
 #ifdef FP8B_PROFILE
-                        const long long t_e0 = (dbg && blockIdx.x == 0 && warp == kWarpEpi0 && lane == 0) ? clock64() : 0;
+                    const long long t_e0 = (dbg && blockIdx.x == 0 && warp == kWarpEpi0 && lane == 0) ? clock64() : 0;
 #endif
-                        mbar_wait(tfull_bar(acc), acc_phase);
-                        tc_fence_after();
+                    mbar_wait(tfull_bar(acc), acc_phase);
+                    tc_fence_after();
 #ifdef FP8B_PROFILE
-                        const long long t_e1 = (dbg && blockIdx.x == 0 && warp == kWarpEpi0 && lane == 0) ? clock64() : 0;
+                    const long long t_e1 = (dbg && blockIdx.x == 0 && warp == kWarpEpi0 && lane == 0) ? clock64() : 0;
 #endif
-                        const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
-                        auto release_acc = [&]() {                        // every tcgen05.ld of this accumulator has completed
-                            tc_fence_before();
-                            __syncwarp();
-                            if (lane == 0) { if (CG == 2) mbar_arrive_leader(tempty_bar(acc)); else mbar_arrive(tempty_bar(acc)); }
-                        };
-                        auto chunk = [&](int c0, uint32_t (&r)[32]) {
-                            const int n0 = n_idx + c0;
-                            const int n_box = n_idx + (c0 & ~(cols_per_box - 1));
-                            if (n_box >= p.N) return;                     // whole box outside the matrix (warp-uniform): the store warp skips it too
-                            const bool box_first = (c0 & (cols_per_box - 1)) == 0;
-                            const bool box_last = ((c0 + 32) & (cols_per_box - 1)) == 0 || c0 + 32 == tc.width;
-                            const uint32_t slot = seq % Cfg::kStoreSlots;
-                            if (box_first) mbar_wait(sfree_bar(slot), ((seq / Cfg::kStoreSlots) & 1) ^ 1);
-                            if (n0 < p.N) {
-                                float sbv[32];
-                                float bv[32];
-                                if (SBV || BIAS) {
-                                    if ((n0 + 32 <= p.N) && p.col_vec_ok) {
-                                        load_col_params(e, n0, p.N, true, sbv, bv);
-                                    } else {                              // ragged edge / unaligned arrays (cold)
-                                        float t_sb[32], t_b[32];
-                                        load_col_params_edge(e, n0, p.N, t_sb, t_b);
-#pragma unroll
-                                        for (int j = 0; j < 32; ++j) { sbv[j] = t_sb[j]; bv[j] = t_b[j]; }
-                                    }
-                                }
-                                // NaN-byte fix-up (cold): a NaN accumulator can only come from a 0x7F/0xFF operand byte
-                                if (__any_sync(0xFFFFFFFFu, m_ok && any_nan32(r))) {
-                                    uint32_t t[32];
-#pragma unroll
-                                    for (int j = 0; j < 32; ++j) t[j] = r[j];
-                                    if (m_ok) fix_nan_chunk(t, p.A + (size_t)m * p.K, p.B + (size_t)n0 * p.K, p.K, p.N - n0,
-                                                            (p.debug >> 8) & 1, (p.debug >> 9) & 1);
-#pragma unroll
-                                    for (int j = 0; j < 32; ++j) r[j] = t[j];
-                                }
-                                float v[32];
-                                epi_math32<SBV, BIAS, SR>(r, sa, sb0, sr, sbv, bv, v);
-                                const uint32_t dst = stage_base + slot * Cfg::kSlotBytes + row_off;
-                                const uint32_t sw = (uint32_t)(lane & 7);
-                                // first 16-byte piece of this chunk inside the box row
-                                const uint32_t piece0 = (uint32_t)(((c0 & (cols_per_box - 1)) * (is_f32 ? 4 : 2)) >> 4);
-                                if (is_f32) {
-#pragma unroll
-                                    for (int j = 0; j < 8; ++j)
-                                        sts_v4(dst + (((piece0 + j) ^ sw) << 4), __float_as_uint(v[4 * j]), __float_as_uint(v[4 * j + 1]),
-                                               __float_as_uint(v[4 * j + 2]), __float_as_uint(v[4 * j + 3]));
-                                } else {
-                                    uint32_t pk[16];
-                                    if (e.out_dtype == FP8B_BF16) {
-#pragma unroll
-                                        for (int j = 0; j < 16; ++j) {
-                                            __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
-                                            pk[j] = *reinterpret_cast<uint32_t*>(&b);
-                                        }
-                                    } else {
-#pragma unroll
-                                        for (int j = 0; j < 16; ++j) {
-                                            __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
-                                            pk[j] = *reinterpret_cast<uint32_t*>(&h);
-                                        }
-                                    }
-#pragma unroll
-                                    for (int j = 0; j < 4; ++j)
-                                        sts_v4(dst + (((piece0 + j) ^ sw) << 4), pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
-                                }
-                            }
-                            if (box_last) {
-                                fence_proxy_async_smem();   // generic-proxy writes -> visible to the TMA (async proxy)
-                                __syncwarp();
-                                if (lane == 0) mbar_arrive(sfull_bar(slot));
-                                ++seq;
-                            }
-                        };
-                        uint32_t ra[32], rb[32];
-                        __syncwarp();
-                        tmem_ld_x32(t_row, ra);
-#pragma unroll 1
-                        for (int ch = 0; ch < nch; ch += 2) {
-                            __syncwarp();                   // lanes may have diverged in chunk() (row mask, NaN fix-up);
-                            tmem_ld_wait_for(ra);           // tcgen05.wait / .ld are warp-collective (.sync.aligned)
-                            if (ch + 1 < nch) tmem_ld_x32(t_row + (uint32_t)((ch + 1) * 32), rb); else release_acc();
-                            chunk(ch * 32, ra);
-                            if (ch + 1 < nch) {
-                                __syncwarp();
-                                tmem_ld_wait_for(rb);
-                                if (ch + 2 < nch) tmem_ld_x32(t_row + (uint32_t)((ch + 2) * 32), ra); else release_acc();
-                                chunk((ch + 1) * 32, rb);
-                            }
-                        }
-#ifdef FP8B_PROFILE
-                        if (dbg && blockIdx.x == 0 && warp == kWarpEpi0 && lane == 0) {
-                            const int ti = (tile - worker) / num_workers;
-                            if (ti < 64) { dbg[ti * 8 + 4] = t_e0; dbg[ti * 8 + 5] = t_e1; dbg[ti * 8 + 6] = clock64(); }
-                            dbg[23] = clock64();                                   // last epilogue end so far
-                        }
-#endif
-                        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-                    }
-                };
-                switch ((e.sb_stride ? 1 : 0) | (e.bias ? 2 : 0) | (e.sr ? 4 : 0)) {          // grid-uniform
-                    case 0: run_tiles(std::integral_constant<int, 0>{}); break;
-                    case 1: run_tiles(std::integral_constant<int, 1>{}); break;
-                    case 2: run_tiles(std::integral_constant<int, 2>{}); break;
-                    case 3: run_tiles(std::integral_constant<int, 3>{}); break;
-                    case 4: run_tiles(std::integral_constant<int, 4>{}); break;
-                    case 5: run_tiles(std::integral_constant<int, 5>{}); break;
-                    case 6: run_tiles(std::integral_constant<int, 6>{}); break;
-                    default: run_tiles(std::integral_constant<int, 7>{}); break;
-                }
-            } else
-            for (int tile = worker; tile < num_tiles; tile += num_workers) {
-                const TileCoord tc = decode_tile(p, tile, BN);
-                const int m_idx = tc.m_blk * kTileM + (int)cta_rank * kBM;
-                const int n_idx = tc.n0;
-                const int m = m_idx + row_in_tile;
-                const bool m_ok = m < p.M;
-                const float sa = e.sa[(size_t)(m_ok ? m : 0) * e.sa_stride];
-                mbar_wait(tfull_bar(acc), acc_phase);
-                tc_fence_after();
-                const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
-#pragma unroll 1
-                for (int c0 = 0; c0 < tc.width; c0 += 32) {
-                    uint32_t r[32];
-                    __syncwarp();
-                    tmem_ld_x32(t_row + c0, r);
-                    const int n0 = n_idx + c0;
-                    const int n_box = kWide ? n_idx : n_idx + (c0 & ~(cols_per_box - 1));
-                    const bool box_first = kWide ? c0 == 0 : (c0 & (cols_per_box - 1)) == 0;
-                    const bool box_last = kWide ? false : ((c0 + 32) & (cols_per_box - 1)) == 0;    // (or the tile's last chunk, below)
-                    const bool box_ok = n_box < p.N;                                   // warp-uniform
-                    const bool chunk_ok = n0 < p.N;
-                    float sbv[32];
-                    float bv[32];
-                    if (chunk_ok) load_col_params(e, n0, p.N, (n0 + 32 <= p.N) && p.col_vec_ok, sbv, bv);
-                    const uint32_t slot = seq % Cfg::kStoreSlots;
-                    if (box_ok && box_first) mbar_wait(sfree_bar(slot), ((seq / Cfg::kStoreSlots) & 1) ^ 1);
-                    tmem_ld_wait();
-                    if (c0 + 32 == tc.width) {              // last read of this accumulator: hand it back to the MMA warp
+                    const uint32_t t_row = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * BN);
+                    auto release_acc = [&]() {                        // every tcgen05.ld of this accumulator has completed
                         tc_fence_before();
                         __syncwarp();
                         if (lane == 0) { if (CG == 2) mbar_arrive_leader(tempty_bar(acc)); else mbar_arrive(tempty_bar(acc)); }
-                    }
-                    if (!box_ok) continue;
-                    if (chunk_ok) {
-                        // NaN-byte fix-up (cold): a NaN accumulator can only come from a 0x7F/0xFF operand byte
-                        float nan_probe = 0.0f;
+                    };
+                    auto chunk = [&](int c0, uint32_t (&r)[32]) {
+                        const int n0 = n_idx + c0;
+                        const int n_box = n_idx + (c0 & ~(cols_per_box - 1));
+                        if (n_box >= p.N) return;                     // whole box outside the matrix (warp-uniform): the store warp skips it too
+                        const bool box_first = (c0 & (cols_per_box - 1)) == 0;
+                        const bool box_last = ((c0 + 32) & (cols_per_box - 1)) == 0 || c0 + 32 == tc.width;
+                        const uint32_t slot = seq % FP8B_TMA_SLOTS;
+                        if (box_first) mbar_wait(sfree_bar(slot), ((seq / FP8B_TMA_SLOTS) & 1) ^ 1);
+                        if (n0 < p.N) {
+                            float sbv[32];
+                            float bv[32];
+                            if (SBV || BIAS) {
+                                if ((n0 + 32 <= p.N) && p.col_vec_ok) {
+                                    load_col_params(e, n0, p.N, true, sbv, bv);
+                                } else {                              // ragged edge / unaligned arrays (cold)
+                                    float t_sb[32], t_b[32];
+                                    load_col_params_edge(e, n0, p.N, t_sb, t_b);
 #pragma unroll
-                        for (int j = 0; j < 32; ++j) nan_probe += __uint_as_float(r[j]);
-                        if (__any_sync(0xFFFFFFFFu, m_ok && nan_probe != nan_probe)) {
-#pragma unroll
-                            for (int j = 0; j < 32; ++j) {
-                                const float a = __uint_as_float(r[j]);
-                                if (a != a && m_ok && n0 + j < p.N)
-                                    r[j] = __float_as_uint(slow_dot_fmt(p.A + (size_t)m * p.K, p.B + (size_t)(n0 + j) * p.K, p.K,
-                                                                        (p.debug >> 8) & 1, (p.debug >> 9) & 1));
-                            }
-                        }
-                        float v[32];
-#pragma unroll
-                        for (int j = 0; j < 32; ++j) {
-                            float x = __fmul_rn(__uint_as_float(r[j]), sa);
-                            x = __fmul_rn(x, e.sb_stride ? sbv[j] : sb0);
-                            if (e.bias) x = __fadd_rn(x, bv[j]);
-                            if (e.sr) x = __fmul_rn(x, sr);
-                            v[j] = x;
-                        }
-                        const uint32_t dst = stage_base + slot * Cfg::kSlotBytes + row_off;
-                        const uint32_t sw = kWide ? 0u : (uint32_t)(lane & 7);
-                        // first 16-byte piece of this chunk inside the box row
-                        const uint32_t piece0 = kWide ? (uint32_t)(c0 >> 3) : (uint32_t)(((c0 & (cols_per_box - 1)) * (is_f32 ? 4 : 2)) >> 4);
-                        if (is_f32) {
-#pragma unroll
-                            for (int j = 0; j < 8; ++j)
-                                sts_v4(dst + (((piece0 + j) ^ sw) << 4), __float_as_uint(v[4 * j]), __float_as_uint(v[4 * j + 1]),
-                                       __float_as_uint(v[4 * j + 2]), __float_as_uint(v[4 * j + 3]));
-                        } else {
-                            uint32_t pk[16];
-#pragma unroll
-                            for (int j = 0; j < 16; ++j) {
-                                if (e.out_dtype == FP8B_BF16) {
-                                    __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
-                                    pk[j] = *reinterpret_cast<uint32_t*>(&b);
-                                } else {
-                                    __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
-                                    pk[j] = *reinterpret_cast<uint32_t*>(&h);
+                                    for (int j = 0; j < 32; ++j) { sbv[j] = t_sb[j]; bv[j] = t_b[j]; }
                                 }
                             }
+                            // NaN-byte fix-up (cold): a NaN accumulator can only come from a 0x7F/0xFF operand byte
+                            if (__any_sync(0xFFFFFFFFu, m_ok && any_nan32(r))) {
+                                uint32_t t[32];
 #pragma unroll
-                            for (int j = 0; j < 4; ++j)
-                                sts_v4(dst + (((piece0 + j) ^ sw) << 4), pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+                                for (int j = 0; j < 32; ++j) t[j] = r[j];
+                                if (m_ok) fix_nan_chunk(t, p.A + (size_t)m * p.K, p.B + (size_t)n0 * p.K, p.K, p.N - n0,
+                                                        (p.debug >> 8) & 1, (p.debug >> 9) & 1);
+#pragma unroll
+                                for (int j = 0; j < 32; ++j) r[j] = t[j];
+                            }
+                            float v[32];
+                            epi_math32<SBV, BIAS, SR>(r, sa, sb0, sr, sbv, bv, v);
+                            const uint32_t dst = stage_base + slot * kStoreBoxBytes + row_off;
+                            const uint32_t sw = (uint32_t)(lane & 7);
+                            // first 16-byte piece of this chunk inside the box row
+                            const uint32_t piece0 = (uint32_t)(((c0 & (cols_per_box - 1)) * (is_f32 ? 4 : 2)) >> 4);
+                            if (is_f32) {
+#pragma unroll
+                                for (int j = 0; j < 8; ++j)
+                                    sts_v4(dst + (((piece0 + j) ^ sw) << 4), __float_as_uint(v[4 * j]), __float_as_uint(v[4 * j + 1]),
+                                           __float_as_uint(v[4 * j + 2]), __float_as_uint(v[4 * j + 3]));
+                            } else {
+                                uint32_t pk[16];
+                                if (e.out_dtype == FP8B_BF16) {
+#pragma unroll
+                                    for (int j = 0; j < 16; ++j) {
+                                        __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
+                                        pk[j] = *reinterpret_cast<uint32_t*>(&b);
+                                    }
+                                } else {
+#pragma unroll
+                                    for (int j = 0; j < 16; ++j) {
+                                        __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
+                                        pk[j] = *reinterpret_cast<uint32_t*>(&h);
+                                    }
+                                }
+#pragma unroll
+                                for (int j = 0; j < 4; ++j)
+                                    sts_v4(dst + (((piece0 + j) ^ sw) << 4), pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+                            }
+                        }
+                        if (box_last) {
+                            fence_proxy_async_smem();   // generic-proxy writes -> visible to the TMA (async proxy)
+                            __syncwarp();
+                            if (lane == 0) mbar_arrive(sfull_bar(slot));
+                            ++seq;
+                        }
+                    };
+                    uint32_t ra[32], rb[32];
+                    __syncwarp();
+                    tmem_ld_x32(t_row, ra);
+#pragma unroll 1
+                    for (int ch = 0; ch < nch; ch += 2) {
+                        __syncwarp();                   // lanes may have diverged in chunk() (row mask, NaN fix-up);
+                        tmem_ld_wait_for(ra);           // tcgen05.wait / .ld are warp-collective (.sync.aligned)
+                        if (ch + 1 < nch) tmem_ld_x32(t_row + (uint32_t)((ch + 1) * 32), rb); else release_acc();
+                        chunk(ch * 32, ra);
+                        if (ch + 1 < nch) {
+                            __syncwarp();
+                            tmem_ld_wait_for(rb);
+                            if (ch + 2 < nch) tmem_ld_x32(t_row + (uint32_t)((ch + 2) * 32), ra); else release_acc();
+                            chunk((ch + 1) * 32, rb);
                         }
                     }
-                    if (box_last || c0 + 32 == tc.width) {
-                        fence_proxy_async_smem();           // generic-proxy writes -> visible to the TMA (async proxy)
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(sfull_bar(slot));
-                        ++seq;
+#ifdef FP8B_PROFILE
+                    if (dbg && blockIdx.x == 0 && warp == kWarpEpi0 && lane == 0) {
+                        const int ti = (tile - worker) / num_workers;
+                        if (ti < 64) { dbg[ti * 8 + 4] = t_e0; dbg[ti * 8 + 5] = t_e1; dbg[ti * 8 + 6] = clock64(); }
+                        dbg[23] = clock64();                                   // last epilogue end so far
                     }
+#endif
+                    if (++acc == 2) { acc = 0; acc_phase ^= 1; }
                 }
-                if (++acc == 2) { acc = 0; acc_phase ^= 1; }
+            };
+            switch ((e.sb_stride ? 1 : 0) | (e.bias ? 2 : 0) | (e.sr ? 4 : 0)) {          // grid-uniform
+                case 0: run_tiles(std::integral_constant<int, 0>{}); break;
+                case 1: run_tiles(std::integral_constant<int, 1>{}); break;
+                case 2: run_tiles(std::integral_constant<int, 2>{}); break;
+                case 3: run_tiles(std::integral_constant<int, 3>{}); break;
+                case 4: run_tiles(std::integral_constant<int, 4>{}); break;
+                case 5: run_tiles(std::integral_constant<int, 5>{}); break;
+                case 6: run_tiles(std::integral_constant<int, 6>{}); break;
+                default: run_tiles(std::integral_constant<int, 7>{}); break;
             }
         }
     } else {
@@ -1458,22 +1327,21 @@ static PFN_encodeTiled get_encode_fn()
 // analogue of the reference bridge's one-time pipeline cache, fp8_bridge.cpp:103-141).  A map holds only addresses
 // and extents, never data, so a stale entry for a freed-and-reallocated pointer with the same geometry is still right.
 struct MapKey {
-    const void* base; uint64_t rows, row_bytes, pitch; uint32_t box_rows, box_bytes, esz_swz;
+    const void* base; uint64_t rows, row_bytes, pitch; uint32_t box_rows, box_bytes;
     bool operator==(const MapKey& o) const {
         return base == o.base && rows == o.rows && row_bytes == o.row_bytes && pitch == o.pitch &&
-               box_rows == o.box_rows && box_bytes == o.box_bytes && esz_swz == o.esz_swz;
+               box_rows == o.box_rows && box_bytes == o.box_bytes;
     }
 };
 struct MapSlot { MapKey key; CUtensorMap map; bool valid; };
 constexpr int kMapCacheSlots = 64;
 
-// rows x row_elems matrix of esz-byte elements with a row pitch (bytes), box = box_rows x box_elems; 128B swizzle
-// (box_elems * esz <= 128) or none (linear box, box_elems <= 256).
+// rows x row_bytes uint8 matrix with a row pitch, box = box_rows x box_bytes (<= 128), 128B swizzle.
 static bool get_tensor_map(CUtensorMap* out, const void* base, uint64_t rows, uint64_t row_bytes, uint64_t pitch,
-                           uint32_t box_rows, uint32_t box_bytes, uint32_t esz = 1, bool swizzle128 = true)
+                           uint32_t box_rows, uint32_t box_bytes)
 {
     static thread_local MapSlot cache[kMapCacheSlots];
-    const MapKey key = {base, rows, row_bytes, pitch, box_rows, box_bytes, esz * 2 + (swizzle128 ? 1u : 0u)};
+    const MapKey key = {base, rows, row_bytes, pitch, box_rows, box_bytes};
     uint64_t h = reinterpret_cast<uintptr_t>(base) >> 4;
     h ^= rows * 0x9E3779B97F4A7C15ull; h ^= row_bytes * 0xC2B2AE3D27D4EB4Full; h ^= pitch << 7; h ^= (uint64_t)box_rows << 40;
     h ^= h >> 29;
@@ -1485,9 +1353,9 @@ static bool get_tensor_map(CUtensorMap* out, const void* base, uint64_t rows, ui
     cuuint64_t strides[1] = {(cuuint64_t)pitch};
     cuuint32_t box[2] = {(cuuint32_t)box_bytes, (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(out, esz == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base),
+    CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base),
                      dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return false;
     s.key = key; s.map = *out; s.valid = true;
@@ -1576,7 +1444,6 @@ static int launch_tcgen05_cfg(const MMArgs& a)
         const int rem = tiles_all % workers_cap;
         bool can_split = (BN % 64 == 0) && ((BN / 2 / CG) % 8 == 0) && tiles_all > workers_cap;
         if (MODE == kStTma) can_split = can_split && ((BN / 2) * esz) % 128 == 0;      // half tiles must be whole store boxes
-        if (MODE == kStWide) can_split = false;                                        // one fixed-width box per tile
 #ifdef FP8B_PROFILE
         can_split = can_split && !(tune_int("FP8B_GEMM_DEBUG", 0) & 8);
 #endif
@@ -1603,17 +1470,6 @@ static int launch_tcgen05_cfg(const MMArgs& a)
         if (n_dst < 1 || n_dst > kMaxDst || !tma_store_ok(a, dsts, n_dst)) return FP8B_ERR_UNSUPPORTED;
         for (int d = 0; d < n_dst; ++d)
             if (!get_tensor_map(&smaps.m[d], dsts[d], (uint64_t)a.M, (uint64_t)a.N * esz, (uint64_t)a.ldc * esz, 128, 128))
-                return FP8B_ERR_CUDA;
-        for (int d = n_dst; d < kMaxDst; ++d) smaps.m[d] = smaps.m[0];
-        fill_signal(smaps, a);
-    } else if constexpr (MODE == kStWide) {  // same arguments; 16-bit outputs, one linear box per tile
-        const int n_dst = a.store_mc >> 8;
-        void* const* dsts = static_cast<void* const*>(a.ws);
-        void* self[1] = {a.C};
-        if (!dsts) dsts = self;
-        if (esz != 2 || n_dst < 1 || n_dst > kMaxDst || !tma_store_ok(a, dsts, n_dst)) return FP8B_ERR_UNSUPPORTED;
-        for (int d = 0; d < n_dst; ++d)
-            if (!get_tensor_map(&smaps.m[d], dsts[d], (uint64_t)a.M, (uint64_t)a.N, (uint64_t)a.ldc * 2, 128, BN, 2, false))
                 return FP8B_ERR_CUDA;
         for (int d = n_dst; d < kMaxDst; ++d) smaps.m[d] = smaps.m[0];
         fill_signal(smaps, a);
@@ -1760,7 +1616,6 @@ static int pick_split_k(const MMArgs& a)
     return 0;
 }
 
-constexpr bool kPushWideDefault = false;   // push to peers: one linear box per tile instead of 128-byte-wide boxes (measured choice)
 constexpr int kDefaultGemmStore = 2;      // epilogue of plain fp8b_scaled_mm calls: 1 = st.global from the epilogue warps, 2 = TMA
                                           // store (C4: 109.7 vs 112.0 us in the same bench run; falls back to 1 when C is not TMA-storable)
 
@@ -1825,19 +1680,6 @@ int launch_gemm_tcgen05(const MMArgs& a)
         }
     }
     if (mode == 3) {          // store-ring epilogue, 1..8 destinations
-        // 16-bit outputs going to peers: one linear box per tile (256- / 512-byte NVLink writes); else 128-byte-wide
-        // swizzled boxes.  FP8B_OPT_TUNE_GEMM_STORE 3 / 4 force the wide / the 128-byte form.
-        const int st = tune(kTuneGemmStore, 0);
-        const bool wide = dtype_size(a.out_dtype) == 2 && (st == 3 || (st != 4 && kPushWideDefault && (a.store_mc >> 8) > 1));
-        if (wide) {
-            switch (cfg) {
-                case 1: return launch_tcgen05_cfg<256, 1, kStWide>(a);
-                case 3: return launch_tcgen05_cfg<256, 2, kStWide>(a);
-                case 4: return launch_tcgen05_cfg<128, 2, kStWide>(a);
-                case 5: return launch_tcgen05_cfg<192, 2, kStWide>(a);
-                default: return launch_tcgen05_cfg<128, 1, kStWide>(a);
-            }
-        }
         switch (cfg) {
             case 1: return launch_tcgen05_cfg<256, 1, kStTma>(a);
             case 3: return launch_tcgen05_cfg<256, 2, kStTma>(a);

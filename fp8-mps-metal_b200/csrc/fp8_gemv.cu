@@ -494,28 +494,20 @@ static int launch_gemv_xq_mt(const GemvXqParams& xp, int S, size_t smem, cudaStr
 
 int launch_gemv_fhfma(const MMArgs& a, const Epi& epi, const void* X, int x_dtype, float* inv_scale_out);
 
-constexpr bool kGemvRingDefault = false;     // measured choice, see DESIGN.md 3.2
-
 int launch_gemv(const MMArgs& a)
 {
     if (!gemv_supported(a)) return FP8B_ERR_UNSUPPORTED;
     // kernel choice: M == 1 -> CUDA-core FHFMA kernel (exact fp32 accumulation order per lane);
     // M >= 2 -> warp-level tensor-core kernel (weights streamed once for all M rows).
-    // FP8B_GEMV_IMPL=1 / 2 forces the first / second (profiling knob).
-    int impl = tune(kTuneGemvImpl, 0);
+    // FP8B_GEMV_IMPL=1 / 2 forces the first / second (profiling knob); any other value takes this rule.
+    const int impl = tune(kTuneGemvImpl, 0);
     if (a.a_fmt | a.b_fmt) {        // an e5m2 operand: the warp-MMA kernel has all four type pairs; else the generic kernel
         if (gemv_mma_supported(a)) return launch_gemv_mma(a);
         fp8_gemv_generic_kernel<<<(a.N + kGemvWarps - 1) / kGemvWarps, kGemvThreads, 0, a.st>>>(a.A, a.B, a.M, a.N, a.K, make_epi(a),
                                                                                              a.a_fmt, a.b_fmt);
         return after_launch();
     }
-    // impl 4: the persistent TMA-ring kernel (fp8_gemv_ring.cu); where it does not apply the default rule decides
-    if (impl == 4 || (impl == 0 && kGemvRingDefault)) {
-        if (!a.chain_pdl && gemv_ring_supported(a)) return launch_gemv_ring(a);
-        impl = 0;
-    }
-    if (gemv_mma_supported(a) && (impl == 2 || (impl == 0 && a.M >= 2))) return launch_gemv_mma(a);
-    if (gemv_rows_supported(a) && (impl == 3)) return launch_gemv_rows(a);
+    if (gemv_mma_supported(a) && (impl == 2 || (impl != 1 && a.M >= 2))) return launch_gemv_mma(a);
     const Epi epi = make_epi(a);
     const bool fast = (a.K % 16 == 0) && a.K >= 16 && aligned(a.A, 16) && aligned(a.B, 16);
     if (!fast) {

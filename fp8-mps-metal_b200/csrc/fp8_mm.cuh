@@ -38,10 +38,6 @@ struct MMArgs {
 bool gemv_supported(const MMArgs& a);
 bool tcgen05_supported(const MMArgs& a);
 int launch_gemv(const MMArgs& a);
-bool gemv_rows_supported(const MMArgs& a);
-int launch_gemv_rows(const MMArgs& a);
-bool gemv_ring_supported(const MMArgs& a);
-int launch_gemv_ring(const MMArgs& a);
 bool gemv_mma_supported(const MMArgs& a);
 int launch_gemv_mma(const MMArgs& a);
 int launch_gemm_simt(const MMArgs& a);

@@ -88,7 +88,7 @@ FP8B_API uint64_t fp8b_launch_count(void);
  *                            same name without the OPT_TUNE_ part (FP8B_GEMM_CFG, ...), read once at load time.
  *                              GEMM_CFG      tcgen05 tile: 1 = 128x256, 2 = 128x128 (one CTA); 3 = 256x256, 4 = 256x128,
  *                                            5 = 256x192 (CTA pairs)
- *                              GEMV_IMPL     1 = FHFMA warp-per-row, 2 = warp-MMA, 3 = SM-balanced rows, 4 = persistent TMA ring
+ *                              GEMV_IMPL     1 = FHFMA warp-per-row, 2 = warp-MMA (other values: the built-in rule)
  *                              DYNAMIC_PLAN  fp8b_linear_dynamic: 1 = single kernel, 2 = quantise + chained GEMV
  *                              CAST_SHAPE    cast launch shape: 1 = small tiles, 2 = big tiles
  *                              GEMM_STORE    tcgen05 epilogue: 1 = st.global from the epilogue warps, 2 = TMA store

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Launch one hot-path kernel a few times -- the short command ncu wraps (profiles/README.md).
 
-    python profiles/run_kernels.py gemm|gemm_stg|gemm_push2|gemv|gemv4|gemv1k4|gemv_ring|quant|dequant [reps]
+    python profiles/run_kernels.py gemm|gemm_stg|gemm_push2|gemv|gemv4|gemv1k4|quant|dequant [reps]
     python profiles/run_kernels.py mm:M,K,N[:cfg] [reps]        # any fp8b_scaled_mm shape (AUTO dispatch), optional tile cfg
 """
 import ctypes
@@ -42,13 +42,11 @@ def main():
             rc = L.fp8b_scaled_mm_push(P(A), P(Bs[i % 4]), arr, 2, dt_code(torch.bfloat16), M, N, K, 2 * N, P(one), 1, P(one), 1,
                                        None, 0, None, st)
             assert rc == 0, rc
-    elif which in ("gemm", "gemm_stg", "gemv", "gemv4", "gemv1k4", "gemv_ring"):
+    elif which in ("gemm", "gemm_stg", "gemv", "gemv4", "gemv1k4"):
         M, K, N, algo = {"gemm": (4096, 3072, 12288, 2), "gemm_stg": (4096, 3072, 12288, 2), "gemv": (1, 14336, 4096, 1),
-                         "gemv4": (4, 4096, 4096, 1), "gemv1k4": (1, 4096, 4096, 1), "gemv_ring": (1, 14336, 4096, 1)}[which]
+                         "gemv4": (4, 4096, 4096, 1), "gemv1k4": (1, 4096, 4096, 1)}[which]
         if which == "gemm_stg":
             L.fp8b_set_option(20, 1)           # the round-1 st.global epilogue, for comparison
-        if which == "gemv_ring":
-            L.fp8b_set_option(17, 4)
         A = rand_u8(M, K)
         Bs = [rand_u8(N, K) for _ in range(4)]
         C = torch.empty(M, N, dtype=torch.bfloat16, device=dev)

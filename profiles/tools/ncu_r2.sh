@@ -14,7 +14,6 @@ cap gemm_push2 fp8_gemm_tcgen05 gemm_push2
 cap gemv fp8_gemv_kernel gemv
 cap gemv4 fp8_gemv_mma gemv4
 cap gemv1k4 fp8_gemv_kernel gemv1k4
-cap gemv_ring fp8_gemv_ring gemv_ring
 cap gemm_stg fp8_gemm_tcgen05 gemm_stg
 cap gemm_splitk fp8_gemm_splitk mm:32,3072,3072
 cap dequant fp8_to_wide dequant

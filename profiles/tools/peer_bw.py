@@ -79,7 +79,7 @@ for K in (64, 3072):
         out.append(f"GEMM+push K={K:4d} {name:14s}: {us:7.1f} us  {shard_bytes * (len(dsts) - (1 if name != 'peer only' else 0)) / us / 1e3:6.0f} GB/s to peers")
     us = timed(lambda: lin.local(a, sa, torch.bfloat16))
     out.append(f"GEMM K={K:4d} st.global epilogue, local shard: {us:7.1f} us")
-# the exchange path alone (K = 64, peer only) under the kernel's knobs: tile shape, tile order, box form
+# the exchange path alone (K = 64, peer only) under the kernel's knobs: tile shape, tile order
 K = 64
 g = torch.Generator(device=dev).manual_seed(3)
 a = torch.randint(0, 120, (M, K), dtype=torch.uint8, device=dev, generator=g)
@@ -92,14 +92,13 @@ order = lin._push_order(0, h2)
 lib = nat._get_lib()
 for cfg in (3, 4, 2):
     for raster in (1, 2):
-        for store in (4, 3):
-            lib.set_option(16, cfg); lib.set_option(24, raster); lib.set_option(20, store)
-            try:
-                us = timed(lambda: lib.fp8_scaled_mm_push(a, w, sa, sb, None, b2, order[1:2], int(n0)))
-                out.append(f"K=64 peer only cfg{cfg} raster{raster} store{store}: {us:7.1f} us {M * (n1 - n0) * 2 / us / 1e3:6.0f} GB/s")
-            except Exception as e:
-                out.append(f"K=64 cfg{cfg} raster{raster} store{store}: {str(e)[:80]}")
-lib.set_option(16, -1); lib.set_option(24, -1); lib.set_option(20, -1)
+        lib.set_option(16, cfg); lib.set_option(24, raster)
+        try:
+            us = timed(lambda: lib.fp8_scaled_mm_push(a, w, sa, sb, None, b2, order[1:2], int(n0)))
+            out.append(f"K=64 peer only cfg{cfg} raster{raster}: {us:7.1f} us {M * (n1 - n0) * 2 / us / 1e3:6.0f} GB/s")
+        except Exception as e:
+            out.append(f"K=64 cfg{cfg} raster{raster}: {str(e)[:80]}")
+lib.set_option(16, -1); lib.set_option(24, -1)
 # does the destination ROW PITCH matter (NVLink / memory address interleaving)?  Same K = 64 push into wider buffers.
 for pad in (0, 64, 128, 256, 320, 1024, 2048):
     wide_buf = symm_mem.empty((M, N + pad), dtype=torch.bfloat16, device=dev)

@@ -13,9 +13,7 @@ KERNELS = [
     ("gemm_tcgen05_256x256_pair", r"fp8_gemm_tcgen05_kernel<256, 2, 0>", [r"UTCQMMA", r"UTMALDG", r"LDTM", r"UTCBAR", r"STG\.E\.128"], 6),
     ("gemm_tcgen05_push_256x256_pair", r"fp8_gemm_tcgen05_kernel<256, 2, 2>", [r"UTMASTG", r"UTCQMMA", r"LDTM", r"STS\.128", r"UTMACMDFLUSH|DEPBAR|UTMACCTL"], 6),
     ("gemm_splitk_x4", r"fp8_gemm_splitk_kernel<4>", [r"UTCQMMA", r"UBLKCP|UBLKRED|UBLK", r"LDTM", r"UCGABAR", r"MAPA|UMAPA"], 5),
-    ("gemv_ring_m8", r"fp8_gemv_ring_kernel<1>", [r"UBLKCP", r"HMMA", r"SYNCS", r"LDS\.128"], 5),
     ("gemv_fhfma_m1", r"fp8_gemv_kernel<1, 4>", [r"FHFMA", r"LDG\.E\.128", r"ACQBULK|GRIDDEP"], 5),
-    ("dequant_tma_f16", r"fp8_to_wide_tma_kernel<1, false, 0>", [r"UBLKCP", r"F2FP", r"STS\.128", r"SYNCS"], 5),
     ("dequant_ldg_f16", r"fp8_to_wide_kernel<1, false, 512, 8, 0>", [r"F2FP", r"LDG", r"STG"], 4),
     ("encode_bf16", r"wide_to_fp8_kernel<2, false, 512, 4, 32>", [r"F2FP", r"LDG\.E\.(ENL2\.)?256|LDG", r"STG"], 4),
 ]

@@ -1,6 +1,7 @@
 #!/usr/bin/env python3
-"""One GPU: fp8 -> fp16 dequant variants (FP8B_OPT_TUNE_CAST_SHAPE 0 = LDG/STG kernel, 3 / 4 = TMA-pipelined kernel with
-1 / 2 CTAs per SM) on FLUX-shaped tensors, one launch per tensor, in one CUDA graph; bit-equality between variants.
+"""One GPU: fp8 -> wide dequant bandwidth of the default launch rule (FP8B_OPT_TUNE_CAST_SHAPE = -1) on FLUX-shaped
+tensors, one launch per tensor, in one CUDA graph.  With the profiling library, CAST_SWEEP=11,12,... adds the fp16
+launch-shape sweep (CAST_SHAPE 11..19) and checks it bit-equal to the default.
     python profiles/tools/time_cast.py"""
 import ctypes, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -18,14 +19,13 @@ for _ in range(12):
     sizes += [r * c for r, c in SINGLE]
 total = sum(sizes)
 q = torch.randint(0, 256, (total,), dtype=torch.uint8, device=dev)
-outs = {m: torch.empty(total, dtype=torch.float16, device=dev) for m in (0, 3, 4)}
 offs = [0]
 for s in sizes: offs.append(offs[-1] + s)
 print(f"{len(sizes)} tensors, {total/1e9:.2f} G elements, {3*total/1e9:.1f} GB traffic per sweep", flush=True)
 SWEEP = [int(x) for x in os.environ.get("CAST_SWEEP", "").split(",") if x]      # profiling library only: modes 11..19
 for out_dt, code, esz in ((torch.float16, 1, 2), (torch.bfloat16, 2, 2), (torch.float32, 0, 4)):
     res = {}
-    modes = (0, 3, 4) + (tuple(SWEEP) if out_dt == torch.float16 else ())
+    modes = (0,) + (tuple(SWEEP) if out_dt == torch.float16 else ())
     for mode in modes:
         h = torch.empty(total, dtype=out_dt, device=dev)
         L.fp8b_set_option(19, mode if mode else -1)
@@ -56,7 +56,7 @@ for n in (1 << 30, 50_000_017):
     qq = q[:n]
     line = []
     ref = None
-    for mode in (0, 3, 4):
+    for mode in (0,) + tuple(SWEEP):
         L.fp8b_set_option(19, mode if mode else -1)
         h = torch.empty(n, dtype=torch.float16, device=dev)
         sp = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)

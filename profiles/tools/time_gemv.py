@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """One GPU: the GEMV configs (C1, C2, C3, the reference's square shape) with every kernel variant
-(FP8B_OPT_TUNE_GEMV_IMPL 0 = dispatch rule, 1 = FHFMA, 2 = warp-MMA, 4 = persistent TMA ring), HBM-cold rotation in one
+(FP8B_OPT_TUNE_GEMV_IMPL 0 = dispatch rule, 1 = FHFMA, 2 = warp-MMA), HBM-cold rotation in one
 CUDA graph, default PDL; plus the static-weights option.   python profiles/tools/time_gemv.py"""
 import ctypes, os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -27,10 +27,9 @@ for name, M, K, N, odt, nbytes, rot in CFG:
                                   None, None, 0, 1, st)
             assert rc == 0, rc
     res = []
-    for impl in (0, 1, 2, 4, 42):
+    for impl in (0, 1, 2):
         for static in (0, 1):
-            L.fp8b_set_option(17, (impl if impl < 10 else 4) if impl else -1); L.fp8b_set_option(1, static)
-            L.fp8b_set_option(21, 2 if impl == 42 else -1)              # ring kernel: two half-size rings per SM
+            L.fp8b_set_option(17, impl if impl else -1); L.fp8b_set_option(1, static)
             try:
                 for _ in range(2): run()
                 torch.cuda.synchronize()
@@ -49,7 +48,7 @@ for name, M, K, N, odt, nbytes, rot in CFG:
                 res.append(f"impl{impl}{'s' if static else ' '} {best:6.2f} us {nbytes / best / 1e3:5.0f} GB/s")
             except Exception as e:
                 res.append(f"impl{impl}{'s' if static else ' '} ERR {str(e)[:40]}")
-    L.fp8b_set_option(17, -1); L.fp8b_set_option(1, 0); L.fp8b_set_option(21, -1)
+    L.fp8b_set_option(17, -1); L.fp8b_set_option(1, 0)
     print(f"{name:3s} M{M} K{K} N{N}: " + " | ".join(res), flush=True)
     del Ws
     torch.cuda.empty_cache()

@@ -42,25 +42,6 @@ for cfg in [int(c) for c in os.environ.get("CFGS", "").split(",") if c]:
                 nat._get_lib().set_option(16, -1)
         return run
     variants[f"push_cfg{cfg}"] = mk(cfg)
-for st_name, st_val in (("push_box128", 4), ("push_wide", 3)):
-    def mk2(v):
-        def run():
-            nat._get_lib().set_option(20, v)
-            try:
-                lin(a, sa, torch.bfloat16, mode="push")
-            finally:
-                nat._get_lib().set_option(20, -1)
-        return run
-    variants[st_name] = mk2(st_val)
-    def mk3(v):
-        def run():
-            nat._get_lib().set_option(20, v)
-            try:
-                push_kernel_only()
-            finally:
-                nat._get_lib().set_option(20, -1)
-        return run
-    variants[st_name + "_kernel_only"] = mk3(st_val)
 def mk_raster(v, kernel_only):
     def run():
         nat._get_lib().set_option(24, v)
@@ -108,14 +89,10 @@ for name, fn in variants.items():
         out[name] = repr(e)[:120]
 # parity of the push plan against the all-gather of the same shards
 try:
-    nat._get_lib().set_option(20, 3)
-    y_wide = lin(a, sa, torch.bfloat16, mode="push").clone()
-    nat._get_lib().set_option(20, -1)
     y_push = lin(a, sa, torch.bfloat16, mode="push").clone()
     y_ag = lin(a, sa, torch.bfloat16, layout="row_major")
     torch.cuda.synchronize()
     out["push==allgather"] = bool(torch.equal(y_push, y_ag))
-    out["push_wide==allgather"] = bool(torch.equal(y_wide, y_ag))
 except Exception as e:
     out["push==allgather"] = repr(e)[:200]
 if rank == 0:

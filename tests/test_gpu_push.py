@@ -68,8 +68,9 @@ def _case(M, K, N, odt, n_dst=1, ldc=None, n0=0, per_row=False, bias_dt=None, sc
 ])
 @pytest.mark.parametrize("store", [4, 3])
 def test_push_matches_direct_and_oracle(tune, store, M, K, N, odt, kw):
-    """store = 4: 128B-swizzled boxes of 128-byte rows; store = 3: one linear box per tile, 256- / 512-byte rows
-    (16-bit outputs; fp32 keeps the 128-byte form) -- FP8B_OPT_TUNE_GEMM_STORE."""
+    """FP8B_OPT_TUNE_GEMM_STORE = 4 / 3 once chose between two push epilogues; either value must still give the one push
+    epilogue.  Either also makes the direct kernel of _case store with st.global, not with the TMA-store epilogue the
+    push path uses."""
     tune("GEMM_STORE", store)
     _case(M, K, N, odt, seed=M + K + N, **kw)
 
@@ -77,7 +78,8 @@ def test_push_matches_direct_and_oracle(tune, store, M, K, N, odt, kw):
 @pytest.mark.parametrize("cfg", [1, 2, 3, 4, 5])
 @pytest.mark.parametrize("store", [4, 3])
 def test_push_all_tile_configs(tune, cfg, store):
-    """Every tile configuration (FP8B_OPT_TUNE_GEMM_CFG) with both store-ring epilogues."""
+    """Every tile configuration (FP8B_OPT_TUNE_GEMM_CFG), with both former push-epilogue values of GEMM_STORE (see
+    test_push_matches_direct_and_oracle)."""
     tune("GEMM_CFG", cfg)
     tune("GEMM_STORE", store)
     _case(640, 512, 1000, torch.bfloat16, n_dst=2, ldc=2000, n0=1000, per_row=True, bias_dt=torch.bfloat16, seed=11)
@@ -131,9 +133,10 @@ def test_push_rejects_unaligned():
 
 @pytest.mark.parametrize("store", [4, 3])
 def test_push_ragged_column_block(tune, store):
-    """A column block whose rows end on a 16-byte boundary but not on a box boundary: the tensor map clips the last box
-    in both store forms.  A block that does not end on 16 bytes is refused (TMA stores move 16-byte units and would
-    write past column N) -- and plain fp8b_scaled_mm, whose default epilogue is the TMA store, falls back to st.global."""
+    """A column block whose rows end on a 16-byte boundary but not on a box boundary: the tensor map clips the last box,
+    with both former push-epilogue values of GEMM_STORE.  A block that does not end on 16 bytes is refused (TMA stores
+    move 16-byte units and would write past column N) -- and plain fp8b_scaled_mm, whose default epilogue is the TMA
+    store, falls back to st.global."""
     tune("GEMM_STORE", store)
     _case(300, 256, 328, torch.bfloat16, n_dst=2, ldc=1000, n0=8, per_row=True, seed=3)
     M, K, N = 130, 64, 333

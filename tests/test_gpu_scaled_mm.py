@@ -116,31 +116,24 @@ def test_gemv_both_kernels(tune, impl, M, K, N, odt, kw):
     _run_case(M, K, N, odt, ALGO_GEMV, seed=impl + M + K + N, **kw)
 
 
-@pytest.mark.parametrize("K,N,odt,kw", [
-    (14336, 4096, torch.bfloat16, {}),
-    (4096, 4096, torch.float16, {"per_row_b": True, "bias_dtype": torch.float16}),
-    (512, 300, None, {}),                       # 2 vectors per warp, ragged rows per CTA
-    (30000, 1000, None, {"scale_result": True}),  # K % 512 != 0, 4 vectors per lane
-    (16, 2000, None, {}),
-])
-def test_gemv_rows_kernel(tune, K, N, odt, kw):
-    """FP8B_GEMV_IMPL=3: the SM-balanced persistent M=1 kernel (falls back to the warp-per-row kernel
-    where it does not apply, e.g. N < 2 x SM count)."""
-    tune("GEMV_IMPL", 3)
-    _run_case(1, K, N, odt, ALGO_GEMV, seed=K + N, **kw)
-
-
-def test_gemv_rows_nan_bytes(tune):
-    tune("GEMV_IMPL", 3)
-    rng = np.random.default_rng(3)
-    A = rng.integers(0, 256, (1, 2048), dtype=np.uint8)
-    B = rng.integers(0, 256, (600, 2048), dtype=np.uint8)
-    A[0, 5] = 0x7F
-    sa = np.array([0.5], np.float32)
-    sb = np.array([0.25], np.float32)
-    rc, C = mm_capi(torch.from_numpy(A).to(DEV), torch.from_numpy(B).to(DEV), torch.from_numpy(sa), torch.from_numpy(sb))
+@pytest.mark.parametrize("impl", [3, 4])
+@pytest.mark.parametrize("M", [1, 4, 16])
+def test_gemv_retired_impl_values_take_the_built_in_rule(tune, impl, M):
+    """FP8B_GEMV_IMPL = 3 / 4 selected two GEMV kernels that measured slower and were removed (DESIGN.md 3.2, 3.3b).
+    Such a value must still work: one launch, bit-identical to the built-in rule."""
+    A = torch.from_numpy(_rand_fp8((M, 2048), 5)).to(DEV)
+    B = torch.from_numpy(_rand_fp8((1000, 2048), 6)).to(DEV)
+    s = torch.tensor([0.01], device=DEV)
+    rc, ref = mm_capi(A, B, s, s, algo=ALGO_GEMV)
     assert rc == 0
-    _check(C, o.scaled_mm(A, B, sa, sb), None, what="rows nan bytes")
+    tune("GEMV_IMPL", impl)
+    L = capi()
+    n0 = L.fp8b_launch_count()
+    rc, out = mm_capi(A, B, s, s, algo=ALGO_GEMV)
+    assert rc == 0
+    assert L.fp8b_launch_count() == n0 + 1
+    torch.cuda.synchronize()
+    assert torch.equal(out, ref)
 
 
 def test_gemv_mma_nan_bytes(tune):
@@ -153,77 +146,6 @@ def test_gemv_mma_nan_bytes(tune):
     rc, C = mm_capi(torch.from_numpy(A).to(DEV), torch.from_numpy(B).to(DEV), torch.from_numpy(sa), torch.from_numpy(sb))
     assert rc == 0
     _check(C, o.scaled_mm(A, B, sa, sb), None, what="mma nan bytes")
-
-
-@pytest.mark.parametrize("M,K,N,odt,kw", [
-    (1, 4096, 4096, torch.float16, {}),                        # BASELINE config 1
-    (1, 14336, 4096, torch.bfloat16, {}),                      # BASELINE config 2
-    (4, 4096, 4096, torch.bfloat16, {"bias_dtype": torch.bfloat16}),   # BASELINE config 3
-    (1, 14336, 14336, None, {}),                               # the reference's own benchmark shape (test_fp8_metal.py:232)
-    (2, 4160, 1184, None, {"per_row_a": True, "per_row_b": True}),     # minimum N (8 rows per SM), K = 65 chunks
-    (8, 2048, 5001, torch.float16, {"per_row_a": True, "bias_dtype": torch.float32, "scale_result": True}),  # ragged N
-    (9, 1024, 3000, None, {"per_row_a": True}),                # two activation tiles (M > 8)
-    (16, 2048, 2400, torch.bfloat16, {"per_row_b": True, "bias_dtype": torch.bfloat16}),   # largest x: 64 KB of fp16 in shared memory
-    (3, 64, 1500, None, {}),                                   # one 64-byte chunk
-    (1, 28672, 2000, None, {}),                                # 14 K-segments per row tile
-    (5, 6208, 4096, None, {"scale_result": True}),             # K = 97 chunks: uneven last segment
-])
-def test_gemv_ring_kernel(tune, M, K, N, odt, kw):
-    """FP8B_OPT_TUNE_GEMV_IMPL = 4: the persistent TMA-ring warp-MMA kernel (csrc/fp8_gemv_ring.cu), M = 1..16."""
-    tune("GEMV_IMPL", 4)
-    L = capi()
-    n0 = L.fp8b_launch_count()
-    _run_case(M, K, N, odt, ALGO_GEMV, seed=4 + M + K + N, **kw)
-    assert L.fp8b_launch_count() == n0 + 1                     # one launch: it really was the ring kernel
-
-
-def test_gemv_ring_nan_bytes_and_static_weights(tune):
-    import fp8_mps_native
-    tune("GEMV_IMPL", 4)
-    rng = np.random.default_rng(9)
-    A = rng.integers(0, 256, (3, 1024), dtype=np.uint8)
-    B = rng.integers(0, 256, (1500, 1024), dtype=np.uint8)
-    A[1, 5] = 0x7F; B[77, 0] = 0xFF
-    sa = np.array([0.5], np.float32)
-    sb = np.array([0.25], np.float32)
-    tA, tB = torch.from_numpy(A).to(DEV), torch.from_numpy(B).to(DEV)
-    rc, C = mm_capi(tA, tB, torch.from_numpy(sa), torch.from_numpy(sb))
-    assert rc == 0
-    ref = o.scaled_mm(A, B, sa, sb)
-    _check(C, ref, None, what="ring nan bytes")
-    fp8_mps_native.set_static_weights(True)                    # producer streams B before griddepcontrol.wait
-    try:
-        buf = torch.empty_like(tA)
-        outs, refs = [], []
-        for it in range(16):
-            buf.copy_(torch.roll(tA, it, dims=1))              # predecessor writes the activations
-            outs.append(mm_capi(buf, tB, torch.from_numpy(sa), torch.from_numpy(sb))[1])
-            refs.append(o.scaled_mm(np.roll(A, it, axis=1), B, sa, sb))
-        torch.cuda.synchronize()
-    finally:
-        fp8_mps_native.set_static_weights(False)
-    for it in range(16):
-        _check(outs[it], refs[it], None, what=f"ring static weights, iteration {it}")
-
-
-def test_gemv_ring_chain_sees_fresh_activations(tune):
-    """PDL hazard for the ring kernel: x is written by the kernel just before each call (same address every time)."""
-    tune("GEMV_IMPL", 4)
-    K, N = 4096, 2048
-    W = torch.from_numpy(_rand_fp8((N, K), 3)).to(DEV)
-    base = torch.from_numpy(_rand_fp8((2, K), 4)).to(DEV)
-    sa = torch.tensor([0.5], device=DEV); sb = torch.tensor([0.02], device=DEV)
-    buf = torch.empty_like(base)
-    outs = []
-    for it in range(32):
-        buf.copy_(torch.roll(base, it, dims=1))
-        outs.append(mm_capi(buf, W, sa, sb)[1])
-    torch.cuda.synchronize()
-    tune("GEMV_IMPL", 2)
-    for it in range(32):
-        ref = mm_capi(torch.roll(base, it, dims=1).contiguous(), W, sa, sb)[1]
-        torch.cuda.synchronize()
-        assert o.rel_rmse(to_np(outs[it]), to_np(ref)) <= 5e-6, f"iteration {it}"
 
 
 def test_gemv_matches_reference_summation_to_fp32_noise():
