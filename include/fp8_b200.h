@@ -221,6 +221,10 @@ FP8B_API int fp8b_quantize_rows(const void* in, int in_dtype, int rows, size_t c
  *                FP8B_ERR_UNSUPPORTED (no re-dispatch).
  *
  * NaN bytes (0x7F/0xFF) in A or B contribute 0, as in the reference (fp8_matmul.metal:21).
+ *
+ * Degenerate extents: M == 0 or N == 0 returns FP8B_OK and launches nothing.  K == 0 is a valid problem whose sum
+ * is 0, so C = cast_out(((0 * sa) * sb [+ bias]) [* scale_result]); AUTO, GEMV (M <= 16) and SIMT serve it,
+ * TCGEN05 needs K >= 16 and returns FP8B_ERR_UNSUPPORTED without touching C.
  */
 FP8B_API int fp8b_scaled_mm(const uint8_t* A, const uint8_t* B, void* C, int out_dtype,
                    int M, int N, int K, int64_t ldc,
@@ -282,6 +286,8 @@ FP8B_API int fp8b_scaled_mm_fmt(const uint8_t* A, int a_format, const uint8_t* B
  *                              aligned X and B, else FP8B_ERR_UNSUPPORTED.  Same result bits as the chained plan.
  *   M  > 16                  : workspace required (FP8B_ERR_UNSUPPORTED without); quantise kernel, then the GEMM
  *                              fp8b_scaled_mm would pick, with per-row scale_a.
+ * K == 0: the workspace plans serve it (every row has amax 0, so its scale is 1.0 and its sum 0); without a workspace
+ * it is FP8B_ERR_UNSUPPORTED.
  */
 FP8B_API int fp8b_linear_dynamic(const void* X, int x_dtype, const uint8_t* B, void* C, int out_dtype,
                       int M, int N, int K, int64_t ldc,
