@@ -183,6 +183,13 @@ FP8B_API int fp8b_dequant_batch(const fp8b_span* spans, int count, int out_dtype
  *     scale_out[0]     = (float)scale_d                         (what fp8b_encode takes as prescale)
  *     inv_scale_out[0] = (float)(1.0 / scale_d)                 (what fp8_quantize returns)
  * scratch: device pointer to one uint32 the call may clobber (it is reset by the call itself).
+ * Special amax values give (here, in fp8b_quantize_rows and in fp8b_linear_dynamic, per row):
+ *     n == 0 or amax == 0       : scale 1, inv 1
+ *     amax NaN (a NaN input)    : amax > 0 fails, so scale 1, inv 1; NaN inputs encode to 0x7F
+ *     amax +inf (an inf input)  : scale 0, inv = (float)(1.0/0.0) = +inf (the reference raises ZeroDivisionError);
+ *                                 finite inputs encode to 0x00, +-inf to 0x7F (inf * 0 = NaN)
+ *     amax < A* ~= 1.3166e-36   : (float)scale_d overflows to +inf, inv is a subnormal or 0; zeros encode to 0x7F
+ *                                 (0 * inf = NaN), nonzeros to 0x7E / 0xFE
  */
 FP8B_API int fp8b_amax_scale(const void* in, int in_dtype, size_t n, float* scale_out, float* inv_scale_out,
                     uint32_t* scratch, void* stream);
@@ -193,6 +200,7 @@ FP8B_API int fp8b_amax_scale(const void* in, int in_dtype, size_t n, float* scal
  *     amax_r = max_j |f32(in[r,j])|;  scale_r = amax_r > 0 ? 448.0/amax_r : 1.0 (double)
  *     out[r,j] = enc( f32(in[r,j]) * (float)scale_r );   inv_scale_out[r] = (float)(1.0/scale_r)
  * inv_scale_out (device float[rows]) is what fp8b_scaled_mm takes as a per-row scale_a / scale_b.
+ * NaN, inf and tiny amax values give the results listed at fp8b_amax_scale, row by row.
  * (The reference only quantises per tensor; its kernels accept per-row scales, fp8_matmul.metal:144-145.)
  */
 FP8B_API int fp8b_quantize_rows(const void* in, int in_dtype, int rows, size_t cols, uint8_t* out,
@@ -277,6 +285,9 @@ FP8B_API int fp8b_scaled_mm_fmt(const uint8_t* A, int a_format, const uint8_t* B
  * X is (M,K) float32 / float16 / bfloat16, contiguous.  For M == 1 this is exactly the reference composition
  * fp8_quantize(x) then torch._scaled_mm(x8, w8.t(), scale_a=inv, ...); for M > 1 each row gets its own scale
  * (= fp8b_quantize_rows).  inv_scale_a_out (device float[M], nullable) receives the row scales.
+ * Special rows follow fp8b_amax_scale: a NaN amax gives inv_m = 1; an infinite amax gives inv_m = +inf, so that row of C
+ * is NaN (every q is 0x00 or 0x7F, which decodes to 0, and 0 * inf = NaN); an amax below A* gives q = 0x7E / 0xFE
+ * (zeros 0x7F) and a subnormal or zero inv_m.
  *
  * workspace: device, 16-byte aligned, >= fp8b_linear_dynamic_workspace_bytes(M,K).
  *   M <= 16, workspace given : rows quantised once by a one-CTA-per-row kernel, the GEMV chained behind it with

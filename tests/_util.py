@@ -4,6 +4,7 @@ import os
 import re
 
 import numpy as np
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "fp8-mps-metal_b200")
@@ -14,6 +15,12 @@ F32, F16, BF16 = 0, 1, 2
 ALGO_AUTO, ALGO_GEMV, ALGO_TCGEN05, ALGO_SIMT = 0, 1, 2, 3
 
 _lib = None
+
+DEV = "cuda"
+GUARD_ROWS = 3
+SENT = {torch.float32: 0x7FA5A5A5, torch.float16: 0x7DA5, torch.bfloat16: 0x7FA5}    # NaN payloads no kernel writes
+_INT = {torch.float32: torch.int32, torch.float16: torch.int16, torch.bfloat16: torch.int16}
+BIG_SCALE = 1024.0                                    # what sits behind per-row scales
 
 
 def declared_symbols():
@@ -171,3 +178,59 @@ def to_np(t):
 def u8_np(t):
     import torch
     return t.detach().view(torch.uint8).cpu().numpy()
+
+
+# ------------------------------------------------------------------ device buffers with guard bands
+
+class Out:
+    """C as an interior view of a sentinel-filled buffer: GUARD_ROWS rows above and below, `cl` columns left and at
+    least 8 right.  aligned=True keeps the view 16-byte aligned with ldc * esz % 16 == 0 (the vector / TMA store
+    paths); False shifts it by one element and makes ldc odd (the scalar store paths)."""
+
+    def __init__(self, M, N, dtype, aligned=True, cl=None):
+        esz = torch.empty(0, dtype=dtype).element_size()
+        self.dtype, self.M, self.N = dtype, M, N
+        self.cl = (16 // esz if aligned else 1) if cl is None else cl
+        ldc = self.cl + N + 8
+        if aligned:
+            ldc += (-ldc * esz) % 16 // esz
+        elif ldc % 2 == 0:
+            ldc += 1
+        self.ldc = ldc
+        self.buf = torch.full((M + 2 * GUARD_ROWS, ldc), SENT[dtype], dtype=_INT[dtype], device=DEV).view(dtype)
+        self.view = self.buf[GUARD_ROWS:GUARD_ROWS + M, self.cl:self.cl + N]
+
+    @property
+    def ptr(self):
+        return self.buf.data_ptr() + (GUARD_ROWS * self.ldc + self.cl) * self.buf.element_size()
+
+    def check_guard(self, what, interior_written=True):
+        raw = self.buf.view(_INT[self.dtype]).clone()
+        if interior_written:
+            raw[GUARD_ROWS:GUARD_ROWS + self.M, self.cl:self.cl + self.N] = SENT[self.dtype]
+        bad = (raw != SENT[self.dtype]).nonzero()
+        assert bad.numel() == 0, f"{what}: {bad.shape[0]} elements written outside C, first at buffer {bad[0].tolist()} " \
+                                 f"(C = rows [{GUARD_ROWS}, {GUARD_ROWS + self.M}), cols [{self.cl}, {self.cl + self.N}))"
+
+
+def dev_f32(v, big=BIG_SCALE, extra=8):
+    v = np.asarray(v, np.float32).reshape(-1)
+    return torch.from_numpy(np.concatenate([v, np.full(extra, big, np.float32)])).to(DEV)
+
+
+# ------------------------------------------------------------------ exact comparison
+
+def assert_bits_equal(got, ref, what, any_nan=False):
+    """float32 arrays holding values of the output dtype: equal bit patterns, with +0 == -0.  any_nan: a NaN matches
+    a NaN of any sign and payload."""
+    g = (np.asarray(got, np.float32) + np.float32(0.0)).view(np.uint32)
+    r = (np.asarray(ref, np.float32) + np.float32(0.0)).view(np.uint32)
+    assert g.shape == r.shape
+    if any_nan:
+        nan = np.isnan(np.asarray(ref, np.float32))
+        g, r = np.where(nan & np.isnan(np.asarray(got, np.float32)), 0x7FC00000, g), np.where(nan, 0x7FC00000, r)
+    if not np.array_equal(g, r):
+        bad = np.argwhere(g != r)
+        i = tuple(bad[0])
+        raise AssertionError(f"{what}: {len(bad)} of {g.size} outputs differ from the exact result; first at {list(i)}: "
+                             f"got {got[i]!r} want {ref[i]!r}")

@@ -167,11 +167,16 @@ def test_quantize_golden_and_random(golden):
 
 @pytest.mark.parametrize("rows,cols,dtype", [(7, 1000, torch.float32), (64, 4096, torch.bfloat16), (3, 17, torch.float16),
                                              (12288, 3072, torch.bfloat16), (5, 8, torch.float32), (1, 1, torch.float32),
-                                             # register-resident kernel: warp-per-row with 2/4/8/16 vectors per lane,
-                                             # CTA-per-row with 4/8 per thread; then the two-pass kernel again
+                                             # register-resident kernel, few rows: a CTA per row with 1/2/4/8 vectors per
+                                             # thread; then the two-pass kernel again
                                              (19, 64, torch.bfloat16), (9, 1000, torch.float16), (33, 2048, torch.bfloat16),
                                              (21, 2048, torch.float32), (10, 8192, torch.bfloat16), (16, 14336, torch.bfloat16),
-                                             (5, 8192, torch.float32), (4, 20000, torch.bfloat16), (6, 1004, torch.bfloat16)])
+                                             (5, 8192, torch.float32), (4, 20000, torch.bfloat16), (6, 1004, torch.bfloat16),
+                                             # >= 32 rows per SM (4736 on 148 SMs): 2 or 4 vectors per thread and 32 / 32 /
+                                             # 64 / 128 threads per row, several rows per CTA, a partial last CTA
+                                             (4801, 256, torch.float32), (4801, 500, torch.float32), (4801, 1024, torch.float32),
+                                             (4801, 2048, torch.float32), (4801, 512, torch.float16), (4801, 1000, torch.float16),
+                                             (4801, 2048, torch.float16), (4801, 4096, torch.float16)])
 def test_quantize_rowwise(rows, cols, dtype):
     """Per-row quantise == the reference's fp8_quantize arithmetic applied row by row (oracle), bit for bit,
     and its inverse scales feed _scaled_mm as per-row scales."""

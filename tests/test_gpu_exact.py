@@ -31,7 +31,8 @@ import pytest
 import torch
 
 import fp8_oracle as o
-from _util import ALGO_AUTO, ALGO_GEMV, ALGO_SIMT, ALGO_TCGEN05, GemvItem, capi, dt_code, dt_name, p, stream_ptr, to_np
+from _util import (ALGO_AUTO, ALGO_GEMV, ALGO_SIMT, ALGO_TCGEN05, SENT, GemvItem, Out, assert_bits_equal, capi, dev_f32, dt_code,
+                   dt_name, p, stream_ptr, to_np)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -39,44 +40,10 @@ OPT_PDL, OPT_STATIC_WEIGHTS = 0, 1
 E4M3, E5M2 = 0, 1
 ODTS = (torch.float32, torch.float16, torch.bfloat16)
 
-_INT = {torch.float32: torch.int32, torch.float16: torch.int16, torch.bfloat16: torch.int16}
-_SENT = {torch.float32: 0x7FA5A5A5, torch.float16: 0x7DA5, torch.bfloat16: 0x7FA5}    # NaN payloads no kernel writes
-_GUARD_ROWS = 3
-BIG_SCALE, BIG_BIAS = 1024.0, 30000.0                 # what sits behind per-row scales / biases
+BIG_BIAS = 30000.0                                    # what sits behind per-row biases
 
 
 # ------------------------------------------------------------------ device buffers with guard bands
-
-class Out:
-    """C as an interior view of a sentinel-filled buffer: _GUARD_ROWS rows above and below, `cl` columns left and at
-    least 8 right.  aligned=True keeps the view 16-byte aligned with ldc * esz % 16 == 0 (the vector / TMA store
-    paths); False shifts it by one element and makes ldc odd (the scalar store paths)."""
-
-    def __init__(self, M, N, dtype, aligned=True, cl=None):
-        esz = torch.empty(0, dtype=dtype).element_size()
-        self.dtype, self.M, self.N = dtype, M, N
-        self.cl = (16 // esz if aligned else 1) if cl is None else cl
-        ldc = self.cl + N + 8
-        if aligned:
-            ldc += (-ldc * esz) % 16 // esz
-        elif ldc % 2 == 0:
-            ldc += 1
-        self.ldc = ldc
-        self.buf = torch.full((M + 2 * _GUARD_ROWS, ldc), _SENT[dtype], dtype=_INT[dtype], device=DEV).view(dtype)
-        self.view = self.buf[_GUARD_ROWS:_GUARD_ROWS + M, self.cl:self.cl + N]
-
-    @property
-    def ptr(self):
-        return self.buf.data_ptr() + (_GUARD_ROWS * self.ldc + self.cl) * self.buf.element_size()
-
-    def check_guard(self, what, interior_written=True):
-        raw = self.buf.view(_INT[self.dtype]).clone()
-        if interior_written:
-            raw[_GUARD_ROWS:_GUARD_ROWS + self.M, self.cl:self.cl + self.N] = _SENT[self.dtype]
-        bad = (raw != _SENT[self.dtype]).nonzero()
-        assert bad.numel() == 0, f"{what}: {bad.shape[0]} elements written outside C, first at buffer {bad[0].tolist()} " \
-                                 f"(C = rows [{_GUARD_ROWS}, {_GUARD_ROWS + self.M}), cols [{self.cl}, {self.cl + self.N}))"
-
 
 def dev_bytes(X, offset=0, guard_rows=2):
     """uint8 rows of X, then guard rows of 0x7E, starting `offset` bytes into the allocation -> (tensor, pointer)."""
@@ -87,29 +54,10 @@ def dev_bytes(X, offset=0, guard_rows=2):
     return t, t.data_ptr() + offset
 
 
-def dev_f32(v, big=BIG_SCALE, extra=8):
-    v = np.asarray(v, np.float32).reshape(-1)
-    return torch.from_numpy(np.concatenate([v, np.full(extra, big, np.float32)])).to(DEV)
-
-
 def dev_bias(v, dtype, extra=8):
     """bias of `dtype` followed by large finite values -> (tensor, the fp32 values the kernel reads)."""
     t = torch.from_numpy(np.concatenate([np.asarray(v, np.float32), np.full(extra, BIG_BIAS, np.float32)])).to(DEV).to(dtype)
     return t, to_np(t[:len(v)])
-
-
-# ------------------------------------------------------------------ exact comparison
-
-def assert_bits_equal(got, ref, what):
-    """float32 arrays holding values of the output dtype: equal bit patterns, with +0 == -0."""
-    g = (np.asarray(got, np.float32) + np.float32(0.0)).view(np.uint32)
-    r = (np.asarray(ref, np.float32) + np.float32(0.0)).view(np.uint32)
-    assert g.shape == r.shape
-    if not np.array_equal(g, r):
-        bad = np.argwhere(g != r)
-        i = tuple(bad[0])
-        raise AssertionError(f"{what}: {len(bad)} of {g.size} outputs differ from the exact result; first at {list(i)}: "
-                             f"got {got[i]!r} want {ref[i]!r}")
 
 
 def _decode(X, fmt):
@@ -585,7 +533,7 @@ def test_linear_dynamic_exact(tune, M, plan, ws, xdt):
     odt = ODTS[(M + plan) % 3]
     t = Terms.cycle(M + plan, 1, N, rng).device()
     out = Out(M, N, odt)
-    inv = torch.full((M + 8,), _SENT[torch.float32], dtype=torch.int32, device=DEV).view(torch.float32)
+    inv = torch.full((M + 8,), SENT[torch.float32], dtype=torch.int32, device=DEV).view(torch.float32)
     L = capi()
     need = L.fp8b_linear_dynamic_workspace_bytes(M, K)
     wsb = torch.empty(need + 16, dtype=torch.uint8, device=DEV) if ws else None
@@ -599,7 +547,7 @@ def test_linear_dynamic_exact(tune, M, plan, ws, xdt):
     q, inv_ref = np.stack(qs), np.concatenate(invs)
     assert set(np.unique(q).tolist()) <= {0x00, 0x7E, 0xFE}
     assert np.array_equal(inv[:M].cpu().numpy().view(np.uint32), inv_ref.view(np.uint32)), what
-    assert (inv[M:].view(torch.int32) == _SENT[torch.float32]).all(), f"{what}: written past inv_scale_a_out[M]"
+    assert (inv[M:].view(torch.int32) == SENT[torch.float32]).all(), f"{what}: written past inv_scale_a_out[M]"
     out.check_guard(what)
     assert_bits_equal(to_np(out.view), oracle(q, B, inv_ref, t.sb, t.bias, t.sr, odt), what)
 
@@ -632,7 +580,7 @@ def test_zero_k(M):
     bc = dt_code(t.bias_dt) if t.bias_dt is not None else 0
     for ws in (True, False):
         out = Out(M, N, torch.float32)
-        inv = torch.full((M + 8,), _SENT[torch.float32], dtype=torch.int32, device=DEV).view(torch.float32)
+        inv = torch.full((M + 8,), SENT[torch.float32], dtype=torch.int32, device=DEV).view(torch.float32)
         wsb = torch.empty(64, dtype=torch.uint8, device=DEV)
         rc = L.fp8b_linear_dynamic(X.data_ptr(), dt_code(torch.bfloat16), pB, out.ptr, 0, M, N, 0, out.ldc, p(t.t_sb), len(t.sb),
                                    p(t.t_bias), bc, p(t.t_sr), inv.data_ptr(), p(wsb) if ws else None, 64 if ws else 0, stream_ptr())
@@ -640,7 +588,7 @@ def test_zero_k(M):
         if ws:
             assert rc == 0
             out.check_guard("dynamic K = 0")
-            assert (inv[:M] == 1.0).all() and (inv[M:].view(torch.int32) == _SENT[torch.float32]).all()
+            assert (inv[:M] == 1.0).all() and (inv[M:].view(torch.int32) == SENT[torch.float32]).all()
             assert_bits_equal(to_np(out.view), _zero_k_expect(M, N, Terms_with(t, np.ones(M, np.float32)), torch.float32), "dynamic K = 0")
         else:
             assert rc == -2
@@ -720,14 +668,14 @@ def test_unit_sizes_dynamic_and_batch(ws):
     X[0, 9] = -0.3
     tX = X.to(DEV)
     out = Out(1, 1, torch.float32)
-    inv = torch.full((9,), _SENT[torch.float32], dtype=torch.int32, device=DEV).view(torch.float32)
+    inv = torch.full((9,), SENT[torch.float32], dtype=torch.int32, device=DEV).view(torch.float32)
     wsb = torch.empty(64, dtype=torch.uint8, device=DEV) if ws else None
     rc = L.fp8b_linear_dynamic(tX.data_ptr(), 0, pB, out.ptr, 0, 1, 1, 16, out.ldc, p(t.t_sb), 1, p(t.t_bias), bc, p(t.t_sr),
                                inv.data_ptr(), p(wsb), 64 if ws else 0, stream_ptr())
     torch.cuda.synchronize()
     assert rc == 0
     q, inv_ref = o.fp8_quantize(X[0].numpy())
-    assert inv[0].item() == inv_ref[0] and (inv[1:].view(torch.int32) == _SENT[torch.float32]).all()
+    assert inv[0].item() == inv_ref[0] and (inv[1:].view(torch.int32) == SENT[torch.float32]).all()
     out.check_guard("dynamic unit")
     assert_bits_equal(to_np(out.view), oracle(q[None], B, inv_ref, t.sb, t.bias, t.sr, torch.float32), "dynamic unit")
     x = one_hot(1, 16, np.array([15 if ws else 0]), rng)
@@ -778,7 +726,7 @@ def test_tcgen05_output_past_2_31_elements(tune, store):
     sa, sb = np.float32(0.0123 * 1.37), np.float32(0.0217 * 0.91)
     tsa, tsb = dev_f32([sa]), dev_f32([sb])
     bias = torch.from_numpy((rng.standard_normal(N) * 0.7).astype(np.float32)).to(DEV)
-    C = torch.full((M + 2, ldc), _SENT[torch.bfloat16], dtype=torch.int16, device=DEV).view(torch.bfloat16)
+    C = torch.full((M + 2, ldc), SENT[torch.bfloat16], dtype=torch.int16, device=DEV).view(torch.bfloat16)
     view = C[1:M + 1, 32:32 + N]
     L = capi()
     rc = L.fp8b_scaled_mm(tA.data_ptr(), tB.data_ptr(), view.data_ptr(), dt_code(torch.bfloat16), M, N, K, ldc, tsa.data_ptr(), 1,
@@ -798,7 +746,7 @@ def test_tcgen05_output_past_2_31_elements(tune, store):
     ref_np = o.scaled_mm(A[sl], tB[:4096].cpu().numpy(), [sa], [sb], bias[:4096].cpu().numpy(), None, "bf16")
     assert_bits_equal(to_np(ref_rows(M - 8, M)[:, :4096]), ref_np, "torch reference vs oracle")
     raw = C.view(torch.int16)
-    assert (raw[0] == _SENT[torch.bfloat16]).all() and (raw[M + 1] == _SENT[torch.bfloat16]).all(), "rows above / below C written"
+    assert (raw[0] == SENT[torch.bfloat16]).all() and (raw[M + 1] == SENT[torch.bfloat16]).all(), "rows above / below C written"
     step = 2048
     for r0 in range(0, M, step):
         r1 = min(M, r0 + step)
@@ -807,7 +755,7 @@ def test_tcgen05_output_past_2_31_elements(tune, store):
             bad = (got.view(torch.int16) != ref_rows(r0, r1).view(torch.int16)).nonzero()
             raise AssertionError(f"store {store}: {bad.shape[0]} outputs differ in rows [{r0}, {r1}), first at {(bad[0] + torch.tensor([r0, 0], device=DEV)).tolist()}")
         g = raw[1 + r0:1 + r1]
-        assert (g[:, :32] == _SENT[torch.bfloat16]).all() and (g[:, 32 + N:] == _SENT[torch.bfloat16]).all(), \
+        assert (g[:, :32] == SENT[torch.bfloat16]).all() and (g[:, 32 + N:] == SENT[torch.bfloat16]).all(), \
             f"store {store}: columns beside C written in rows [{r0}, {r1})"
 
 

@@ -96,6 +96,47 @@ def test_quantize_golden(golden):
         assert np.array_equal(inv.view(np.uint32), h[f"q{i}_inv"].view(np.uint32))
 
 
+def test_quantize_rows_equals_rowwise_quantize():
+    """fp8_quantize_rows == fp8_quantize row by row, special rows included; the special amax values give the
+    scale and inverse scale the C ABI documents (include/fp8_b200.h)."""
+    rng = np.random.default_rng(11)
+    cols = 37
+    X = (rng.standard_normal((40, cols)) * np.exp2(rng.integers(-20, 20, (40, 1)))).astype(np.float32)
+    specials = {1: 0.0, 2: -0.0, 3: np.nan, 4: np.inf, 5: -np.inf, 6: 448.0, 7: np.finfo(np.float32).max,
+                8: np.float32(2.0 ** -149), 9: np.float32(1e-37), 10: np.float32(2.0 ** -126)}
+    for r, v in specials.items():
+        if r in (1, 2):
+            X[r] = v
+        elif r in (8, 9, 10):
+            X[r] = 0.0
+            X[r, [0, 5, cols - 1]] = [v, -v, v]
+        else:
+            X[r, 3] = v
+    X[11, [2, 7]] = [np.inf, np.nan]
+    X[12] = -1.5
+    for dt in (np.float32, np.float16):
+        with np.errstate(over="ignore"):
+            Xd = X.astype(dt)
+        q, inv = o.fp8_quantize_rows(Xd)
+        assert q.shape == X.shape and inv.shape == (X.shape[0],) and inv.dtype == np.float32
+        for r in range(X.shape[0]):
+            rq, rinv = o.fp8_quantize(Xd[r])
+            assert np.array_equal(q[r], rq), (dt, r)
+            assert inv[r].view(np.uint32) == rinv.view(np.uint32)[0], (dt, r)
+    q, inv = o.fp8_quantize_rows(X)
+    assert inv[1] == inv[2] == 1.0 and not q[1].any() and not q[2].any()             # amax 0: scale 1
+    assert inv[3] == inv[11] == 1.0 and q[3, 3] == q[11, 7] == 0x7F and q[11, 2] == 0x7E   # NaN amax: scale 1
+    for r in (4, 5):                                                                 # inf amax: scale 0, inv +inf
+        assert inv[r] == np.inf
+        finite = np.isfinite(X[r])
+        assert (q[r][finite] == 0).all() and (q[r][~finite] == 0x7F).all()
+    assert inv[12] == np.float32(1.5 / 448.0)
+    for r in (8, 9):                                                                 # float32(448/amax) = inf
+        assert 0.0 <= inv[r] < np.float32(2.0 ** -126)
+        assert (q[r][X[r] == 0] == 0x7F).all() and q[r][0] == 0x7E and q[r][5] == 0xFE
+    assert o.fp8_quantize_rows(np.zeros((3, 0), np.float32))[1].tolist() == [1.0, 1.0, 1.0]
+
+
 def test_quantize_roundtrip_reference_case():
     """test_fp8_metal.py:167-188: max abs error < 50 on the reference's list (it is far smaller)."""
     x = np.array([0.0, 1.0, -1.0, 0.5, -0.5, 100.0, -100.0, 448.0], dtype=np.float32)
