@@ -334,8 +334,12 @@ FP8B_API int fp8b_scaled_mm_multicast(const uint8_t* A, const uint8_t* B, void* 
  * buffer as mapped in this process) - (address of the local buffer); the entry of the calling rank is 0.
  * C_local points at this rank's shard column inside its own buffer (ldc = full N).  Against the multicast mode a
  * rank's own shard does not travel to the switch and back, so each GPU receives (world-1)/world of the output
- * instead of all of it: the better plan for small worlds.  Same 16-byte-path requirements as the multicast mode;
- * CTA-pair tile configurations only (M > 128 and N > 128), else FP8B_ERR_UNSUPPORTED.
+ * instead of all of it: the better plan for small worlds.  Same 16-byte-path requirements as the multicast mode
+ * (N % 32 == 0; 16-byte aligned C_local, ldc * sizeof(out), per-row scale_b and bias; K % 16 == 0, K > 0).  Runs on
+ * the CTA-pair tile configurations only: the built-in tile rule picks one when M > 128 and N > 128, a forced
+ * FP8B_OPT_TUNE_GEMM_CFG 3 / 4 / 5 serves any M and N, and a forced one-CTA configuration (1 / 2) is refused.  Every
+ * unmet requirement returns FP8B_ERR_UNSUPPORTED with nothing launched; world outside 2..8 or a NULL peer_deltas returns
+ * FP8B_ERR_INVALID.  M == 0 or N == 0: FP8B_OK, nothing launched.
  */
 FP8B_API int fp8b_scaled_mm_peers(const uint8_t* A, const uint8_t* B, void* C_local, const int64_t* peer_deltas, int world,
                          int out_dtype, int M, int N, int K, int64_t ldc,

@@ -2,6 +2,7 @@
 import ctypes
 import os
 import re
+import sys
 
 import numpy as np
 import torch
@@ -10,6 +11,10 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "fp8-mps-metal_b200")
 LIB_PATH = os.environ.get("FP8B_LIB") or os.path.join(PKG, "libfp8_b200.so")    # FP8B_LIB: A/B a differently built library
 HEADER = os.path.join(ROOT, "include", "fp8_b200.h")
+if os.path.join(ROOT, "oracle") not in sys.path:       # bench.py imports this module before it adds oracle/
+    sys.path.insert(0, os.path.join(ROOT, "oracle"))
+
+import fp8_oracle as o  # noqa: E402
 
 F32, F16, BF16 = 0, 1, 2
 ALGO_AUTO, ALGO_GEMV, ALGO_TCGEN05, ALGO_SIMT = 0, 1, 2, 3
@@ -21,6 +26,8 @@ GUARD_ROWS = 3
 SENT = {torch.float32: 0x7FA5A5A5, torch.float16: 0x7DA5, torch.bfloat16: 0x7FA5}    # NaN payloads no kernel writes
 _INT = {torch.float32: torch.int32, torch.float16: torch.int16, torch.bfloat16: torch.int16}
 BIG_SCALE = 1024.0                                    # what sits behind per-row scales
+BIG_BIAS = 30000.0                                    # what sits behind per-row biases
+E4M3, E5M2 = 0, 1
 
 
 def declared_symbols():
@@ -234,3 +241,124 @@ def assert_bits_equal(got, ref, what, any_nan=False):
         i = tuple(bad[0])
         raise AssertionError(f"{what}: {len(bad)} of {g.size} outputs differ from the exact result; first at {list(i)}: "
                              f"got {got[i]!r} want {ref[i]!r}")
+
+
+# ------------------------------------------------------------------ structured inputs for the bit-exact matmul tests
+# (test_gpu_exact.py describes the input families and why their sums are exact)
+
+def dev_bytes(X, offset=0, guard_rows=2):
+    """uint8 rows of X, then guard rows of 0x7E, starting `offset` bytes into the allocation -> (tensor, pointer)."""
+    R, K = X.shape
+    flat = np.full(offset + (R + guard_rows) * K + 16, 0x7E, np.uint8)
+    flat[offset:offset + R * K] = X.reshape(-1)
+    t = torch.from_numpy(flat).to(DEV)
+    return t, t.data_ptr() + offset
+
+
+def dev_bias(v, dtype, extra=8):
+    """bias of `dtype` followed by large finite values -> (tensor, the fp32 values the kernel reads)."""
+    t = torch.from_numpy(np.concatenate([np.asarray(v, np.float32), np.full(extra, BIG_BIAS, np.float32)])).to(DEV).to(dtype)
+    return t, to_np(t[:len(v)])
+
+
+def _decode(X, fmt):
+    return o.decode_fmt(X, "e5m2" if fmt == E5M2 else "e4m3fn")
+
+
+def oracle(A, B, sa, sb, bias, sr, odt, fmts=(E4M3, E4M3)):
+    """fp8_oracle.scaled_mm (fp64 sum) restricted to the K columns where A or B has nonzeros: the other columns add
+    exact zeros, and a 100000-long K then costs nothing on the host."""
+    fa, fb = fmts
+    K = A.shape[1]
+    if K > 64:
+        nz = (_decode(A, fa) != 0).any(0)
+        if nz.sum() > K // 4:
+            nzb = (_decode(B, fb) != 0).any(0)
+            nz = nzb if nzb.sum() < nz.sum() else nz
+        cols = np.flatnonzero(nz)
+        A, B = A[:, cols], B[:, cols]
+    return o.scaled_mm(A, B, sa, sb, bias, None if sr is None else np.array([sr], np.float32), dt_name(odt),
+                       accum="f64", a_format="e5m2" if fa == E5M2 else "e4m3fn", b_format="e5m2" if fb == E5M2 else "e4m3fn")
+
+
+NON_NAN = np.array([c for c in range(256) if (c & 0x7F) != 0x7F], np.uint8)
+E5M2_CODES = np.array([c for c in range(256) if (c & 0x7F) < 0x60], np.uint8)       # finite, |v| < 512
+SMALL_INT_CODES = o.encode(np.arange(-16, 17, dtype=np.float32))                     # exact e4m3 codes of -16..16
+
+
+def codes(shape, rng, fmt=E4M3):
+    return rng.choice(E5M2_CODES if fmt == E5M2 else NON_NAN, shape).astype(np.uint8)
+
+
+def edges(K, bounds, rng, n_random=6):
+    """k = 0, the last 16-byte vector, the 16-byte vectors on both sides of every boundary, and random positions."""
+    pos = {0, 15, K - 16, K - 1}
+    for b in bounds:
+        pos |= {b - 16, b - 1, b, b + 15}
+    pos |= set(rng.integers(0, K, n_random).tolist())
+    return np.array(sorted(q for q in pos if 0 <= q < K), np.int64)
+
+
+def one_hot(R, K, positions, rng, fmt=E4M3):
+    """R rows, row r nonzero (a random code, the zero codes included) only at positions[r % len]; a random subset of the
+    positions when there are more of them than rows."""
+    X = np.zeros((R, K), np.uint8)
+    n = len(positions)
+    ks = positions[np.arange(R) % n] if R >= n else positions[np.sort(rng.choice(n, R, replace=False))]
+    X[np.arange(R), ks] = codes(R, rng, fmt)
+    return X
+
+
+def few_hot(R, K, positions, rng):
+    """<= 8 nonzeros per row, all at boundary positions, small integers (|v| <= 16)."""
+    X = np.zeros((R, K), np.uint8)
+    for r in range(R):
+        ks = rng.choice(positions, min(8, len(positions)), replace=False)
+        X[r, ks] = SMALL_INT_CODES[rng.integers(0, 33, len(ks))]
+    return X
+
+
+def small_ints(shape, rng, lo=-16, hi=16):
+    return SMALL_INT_CODES[rng.integers(lo + 16, hi + 17, shape)]
+
+
+def add_nan_rows(B, A, rows, rng):
+    """NaN codes in a few chosen B rows: at the nonzero position of A row 0 (the product must come out as exactly 0 through
+    the NaN fix-up) and at random positions (the fix-up must recompute the one real product)."""
+    k0 = np.flatnonzero(A[0]) if A[0].any() else np.array([0])
+    for i, n in enumerate(rows):
+        B[n, rng.integers(0, B.shape[1], 3)] = 0x7F if i % 2 else 0xFF
+        if i == 0:
+            B[n, k0] = 0x7F
+    return B
+
+
+def sm_count():
+    return torch.cuda.get_device_properties(0).multi_processor_count
+
+
+def tc_bounds(K):
+    return set(range(128, K, 128))
+
+
+class Terms:
+    """Random fp32 epilogue terms: per-tensor or per-row sa / sb, a bias of some dtype, scale_result."""
+
+    def __init__(self, M, N, rng, per_row_a=False, per_row_b=False, bias_dt=None, sr=False):
+        self.sa = ((rng.random(M if per_row_a else 1) + 0.5) * 0.0123).astype(np.float32)
+        self.sb = ((rng.random(N if per_row_b else 1) + 0.5) * 0.0217).astype(np.float32)
+        self.bias_dt = bias_dt
+        self.bias_raw = (rng.standard_normal(N) * 0.7).astype(np.float32) if bias_dt is not None else None
+        self.sr = float(np.float32(0.5 + rng.random())) if sr else None
+
+    @staticmethod
+    def cycle(i, M, N, rng):
+        """the i-th of a fixed rotation over the term combinations."""
+        return Terms(M, N, rng, per_row_a=bool(i & 1), per_row_b=bool(i & 2),
+                     bias_dt=(None, torch.float32, torch.float16, torch.bfloat16)[(i >> 2) % 4], sr=bool(i % 3 == 1))
+
+    def device(self):
+        self.t_sa, self.t_sb = dev_f32(self.sa), dev_f32(self.sb)
+        self.t_bias, self.bias = (None, None) if self.bias_dt is None else dev_bias(self.bias_raw, self.bias_dt)
+        self.t_sr = dev_f32([self.sr]) if self.sr is not None else None
+        return self

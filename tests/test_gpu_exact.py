@@ -31,114 +31,17 @@ import pytest
 import torch
 
 import fp8_oracle as o
-from _util import (ALGO_AUTO, ALGO_GEMV, ALGO_SIMT, ALGO_TCGEN05, SENT, GemvItem, Out, assert_bits_equal, capi, dev_f32, dt_code,
-                   dt_name, p, stream_ptr, to_np)
+from _util import (ALGO_AUTO, ALGO_GEMV, ALGO_SIMT, ALGO_TCGEN05, E4M3, E5M2, SENT, GemvItem, Out, Terms, add_nan_rows, assert_bits_equal,
+                   capi, codes, dev_bytes, dev_f32, dt_code, dt_name, edges, few_hot, one_hot, oracle, p, sm_count, small_ints,
+                   stream_ptr, tc_bounds, to_np)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
 OPT_PDL, OPT_STATIC_WEIGHTS = 0, 1
-E4M3, E5M2 = 0, 1
 ODTS = (torch.float32, torch.float16, torch.bfloat16)
-
-BIG_BIAS = 30000.0                                    # what sits behind per-row biases
-
-
-# ------------------------------------------------------------------ device buffers with guard bands
-
-def dev_bytes(X, offset=0, guard_rows=2):
-    """uint8 rows of X, then guard rows of 0x7E, starting `offset` bytes into the allocation -> (tensor, pointer)."""
-    R, K = X.shape
-    flat = np.full(offset + (R + guard_rows) * K + 16, 0x7E, np.uint8)
-    flat[offset:offset + R * K] = X.reshape(-1)
-    t = torch.from_numpy(flat).to(DEV)
-    return t, t.data_ptr() + offset
-
-
-def dev_bias(v, dtype, extra=8):
-    """bias of `dtype` followed by large finite values -> (tensor, the fp32 values the kernel reads)."""
-    t = torch.from_numpy(np.concatenate([np.asarray(v, np.float32), np.full(extra, BIG_BIAS, np.float32)])).to(DEV).to(dtype)
-    return t, to_np(t[:len(v)])
-
-
-def _decode(X, fmt):
-    return o.decode_fmt(X, "e5m2" if fmt == E5M2 else "e4m3fn")
-
-
-def oracle(A, B, sa, sb, bias, sr, odt, fmts=(E4M3, E4M3)):
-    """fp8_oracle.scaled_mm (fp64 sum) restricted to the K columns where A or B has nonzeros: the other columns add
-    exact zeros, and a 100000-long K then costs nothing on the host."""
-    fa, fb = fmts
-    K = A.shape[1]
-    if K > 64:
-        nz = (_decode(A, fa) != 0).any(0)
-        if nz.sum() > K // 4:
-            nzb = (_decode(B, fb) != 0).any(0)
-            nz = nzb if nzb.sum() < nz.sum() else nz
-        cols = np.flatnonzero(nz)
-        A, B = A[:, cols], B[:, cols]
-    return o.scaled_mm(A, B, sa, sb, bias, None if sr is None else np.array([sr], np.float32), dt_name(odt),
-                       accum="f64", a_format="e5m2" if fa == E5M2 else "e4m3fn", b_format="e5m2" if fb == E5M2 else "e4m3fn")
-
-
-# ------------------------------------------------------------------ input families
-
-NON_NAN = np.array([c for c in range(256) if (c & 0x7F) != 0x7F], np.uint8)
-E5M2_CODES = np.array([c for c in range(256) if (c & 0x7F) < 0x60], np.uint8)       # finite, |v| < 512
-SMALL_INT_CODES = o.encode(np.arange(-16, 17, dtype=np.float32))                     # exact e4m3 codes of -16..16
-
-
-def codes(shape, rng, fmt=E4M3):
-    return rng.choice(E5M2_CODES if fmt == E5M2 else NON_NAN, shape).astype(np.uint8)
-
-
-def edges(K, bounds, rng, n_random=6):
-    """k = 0, the last 16-byte vector, the 16-byte vectors on both sides of every boundary, and random positions."""
-    pos = {0, 15, K - 16, K - 1}
-    for b in bounds:
-        pos |= {b - 16, b - 1, b, b + 15}
-    pos |= set(rng.integers(0, K, n_random).tolist())
-    return np.array(sorted(q for q in pos if 0 <= q < K), np.int64)
-
-
-def one_hot(R, K, positions, rng, fmt=E4M3):
-    """R rows, row r nonzero (a random code, the zero codes included) only at positions[r % len]; a random subset of the
-    positions when there are more of them than rows."""
-    X = np.zeros((R, K), np.uint8)
-    n = len(positions)
-    ks = positions[np.arange(R) % n] if R >= n else positions[np.sort(rng.choice(n, R, replace=False))]
-    X[np.arange(R), ks] = codes(R, rng, fmt)
-    return X
-
-
-def few_hot(R, K, positions, rng):
-    """<= 8 nonzeros per row, all at boundary positions, small integers (|v| <= 16)."""
-    X = np.zeros((R, K), np.uint8)
-    for r in range(R):
-        ks = rng.choice(positions, min(8, len(positions)), replace=False)
-        X[r, ks] = SMALL_INT_CODES[rng.integers(0, 33, len(ks))]
-    return X
-
-
-def small_ints(shape, rng, lo=-16, hi=16):
-    return SMALL_INT_CODES[rng.integers(lo + 16, hi + 17, shape)]
-
-
-def add_nan_rows(B, A, rows, rng):
-    """NaN codes in a few chosen B rows: at the nonzero position of A row 0 (the product must come out as exactly 0 through
-    the NaN fix-up) and at random positions (the fix-up must recompute the one real product)."""
-    k0 = np.flatnonzero(A[0]) if A[0].any() else np.array([0])
-    for i, n in enumerate(rows):
-        B[n, rng.integers(0, B.shape[1], 3)] = 0x7F if i % 2 else 0xFF
-        if i == 0:
-            B[n, k0] = 0x7F
-    return B
 
 
 # ------------------------------------------------------------------ plans (to place the nonzeros)
-
-def sm_count():
-    return torch.cuda.get_device_properties(0).multi_processor_count
-
 
 def fhfma_bounds(M, N, K):
     """split-K rank edges and shared-memory panel edges of the FHFMA GEMV (launch_gemv_fhfma)."""
@@ -164,34 +67,7 @@ def mma_bounds(K, batch=4):
     return {w * kpw + d for w in range(8) for d in (0, 64, 64 * batch)}
 
 
-def tc_bounds(K):
-    return set(range(128, K, 128))
-
-
 # ------------------------------------------------------------------ calls through the C ABI
-
-class Terms:
-    """Random fp32 epilogue terms: per-tensor or per-row sa / sb, a bias of some dtype, scale_result."""
-
-    def __init__(self, M, N, rng, per_row_a=False, per_row_b=False, bias_dt=None, sr=False):
-        self.sa = ((rng.random(M if per_row_a else 1) + 0.5) * 0.0123).astype(np.float32)
-        self.sb = ((rng.random(N if per_row_b else 1) + 0.5) * 0.0217).astype(np.float32)
-        self.bias_dt = bias_dt
-        self.bias_raw = (rng.standard_normal(N) * 0.7).astype(np.float32) if bias_dt is not None else None
-        self.sr = float(np.float32(0.5 + rng.random())) if sr else None
-
-    @staticmethod
-    def cycle(i, M, N, rng):
-        """the i-th of a fixed rotation over the term combinations."""
-        return Terms(M, N, rng, per_row_a=bool(i & 1), per_row_b=bool(i & 2),
-                     bias_dt=(None, torch.float32, torch.float16, torch.bfloat16)[(i >> 2) % 4], sr=bool(i % 3 == 1))
-
-    def device(self):
-        self.t_sa, self.t_sb = dev_f32(self.sa), dev_f32(self.sb)
-        self.t_bias, self.bias = (None, None) if self.bias_dt is None else dev_bias(self.bias_raw, self.bias_dt)
-        self.t_sr = dev_f32([self.sr]) if self.sr is not None else None
-        return self
-
 
 def run_mm(A, B, odt, algo=ALGO_AUTO, terms=None, rng=None, fmts=None, a_offset=0, aligned=True, expect_rc=0, what="",
            dB=None):
