@@ -36,6 +36,17 @@ int to_fp8b_dtype(at::ScalarType t)
     return -1;
 }
 
+// Output dtype of the matmul ops: the three above plus float8_e4m3fn, whose bytes are the reference encoder's bytes of the
+// fp32 epilogue value (what the reference's `_scaled_mm(...).to(float8_e4m3fn)` produces).  Inputs and biases stay with
+// to_fp8b_dtype; float8_e5m2 is never an output.
+int to_fp8b_out_dtype(at::ScalarType t)
+{
+    if (t == at::kFloat8_e4m3fn) return FP8B_OUT_E4M3FN;
+    if (t == at::kFloat || t == at::kHalf || t == at::kBFloat16) return to_fp8b_dtype(t);
+    throw std::runtime_error(std::string("fp8_metal: unsupported output dtype ") + c10::toString(t) +
+                             " (need float32, float16, bfloat16 or float8_e4m3fn)");
+}
+
 // The reference raises std::runtime_error for launch failures (fp8_bridge.cpp:96-101); so does this.
 void check_status(int rc, const char* what)
 {
@@ -112,11 +123,11 @@ torch::Tensor fp8_scaled_mm_fused(torch::Tensor A, torch::Tensor B, torch::Tenso
     if (M == 0 || N == 0) return C;
     int rc;
     if (a_format != FP8B_E4M3FN || b_format != FP8B_E4M3FN)
-        rc = fp8b_scaled_mm_fmt(u8_ptr(A), (int)a_format, u8_ptr(B), (int)b_format, C.data_ptr(), to_fp8b_dtype(odt),
+        rc = fp8b_scaled_mm_fmt(u8_ptr(A), (int)a_format, u8_ptr(B), (int)b_format, C.data_ptr(), to_fp8b_out_dtype(odt),
                                 (int)M, (int)N, (int)K, ldc, sa.data_ptr<float>(), (int)sa.numel(), sb.data_ptr<float>(),
                                 (int)sb.numel(), bias_ptr, bias_dt, sr_ptr, (int)algo, current_stream());
     else
-        rc = fp8b_scaled_mm(u8_ptr(A), u8_ptr(B), C.data_ptr(), to_fp8b_dtype(odt), (int)M, (int)N, (int)K, ldc,
+        rc = fp8b_scaled_mm(u8_ptr(A), u8_ptr(B), C.data_ptr(), to_fp8b_out_dtype(odt), (int)M, (int)N, (int)K, ldc,
                                 sa.data_ptr<float>(), (int)sa.numel(), sb.data_ptr<float>(), (int)sb.numel(),
                                 bias_ptr, bias_dt, sr_ptr, nullptr, 0, (int)algo, current_stream());
     check_status(rc, "fp8b_scaled_mm");
@@ -210,7 +221,7 @@ torch::Tensor scaled_mm_patch(torch::Tensor input, torch::Tensor other, c10::opt
     if (M == 0 || N == 0) return C;
     const int rc = fp8b_scaled_mm_fmt(static_cast<const uint8_t*>(a.data_ptr()), format_of(input),
                                       static_cast<const uint8_t*>(b.data_ptr()), format_of(other), C.data_ptr(),
-                                      to_fp8b_dtype(odt), (int)M, (int)N, (int)K, N, sa, (int)sa_len, sb, (int)sb_len,
+                                      to_fp8b_out_dtype(odt), (int)M, (int)N, (int)K, N, sa, (int)sa_len, sb, (int)sb_len,
                                       bias_ptr, bias_dt, sr, FP8B_MM_AUTO, current_stream());
     check_status(rc, "fp8b_scaled_mm");
     return C;
@@ -419,7 +430,7 @@ std::vector<torch::Tensor> fp8_scaled_mm_many(std::vector<torch::Tensor> xs, std
             q.bias = bt.data_ptr();
         }
     }
-    check_status(fp8b_gemv_batch(items.data(), (int)n, (int)K, to_fp8b_dtype(odt), bias_dt, current_stream()), "fp8b_gemv_batch");
+    check_status(fp8b_gemv_batch(items.data(), (int)n, (int)K, to_fp8b_out_dtype(odt), bias_dt, current_stream()), "fp8b_gemv_batch");
     return outs;
 }
 
@@ -450,7 +461,7 @@ void fp8_scaled_mm_peers(torch::Tensor A, torch::Tensor B, torch::Tensor scale_a
         bias_ptr = bias_t.data_ptr();
         bias_dt = to_fp8b_dtype(bias_t.scalar_type());
     }
-    const int odt = to_fp8b_dtype(out.scalar_type());
+    const int odt = to_fp8b_out_dtype(out.scalar_type());
     void* c_local = static_cast<uint8_t*>(out.data_ptr()) + n0 * out.element_size();
     int rc = fp8b_scaled_mm_peers(u8_ptr(A), u8_ptr(B), c_local, peer_deltas.data_ptr<int64_t>(), (int)peer_deltas.numel(), odt,
                                   (int)M, (int)N, (int)K, full_N, sa.data_ptr<float>(), (int)sa.numel(),
@@ -493,7 +504,7 @@ void fp8_scaled_mm_push(torch::Tensor A, torch::Tensor B, torch::Tensor scale_a,
     for (size_t d = 0; d < dst_ptrs.size(); ++d)
         dsts[d] = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(dst_ptrs[d])) + n0 * out.element_size();
     const int n_dst = (int)dst_ptrs.size();
-    const int odt = to_fp8b_dtype(out.scalar_type());
+    const int odt = to_fp8b_out_dtype(out.scalar_type());
     if (signal_ptrs.empty()) {
         check_status(fp8b_scaled_mm_push(u8_ptr(A), u8_ptr(B), dsts, n_dst, odt, (int)M, (int)N, (int)K, full_N, sa, (int)sa_len,
                                          sb, (int)sb_len, bias_ptr, bias_dt, nullptr, current_stream()),
@@ -572,7 +583,7 @@ std::tuple<torch::Tensor, torch::Tensor> fp8_linear_dynamic(torch::Tensor x, tor
         ws = torch::empty({(int64_t)ws_bytes}, torch::TensorOptions().dtype(torch::kUInt8).device(x.device()));
         ws_ptr = ws.data_ptr();
     }
-    int rc = fp8b_linear_dynamic(xin.data_ptr(), to_fp8b_dtype(xin.scalar_type()), u8_ptr(B), C.data_ptr(), to_fp8b_dtype(odt),
+    int rc = fp8b_linear_dynamic(xin.data_ptr(), to_fp8b_dtype(xin.scalar_type()), u8_ptr(B), C.data_ptr(), to_fp8b_out_dtype(odt),
                                (int)M, (int)N, (int)K, N, sb.data_ptr<float>(), (int)sb.numel(), bias_ptr, bias_dt, nullptr,
                                inv.data_ptr<float>(), ws_ptr, ws_bytes, current_stream());
     check_status(rc, "fp8b_linear_dynamic");
@@ -581,7 +592,7 @@ std::tuple<torch::Tensor, torch::Tensor> fp8_linear_dynamic(torch::Tensor x, tor
 
 int64_t select_algo(torch::Tensor A, torch::Tensor B, at::ScalarType out_dtype)
 {
-    return fp8b_scaled_mm_select(u8_ptr(A), u8_ptr(B), nullptr, to_fp8b_dtype(out_dtype), (int)A.size(0), (int)B.size(0),
+    return fp8b_scaled_mm_select(u8_ptr(A), u8_ptr(B), nullptr, to_fp8b_out_dtype(out_dtype), (int)A.size(0), (int)B.size(0),
                                  (int)A.size(1), B.size(0));
 }
 
@@ -631,7 +642,7 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m)
           py::arg("epoch") = 0, py::arg("wait_flags") = py::none(), py::arg("rank") = 0);
     m.def("push_supported", [](int64_t M, int64_t N, int64_t K, int64_t ldc, at::ScalarType dt) {
         // alignment of torch allocations (>= 256 B) is assumed; this answers the shape part
-        return fp8b_scaled_mm_push_supported(to_fp8b_dtype(dt), (int)M, (int)N, (int)K, ldc, nullptr, nullptr, nullptr) != 0;
+        return fp8b_scaled_mm_push_supported(to_fp8b_out_dtype(dt), (int)M, (int)N, (int)K, ldc, nullptr, nullptr, nullptr) != 0;
     });
     m.def("select_algo", &select_algo, py::arg("A"), py::arg("B"), py::arg("out_dtype"));
     m.def("launch_count", []() { return (uint64_t)fp8b_launch_count(); });

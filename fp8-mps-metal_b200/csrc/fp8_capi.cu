@@ -59,7 +59,7 @@ static int validate(const MMArgs& a)
     if (a.M == 0 || a.N == 0) return FP8B_OK;
     if (!a.C || !a.sa || !a.sb) return FP8B_ERR_INVALID;
     if (a.K > 0 && (!a.A || !a.B)) return FP8B_ERR_INVALID;
-    if (!valid_dtype(a.out_dtype)) return FP8B_ERR_INVALID;
+    if (!valid_out_dtype(a.out_dtype)) return FP8B_ERR_INVALID;
     if (a.bias && !valid_dtype(a.bias_dtype)) return FP8B_ERR_INVALID;
     if (a.ldc < a.N) return FP8B_ERR_INVALID;
     if (!(a.sa_len == 1 || a.sa_len == a.M)) return FP8B_ERR_INVALID;
@@ -199,6 +199,7 @@ extern "C" int fp8b_scaled_mm_multicast(const uint8_t* A, const uint8_t* B, void
     a.store_mc = 1;
     int rc = validate(a);
     if (rc != FP8B_OK) return rc;
+    if (out_dtype == FP8B_OUT_E4M3FN) return FP8B_ERR_UNSUPPORTED;    // no byte output through the multicast mapping
     if (M == 0 || N == 0) return FP8B_OK;
     if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
     return launch_gemm_tcgen05(a);
@@ -220,7 +221,7 @@ extern "C" int fp8b_linear_dynamic(const void* X, int x_dtype, const uint8_t* B,
 {
     if (M < 0 || N < 0 || K < 0) return FP8B_ERR_INVALID;
     if (M == 0 || N == 0) return FP8B_OK;
-    if (!X || !B || !C || !scale_b || !valid_dtype(x_dtype) || !valid_dtype(out_dtype)) return FP8B_ERR_INVALID;
+    if (!X || !B || !C || !scale_b || !valid_dtype(x_dtype) || !valid_out_dtype(out_dtype)) return FP8B_ERR_INVALID;
     if (bias && !valid_dtype(bias_dtype)) return FP8B_ERR_INVALID;
     if (ldc < N || !(scale_b_len == 1 || scale_b_len == N)) return FP8B_ERR_INVALID;
     if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
@@ -350,7 +351,7 @@ extern "C" int fp8b_peer_wait(const uint64_t* flags, int world, int rank, uint64
 extern "C" int fp8b_scaled_mm_push_supported(int out_dtype, int M, int N, int K, int64_t ldc, const void* A, const void* B,
                                              const void* C)
 {
-    if (M < 1 || N < 1 || K < 16 || (K % 16) != 0 || !valid_dtype(out_dtype) || ldc < N) return 0;
+    if (M < 1 || N < 1 || K < 16 || (K % 16) != 0 || !valid_out_dtype(out_dtype) || ldc < N) return 0;
     if (!aligned(A, 16) || !aligned(B, 16) || !aligned(C, 16)) return 0;
     return (((size_t)ldc * dtype_size(out_dtype)) % 16 == 0 && ((size_t)N * dtype_size(out_dtype)) % 16 == 0) ? 1 : 0;
 }

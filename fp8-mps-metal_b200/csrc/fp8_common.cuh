@@ -88,7 +88,10 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 #endif
 
 inline bool aligned(const void* p, size_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) == 0; }
-inline size_t dtype_size(int dt) { return dt == FP8B_F32 ? 4 : 2; }
+inline size_t dtype_size(int dt) { return dt == FP8B_F32 ? 4 : dt == FP8B_OUT_E4M3FN ? 1 : 2; }
+// input types (casts, bias, X of fp8b_linear_dynamic)
 inline bool valid_dtype(int dt) { return dt == FP8B_F32 || dt == FP8B_F16 || dt == FP8B_BF16; }
+// output types of the matmul entry points: the inputs plus e4m3fn bytes
+inline bool valid_out_dtype(int dt) { return valid_dtype(dt) || dt == FP8B_OUT_E4M3FN; }
 
 }  // namespace fp8b

@@ -351,6 +351,47 @@ __device__ __forceinline__ bool any_nan32(const uint32_t (&r)[32]) {
     return s != s;
 }
 
+__device__ __forceinline__ int out_esz(int out_dtype) { return out_dtype == FP8B_F32 ? 4 : out_dtype == FP8B_OUT_E4M3FN ? 1 : 2; }
+
+// The 32 epilogue values of one lane -> the output type, packed little-endian into the row's 16-byte pieces, each handed
+// to store16(j, w0, w1, w2, w3) for piece j: 8 pieces (f32), 4 (f16 / bf16) or 2 (e4m3fn: the reference encoder,
+// enc_prepare_f32 on the input, then the satfinite conversion).  Every vector epilogue of this file stores through it; each
+// output type keeps its own compile-time piece loop, so no packed copy of the 32 values has to stay live.
+template <typename Store16>
+__device__ __forceinline__ void pack_out32(const float (&v)[32], int out_dtype, Store16&& store16) {
+    if (out_dtype == FP8B_F32) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j)
+            store16(j, __float_as_uint(v[4 * j]), __float_as_uint(v[4 * j + 1]), __float_as_uint(v[4 * j + 2]),
+                    __float_as_uint(v[4 * j + 3]));
+    } else if (out_dtype == FP8B_OUT_E4M3FN) {
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            uint32_t w[4];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const int c = 16 * j + 4 * i;
+                w[i] = enc4_f32(v[c], v[c + 1], v[c + 2], v[c + 3]);
+            }
+            store16(j, w[0], w[1], w[2], w[3]);
+        }
+    } else {
+        uint32_t pk[16];
+#pragma unroll
+        for (int j = 0; j < 16; ++j) {
+            if (out_dtype == FP8B_BF16) {
+                __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
+                pk[j] = *reinterpret_cast<uint32_t*>(&b);
+            } else {
+                __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
+                pk[j] = *reinterpret_cast<uint32_t*>(&h);
+            }
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j) store16(j, pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+    }
+}
+
 // Cold paths of the epilogue, out of line and working on local-memory copies, so that they cost the hot loop neither
 // instructions nor instruction-cache footprint (with the NaN fix-up inlined 32 times per chunk the 128 x 256 epilogue took
 // 8 100 cycles, without it 6 800; with the term dispatch hoisted out of the tile loop as well, 3 700).
@@ -603,7 +644,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
         if constexpr (MODE == kStTma) {
             const bool elected = elect_one();
             const int n_dst = p.store_mc >> 8;
-            const int esz = p.epi.out_dtype == FP8B_F32 ? 4 : 2;
+            const int esz = out_esz(p.epi.out_dtype);
             const int cols_per_box = 128 / esz;
             uint32_t seq = 0;
             for (int tile = worker; tile < num_tiles; tile += num_workers) {
@@ -644,8 +685,8 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
             const Epi& e = p.epi;
             const float sr = e.sr ? *e.sr : 1.0f;
             const float sb0 = e.sb[0];
-            const bool is_f32 = e.out_dtype == FP8B_F32;
-            const int cols_per_box = 128 / (is_f32 ? 4 : 2);
+            const int esz = out_esz(e.out_dtype);
+            const int cols_per_box = 128 / esz;
             const uint32_t row_off = (uint32_t)row_in_tile * 128u;
             uint32_t seq = 0;
             int acc = 0; uint32_t acc_phase = 0;
@@ -716,31 +757,10 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                             const uint32_t dst = stage_base + slot * kStoreBoxBytes + row_off;
                             const uint32_t sw = (uint32_t)(lane & 7);
                             // first 16-byte piece of this chunk inside the box row
-                            const uint32_t piece0 = (uint32_t)(((c0 & (cols_per_box - 1)) * (is_f32 ? 4 : 2)) >> 4);
-                            if (is_f32) {
-#pragma unroll
-                                for (int j = 0; j < 8; ++j)
-                                    sts_v4(dst + (((piece0 + j) ^ sw) << 4), __float_as_uint(v[4 * j]), __float_as_uint(v[4 * j + 1]),
-                                           __float_as_uint(v[4 * j + 2]), __float_as_uint(v[4 * j + 3]));
-                            } else {
-                                uint32_t pk[16];
-                                if (e.out_dtype == FP8B_BF16) {
-#pragma unroll
-                                    for (int j = 0; j < 16; ++j) {
-                                        __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
-                                        pk[j] = *reinterpret_cast<uint32_t*>(&b);
-                                    }
-                                } else {
-#pragma unroll
-                                    for (int j = 0; j < 16; ++j) {
-                                        __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
-                                        pk[j] = *reinterpret_cast<uint32_t*>(&h);
-                                    }
-                                }
-#pragma unroll
-                                for (int j = 0; j < 4; ++j)
-                                    sts_v4(dst + (((piece0 + j) ^ sw) << 4), pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
-                            }
+                            const uint32_t piece0 = (uint32_t)(((c0 & (cols_per_box - 1)) * esz) >> 4);
+                            pack_out32(v, e.out_dtype, [&](int j, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
+                                sts_v4(dst + (((piece0 + (uint32_t)j) ^ sw) << 4), w0, w1, w2, w3);
+                            });
                         }
                         if (box_last) {
                             fence_proxy_async_smem();   // generic-proxy writes -> visible to the TMA (async proxy)
@@ -869,31 +889,14 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                         if (e.sr) x = __fmul_rn(x, sr);
                         v[j] = x;
                     }
-                    // pack to the output dtype: 8 (f32) or 4 (f16/bf16) 16-byte pieces per lane
-                    uint32_t pk[32];
-                    const bool is_f32 = e.out_dtype == FP8B_F32;
-                    if (is_f32) {
-#pragma unroll
-                        for (int j = 0; j < 32; ++j) pk[j] = __float_as_uint(v[j]);
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            if (e.out_dtype == FP8B_BF16) {
-                                __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
-                                pk[j] = *reinterpret_cast<uint32_t*>(&b);
-                            } else {
-                                __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
-                                pk[j] = *reinterpret_cast<uint32_t*>(&h);
-                            }
-                        }
-                    }
-                    // Row groups of 256 bytes (128 16-bit or 64 fp32 columns) are staged through a per-warp
+                    const int esz = out_esz(e.out_dtype);
+                    const int ppc = 2 * esz;                             // 16-byte pieces per chunk per row: 8, 4 or 2
+                    // Row groups of 256 bytes (256 e4m3fn, 128 16-bit or 64 fp32 columns) are staged through a per-warp
                     // XOR-swizzled shared-memory tile and written out with 16 lanes per row, so every
                     // store instruction covers 2 rows x 256 contiguous bytes (full 128-byte lines) -- for
                     // local HBM and, in multicast mode, for NVLink, where 16-byte-per-row scatter is fatal.
                     // chunks per row group: 256-byte row segments when the warp's column span allows it, else 128-byte
-                    const int ppc = is_f32 ? 8 : 4;                      // 16-byte pieces per chunk per row
-                    const int cpg_max = is_f32 ? 2 : 4;
+                    const int cpg_max = 8 / esz;
                     const int cpg = (cols_per_warp % (cpg_max * 32) == 0) ? cpg_max : cpg_max / 2;
                     const int ppr = cpg * ppc;                           // 16-byte pieces per staged row: 16 or 8
                     const int rel = (c0 - col_part * cols_per_warp) >> 5; // chunk index inside this warp's span
@@ -904,16 +907,12 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                     if (staged) {
                         const uint32_t wbase = stage_base + (uint32_t)(warp - kWarpEpi0) * 8192u;
                         const uint32_t row_bytes = (uint32_t)ppr * 16u;
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) {
-                            if (j < ppc) {
-                                const uint32_t phys = (uint32_t)((cg * ppc + j) ^ (lane & (ppr - 1)));
-                                sts_v4(wbase + (uint32_t)lane * row_bytes + phys * 16u, pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
-                            }
-                        }
+                        pack_out32(v, e.out_dtype, [&](int j, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
+                            const uint32_t phys = (uint32_t)((cg * ppc + j) ^ (lane & (ppr - 1)));
+                            sts_v4(wbase + (uint32_t)lane * row_bytes + phys * 16u, w0, w1, w2, w3);
+                        });
                         if (cg == cpg - 1) {
                             __syncwarp();
-                            const int esz = is_f32 ? 4 : 2;
                             const int piece = lane & (ppr - 1);
                             const int rows_per_inst = 32 / ppr;          // 2 (256-byte rows) or 4 (128-byte rows)
                             uint8_t* cbase = reinterpret_cast<uint8_t*>(e.C) + (size_t)ng0 * esz + (size_t)piece * 16;
@@ -928,10 +927,10 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                             __syncwarp();
                         }
                     } else if (m_ok && !FP8B_DBG(p, 1)) {
-                        uint8_t* dst = reinterpret_cast<uint8_t*>(e.C) + ((size_t)m * e.ldc + n0) * (is_f32 ? 4 : 2);
-#pragma unroll
-                        for (int j = 0; j < 8; ++j)
-                            if (j < ppc) store16(dst + 16 * j, pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+                        uint8_t* dst = reinterpret_cast<uint8_t*>(e.C) + ((size_t)m * e.ldc + n0) * esz;
+                        pack_out32(v, e.out_dtype, [&](int j, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
+                            store16(dst + 16 * j, w0, w1, w2, w3);
+                        });
                     }
                 } else if (m_ok) {
                     // edge chunk / unaligned output: scalar, bounds-checked
@@ -1170,8 +1169,7 @@ fp8_gemm_splitk_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_
         const float sa = e.sa[(size_t)(m_ok ? m : 0) * e.sa_stride];
         const float sr = e.sr ? *e.sr : 1.0f;
         const float sb0 = e.sb[0];
-        const bool is_f32 = e.out_dtype == FP8B_F32;
-        const int esz = is_f32 ? 4 : 2;
+        const int esz = out_esz(e.out_dtype);
         const int kind = (e.sb_stride ? 1 : 0) | (e.bias ? 2 : 0) | (e.sr ? 4 : 0);
 #pragma unroll 1
         for (int c0 = 0; c0 < kSlice; c0 += 32) {
@@ -1232,29 +1230,9 @@ fp8_gemm_splitk_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_
             if (!m_ok) continue;
             if (full && p.vec_store_ok) {
                 uint8_t* dst = reinterpret_cast<uint8_t*>(e.C) + ((size_t)m * e.ldc + n0) * esz;
-                if (is_f32) {
-#pragma unroll
-                    for (int j = 0; j < 8; ++j)
-                        stg_v4(dst + 16 * j, __float_as_uint(v[4 * j]), __float_as_uint(v[4 * j + 1]), __float_as_uint(v[4 * j + 2]),
-                               __float_as_uint(v[4 * j + 3]), 0);
-                } else {
-                    uint32_t pk[16];
-                    if (e.out_dtype == FP8B_BF16) {
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            __nv_bfloat162 b = __floats2bfloat162_rn(v[2 * j], v[2 * j + 1]);
-                            pk[j] = *reinterpret_cast<uint32_t*>(&b);
-                        }
-                    } else {
-#pragma unroll
-                        for (int j = 0; j < 16; ++j) {
-                            __half2 h = __floats2half2_rn(v[2 * j], v[2 * j + 1]);
-                            pk[j] = *reinterpret_cast<uint32_t*>(&h);
-                        }
-                    }
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) stg_v4(dst + 16 * j, pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3], 0);
-                }
+                pack_out32(v, e.out_dtype, [&](int j, uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3) {
+                    stg_v4(dst + 16 * j, w0, w1, w2, w3, 0);
+                });
             } else {
                 float t[32];                          // (a local copy: v itself stays in registers on the hot path)
 #pragma unroll
@@ -1467,7 +1445,8 @@ static int launch_tcgen05_cfg(const MMArgs& a)
         void* const* dsts = static_cast<void* const*>(a.ws);
         void* self[1] = {a.C};
         if (!dsts) dsts = self;
-        if (n_dst < 1 || n_dst > kMaxDst || !tma_store_ok(a, dsts, n_dst)) return FP8B_ERR_UNSUPPORTED;
+        // (BN * esz) % 128: a tile must be whole 128-byte boxes, or a box store would cover the next tile's columns
+        if (n_dst < 1 || n_dst > kMaxDst || !tma_store_ok(a, dsts, n_dst) || (BN * esz) % 128 != 0) return FP8B_ERR_UNSUPPORTED;
         for (int d = 0; d < n_dst; ++d)
             if (!get_tensor_map(&smaps.m[d], dsts[d], (uint64_t)a.M, (uint64_t)a.N * esz, (uint64_t)a.ldc * esz, 128, 128))
                 return FP8B_ERR_CUDA;
@@ -1620,7 +1599,15 @@ constexpr int kDefaultGemmStore = 2;      // epilogue of plain fp8b_scaled_mm ca
                                           // store (C4: 109.7 vs 112.0 us in the same bench run; falls back to 1 when C is not TMA-storable)
 
 // Tile configuration: 1 = 128x256 one CTA, 2 = 128x128 one CTA, 3 = 256x256 pair, 4 = 256x128 pair, 5 = 256x192 pair.
-static int pick_tile_cfg(const MMArgs& a, bool pairs_only = false)
+// The TMA-store epilogue needs tiles of whole 128-byte boxes; only 256x192 with 1-byte (e4m3fn) elements is not.
+static bool tile_whole_boxes(int cfg, int out_dtype)
+{
+    const int width = cfg == 5 ? 192 : (cfg == 1 || cfg == 3) ? 256 : 128;
+    return (width * dtype_size(out_dtype)) % 128 == 0;
+}
+
+// no_192: leave 256x192 out of the choice (a TMA-store epilogue that cannot take it)
+static int pick_tile_cfg(const MMArgs& a, bool pairs_only = false, bool no_192 = false)
 {
     const int sms = device_info().sm_count;
     // Small problems (one round of 128 x 128 tiles, or two short ones): one-CTA tiles.  A CTA pair spends ~1 300 more cycles
@@ -1644,7 +1631,7 @@ static int pick_tile_cfg(const MMArgs& a, bool pairs_only = false)
         };
         int cfg = 3;
         double best = cost(256);
-        if (cost(192) < best) { best = cost(192); cfg = 5; }
+        if (!no_192 && cost(192) < best) { best = cost(192); cfg = 5; }
         if (cost(128) < best) { best = cost(128); cfg = 4; }
         return cfg;
     }
@@ -1660,7 +1647,8 @@ int launch_gemm_tcgen05(const MMArgs& a)
     // fp8b_set_option(FP8B_OPT_TUNE_GEMM_CFG) -- a result-neutral tuning knob -- forces one.
     const int forced = tune(kTuneGemmCfg, 0);
     const int mode = a.store_mc & 0xFF;
-    int cfg = forced ? forced : pick_tile_cfg(a, /*pairs_only=*/mode == 2);      // (the round-1 peer-store plan exists for CTA pairs only)
+    int cfg = forced ? forced : pick_tile_cfg(a, /*pairs_only=*/mode == 2,      // (the round-1 peer-store plan exists for CTA pairs only)
+                                              /*no_192=*/mode == 3 && !tile_whole_boxes(5, a.out_dtype));
     if (mode == 0 && !forced) {               // plain call: few tiles and a long K -> several CTAs per tile
         const int split = pick_split_k(a);
         if (split == 4) return launch_splitk<4>(a);
@@ -1690,7 +1678,7 @@ int launch_gemm_tcgen05(const MMArgs& a)
     }
     if (mode == 0 && tune(kTuneGemmStore, kDefaultGemmStore) == 2) {      // plain call, TMA-store epilogue to the one output
         void* self[1] = {a.C};
-        if (tma_store_ok(a, self, 1)) {
+        if (tma_store_ok(a, self, 1) && tile_whole_boxes(cfg, a.out_dtype)) {      // else the st.global epilogue (same bits)
             MMArgs t = a;
             t.store_mc = 3 | (1 << 8);
             t.ws = nullptr;

@@ -145,7 +145,7 @@ using namespace fp8b;
 extern "C" int fp8b_gemv_batch(const fp8b_gemv_item* items, int count, int K, int out_dtype, int bias_dtype, void* stream)
 {
     if (count < 0 || (count > 0 && !items) || K < 0) return FP8B_ERR_INVALID;
-    if (out_dtype < FP8B_F32 || out_dtype > FP8B_BF16) return FP8B_ERR_INVALID;
+    if (!valid_out_dtype(out_dtype)) return FP8B_ERR_INVALID;
     if (count == 0) return FP8B_OK;
     bool any_bias = false;
     for (int i = 0; i < count; ++i) {

@@ -96,6 +96,7 @@ __device__ __forceinline__ void epi_store(const Epi& e, int m, int n, float v) {
     const size_t idx = (size_t)m * e.ldc + n;
     if (e.out_dtype == FP8B_F32) reinterpret_cast<float*>(e.C)[idx] = v;
     else if (e.out_dtype == FP8B_F16) reinterpret_cast<__half*>(e.C)[idx] = __float2half_rn(v);
+    else if (e.out_dtype == FP8B_OUT_E4M3FN) reinterpret_cast<uint8_t*>(e.C)[idx] = enc1_f32(v);
     else reinterpret_cast<__nv_bfloat16*>(e.C)[idx] = __float2bfloat16_rn(v);
 }
 

@@ -99,7 +99,9 @@ def fp8_scaled_mm_fused(A, B, scale_a, scale_b, bias=None, scale_result=None, ou
     """`fp8_scaled_mm` with the epilogue the patch applies as separate torch ops
     (fp8_mps_patch.py:95-104: + bias, * scale_result, .to(out_dtype)) fused into the kernel.
     ``out`` may be a row-major (M,N) view with a wider row stride (a column shard of a bigger
-    matrix).  ``a_format`` / ``b_format``: "e4m3fn" (default; the reference codec, NaN bytes count as 0) or
+    matrix).  ``out_dtype=torch.float8_e4m3fn`` returns the reference encoder's bytes of the fp32 result, encoded in
+    the same kernel (what ``fp8_encode`` of the float32 output gives, at a quarter of its output traffic); float8_e5m2
+    is not an output dtype.  ``a_format`` / ``b_format``: "e4m3fn" (default; the reference codec, NaN bytes count as 0) or
     "e5m2" (decoded as e5m2 -- the reference mis-decodes such tensors as e4m3fn -- with IEEE inf/NaN)."""
     lib = _get_lib()
     assert A.dtype == torch.uint8 and B.dtype == torch.uint8

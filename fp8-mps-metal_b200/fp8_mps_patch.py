@@ -19,7 +19,8 @@ Deliberate differences from the reference (SURVEY Appendix B):
   * ``_metal_scaled_mm`` accepts scales positionally (the real aten schema) as well as by keyword
     (reference: keyword-only, fp8_mps_patch.py:53);
   * bias, scale_result and out_dtype are fused into the matmul kernel instead of three extra
-    elementwise passes (fp8_mps_patch.py:95-104);
+    elementwise passes (fp8_mps_patch.py:95-104); out_dtype=float8_e4m3fn gives the bytes the reference's
+    ``result.to(float8_e4m3fn)`` gives, encoded in the same kernel (float8_e5m2 output raises);
   * float8_e5m2 operands are decoded AS e5m2 (the reference sends them to its e4m3fn kernels and
     mis-decodes them, fp8_mps_patch.py:48-49,65); only decode exists: float -> e5m2 stays with torch;
   * FP8 -> float32/bfloat16 is one exact pass, not dequantise-to-fp16 then .to();

@@ -48,6 +48,13 @@ def shard_bounds(N: int, world: int, rank: int, align: int = 16) -> Tuple[int, i
     return n0, n1, width
 
 
+def _refuse_fp8_out(out_dtype) -> None:
+    """FP8 results are not exchanged between ranks yet: raise on every rank alike, before anything is launched or sent."""
+    if out_dtype in (torch.float8_e4m3fn, torch.float8_e5m2):
+        raise ValueError(f"ShardedScaledMM: out_dtype {out_dtype} is not supported (float32, float16 or bfloat16); "
+                         "the single-GPU fp8_scaled_mm_fused takes out_dtype=torch.float8_e4m3fn")
+
+
 def _default_mm(a, b, sa, sb, bias, out_dtype, out=None):
     import fp8_mps_native
     return fp8_mps_native.fp8_scaled_mm_fused(a, b, sa, sb, bias=bias, scale_result=None, out_dtype=out_dtype, out=out)
@@ -108,6 +115,7 @@ class ShardedScaledMM:
     # ------------------------------------------------------------------ NCCL all-gather path
     def __call__(self, x_u8: torch.Tensor, scale_a: torch.Tensor, out_dtype=torch.bfloat16,
                  layout: str = "row_major", mode: str = "allgather") -> torch.Tensor:
+        _refuse_fp8_out(out_dtype)
         if mode == "auto":
             mode = self.best_mode(x_u8.shape[0], x_u8.shape[1], out_dtype or torch.float32, x_u8.device) \
                 if layout == "row_major" else "allgather"
@@ -158,6 +166,7 @@ class ShardedScaledMM:
         call after next.  That is also what makes one barrier per call enough: a rank can only pass the
         closing barrier of call i-1 after every rank has ENTERED call i-1, i.e. finished with result i-2,
         whose buffer call i is about to overwrite."""
+        _refuse_fp8_out(out_dtype)
         import fp8_mps_native
         M = x_u8.shape[0]
         odt = out_dtype or torch.float32
@@ -181,6 +190,7 @@ class ShardedScaledMM:
         """Like forward_multicast, with peer stores: the GEMM epilogue writes every tile into this rank's buffer and
         into each peer's buffer (unicast over NVLink).  A rank's own shard never leaves the GPU, so the NVLink
         ingress per GPU is (w-1)/w of the output instead of all of it.  Same double-buffering and single barrier."""
+        _refuse_fp8_out(out_dtype)
         import fp8_mps_native
         M = x_u8.shape[0]
         odt = out_dtype or torch.float32
@@ -258,6 +268,7 @@ class ShardedScaledMM:
         CUDA-graph capturable once the symmetric buffers exist (call it once eagerly first); capture TWO graphs and
         replay them in turn if the double-buffering matters to the caller.  Do not let the last reference to a
         symmetric buffer die inside a capture (freeing one is not a capturable operation)."""
+        _refuse_fp8_out(out_dtype)
         import fp8_mps_native
         M, K = x_u8.shape
         odt = out_dtype or torch.float32

@@ -48,10 +48,14 @@ typedef enum fp8b_status {
     FP8B_ERR_NO_DEVICE = -4    /* current device is not compute capability 10.x */
 } fp8b_status;
 
+/* Element types.  FP8B_OUT_E4M3FN is an OUTPUT type of the matmul entry points only (1-byte elements, the reference
+ * codec's bytes of the fp32 epilogue value, exactly fp8b_encode with no prescale); every cast entry point, every
+ * bias_dtype and the x_dtype of fp8b_linear_dynamic reject it with FP8B_ERR_INVALID. */
 typedef enum fp8b_dtype {
     FP8B_F32 = 0,
     FP8B_F16 = 1,
-    FP8B_BF16 = 2
+    FP8B_BF16 = 2,
+    FP8B_OUT_E4M3FN = 3
 } fp8b_dtype;
 
 /* Which matmul kernel fp8b_scaled_mm() picked / should pick. */
@@ -218,7 +222,11 @@ FP8B_API int fp8b_quantize_rows(const void* in, int in_dtype, int rows, size_t c
  *   A            (M,K) uint8 row-major, contiguous (lda = K)
  *   B            (N,K) uint8 row-major, contiguous -- the reference's "pre-transposed" weight layout
  *   C            (M,N) out_dtype, row stride ldc elements (ldc >= N); ldc lets a rank write its column
- *                shard straight into a wider matrix
+ *                shard straight into a wider matrix.  out_dtype FP8B_OUT_E4M3FN: C[m,n] = enc(v) where v is the
+ *                fp32 value the same call computes for FP8B_F32 and enc is fp8b_encode's codec (saturate at
+ *                +-448, inf included; flush |v| < 2^-9; no carry into the exponent; -0.0 -> 0x00; NaN -> 0x7F).
+ *                Elements are 1 byte, so ldc counts bytes and every 16-byte rule below counts bytes.  The
+ *                kernel choice does not depend on out_dtype.  (float8_e5m2 output is not offered.)
  *   scale_a      device float[scale_a_len], scale_a_len in {1, M}   (independently of scale_b: fixes the
  *   scale_b      device float[scale_b_len], scale_b_len in {1, N}    reference's all-or-nothing scale_mode)
  *   bias         device [N] of bias_dtype, or NULL
@@ -318,7 +326,8 @@ FP8B_API size_t fp8b_scaled_mm_workspace_bytes(int M, int N, int K);
  * the switch replicates it into every GPU's copy while the next tile is being computed.
  * The caller orders ranks around the call (a barrier before reuse of the buffer and one after).
  * Requires N % 32 == 0, 16-byte aligned C_multicast / ldc / scale_b / bias, and the TMA alignment
- * rules of the tcgen05 kernel; otherwise FP8B_ERR_UNSUPPORTED.
+ * rules of the tcgen05 kernel; otherwise FP8B_ERR_UNSUPPORTED.  out_dtype FP8B_OUT_E4M3FN is FP8B_ERR_UNSUPPORTED
+ * here: the multicast store path can only be exercised on an NVSwitch group, so no byte output is offered on it.
  */
 FP8B_API int fp8b_scaled_mm_multicast(const uint8_t* A, const uint8_t* B, void* C_multicast, int out_dtype,
                              int M, int N, int K, int64_t ldc,
@@ -362,7 +371,9 @@ FP8B_API int fp8b_scaled_mm_peers(const uint8_t* A, const uint8_t* B, void* C_lo
  * next tile's MMAs.  Each GPU receives (world-1)/world of the output.  The caller orders ranks around the call (a
  * barrier before a buffer is reused and one after).  Needs 16-byte aligned A / B / every C_dsts[d], K % 16 == 0,
  * ldc * sizeof(out) % 16 == 0 and N * sizeof(out) % 16 == 0 (TMA stores move 16-byte units); otherwise any M, N -- TMA
- * clips the tile edges (fp8b_scaled_mm_push_supported).  Else FP8B_ERR_UNSUPPORTED.
+ * clips the tile edges (fp8b_scaled_mm_push_supported).  Else FP8B_ERR_UNSUPPORTED.  With FP8B_OUT_E4M3FN (1-byte
+ * elements: N % 16 == 0 and ldc % 16 == 0) a tile must also be a whole number of 128-column boxes, so the built-in tile
+ * rule never picks 256 x 192 for it and a forced FP8B_OPT_TUNE_GEMM_CFG 5 returns FP8B_ERR_UNSUPPORTED.
  */
 FP8B_API int fp8b_scaled_mm_push(const uint8_t* A, const uint8_t* B, void* const* C_dsts, int n_dst,
                         int out_dtype, int M, int N, int K, int64_t ldc,
