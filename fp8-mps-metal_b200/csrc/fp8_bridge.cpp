@@ -577,15 +577,15 @@ std::tuple<torch::Tensor, torch::Tensor> fp8_linear_dynamic(torch::Tensor x, tor
     if (M == 0 || N == 0) return std::make_tuple(C, inv);
     torch::Tensor ws;
     void* ws_ptr = nullptr;
-    size_t ws_bytes = 0;
+    size_t workspace_bytes = 0;
     if (!single_kernel) {
-        ws_bytes = fp8b_linear_dynamic_workspace_bytes((int)M, (int)K);
-        ws = torch::empty({(int64_t)ws_bytes}, torch::TensorOptions().dtype(torch::kUInt8).device(x.device()));
+        workspace_bytes = fp8b_linear_dynamic_workspace_bytes((int)M, (int)K);
+        ws = torch::empty({(int64_t)workspace_bytes}, torch::TensorOptions().dtype(torch::kUInt8).device(x.device()));
         ws_ptr = ws.data_ptr();
     }
     int rc = fp8b_linear_dynamic(xin.data_ptr(), to_fp8b_dtype(xin.scalar_type()), u8_ptr(B), C.data_ptr(), to_fp8b_out_dtype(odt),
                                (int)M, (int)N, (int)K, N, sb.data_ptr<float>(), (int)sb.numel(), bias_ptr, bias_dt, nullptr,
-                               inv.data_ptr<float>(), ws_ptr, ws_bytes, current_stream());
+                               inv.data_ptr<float>(), ws_ptr, workspace_bytes, current_stream());
     check_status(rc, "fp8b_linear_dynamic");
     return std::make_tuple(C, inv);
 }

@@ -74,6 +74,48 @@ static int select_algo(const MMArgs& a)
     return FP8B_MM_SIMT;
 }
 
+static int launch_algo(const MMArgs& a, int algo)
+{
+    switch (algo == FP8B_MM_AUTO ? select_algo(a) : algo) {
+        case FP8B_MM_GEMV: return launch_gemv(a);
+        case FP8B_MM_TCGEN05: return launch_gemm_tcgen05(a);
+        case FP8B_MM_SIMT: return launch_gemm_simt(a);
+        default: return FP8B_ERR_INVALID;
+    }
+}
+
+// The arguments every scaled-matmul entry point shares; the result stores to C (Store::Local).
+static MMArgs mm_args(const uint8_t* A, const uint8_t* B, void* C, int out_dtype, int M, int N, int K, int64_t ldc,
+                      const float* scale_a, int scale_a_len, const float* scale_b, int scale_b_len,
+                      const void* bias, int bias_dtype, const float* scale_result, void* stream)
+{
+    MMArgs a;
+    a.A = A; a.B = B; a.C = C; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
+    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
+    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
+    a.st = (cudaStream_t)stream;
+    return a;
+}
+
+// The exchange entry points (multicast, peers, push): tcgen05 only, no fallback.  `empty` is the status of an
+// empty shard (M == 0 or N == 0).
+static int launch_exchange(const MMArgs& a, int empty)
+{
+    int rc = validate(a);
+    if (rc != FP8B_OK) return rc;
+    if (a.M == 0 || a.N == 0) return empty;
+    if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
+    return launch_gemm_tcgen05(a);          // FP8B_ERR_UNSUPPORTED unless tcgen05_supported(a)
+}
+
+static bool valid_dsts(void* const* dsts, int n_dst)
+{
+    if (n_dst < 1 || n_dst > 8 || !dsts) return false;
+    for (int d = 0; d < n_dst; ++d)
+        if (!dsts[d]) return false;
+    return true;
+}
+
 }  // namespace fp8b
 
 using namespace fp8b;
@@ -131,19 +173,13 @@ extern "C" int fp8b_scaled_mm_select(const uint8_t* A, const uint8_t* B, const v
     return select_algo(a);
 }
 
-static int scaled_mm_impl(MMArgs& a, int algo)
+static int scaled_mm_impl(const MMArgs& a, int algo)
 {
     int rc = validate(a);
     if (rc != FP8B_OK) return rc;
     if (a.M == 0 || a.N == 0) return FP8B_OK;
     if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
-    if (algo == FP8B_MM_AUTO) algo = select_algo(a);
-    switch (algo) {
-        case FP8B_MM_GEMV: return launch_gemv(a);
-        case FP8B_MM_TCGEN05: return launch_gemm_tcgen05(a);
-        case FP8B_MM_SIMT: return launch_gemm_simt(a);
-        default: return FP8B_ERR_INVALID;
-    }
+    return launch_algo(a, algo);
 }
 
 extern "C" int fp8b_scaled_mm(const uint8_t* A, const uint8_t* B, void* C, int out_dtype,
@@ -152,16 +188,11 @@ extern "C" int fp8b_scaled_mm(const uint8_t* A, const uint8_t* B, void* C, int o
                               const float* scale_b, int scale_b_len,
                               const void* bias, int bias_dtype,
                               const float* scale_result,
-                              void* workspace, size_t workspace_bytes,
+                              void* /*workspace*/, size_t /*workspace_bytes*/,     // no kernel needs one
                               int algo, void* stream)
 {
-    MMArgs a;
-    a.A = A; a.B = B; a.C = C; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = workspace; a.ws_bytes = workspace_bytes; a.st = (cudaStream_t)stream;
-    a.store_mc = 0;
-    return scaled_mm_impl(a, algo);
+    return scaled_mm_impl(mm_args(A, B, C, out_dtype, M, N, K, ldc, scale_a, scale_a_len, scale_b, scale_b_len,
+                                  bias, bias_dtype, scale_result, stream), algo);
 }
 
 extern "C" int fp8b_scaled_mm_fmt(const uint8_t* A, int a_format, const uint8_t* B, int b_format, void* C, int out_dtype,
@@ -174,12 +205,8 @@ extern "C" int fp8b_scaled_mm_fmt(const uint8_t* A, int a_format, const uint8_t*
 {
     if ((a_format != FP8B_E4M3FN && a_format != FP8B_E5M2) || (b_format != FP8B_E4M3FN && b_format != FP8B_E5M2))
         return FP8B_ERR_INVALID;
-    MMArgs a;
-    a.A = A; a.B = B; a.C = C; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = nullptr; a.ws_bytes = 0; a.st = (cudaStream_t)stream;
-    a.store_mc = 0;
+    MMArgs a = mm_args(A, B, C, out_dtype, M, N, K, ldc, scale_a, scale_a_len, scale_b, scale_b_len, bias, bias_dtype,
+                       scale_result, stream);
     a.a_fmt = a_format; a.b_fmt = b_format;
     return scaled_mm_impl(a, algo);
 }
@@ -191,18 +218,12 @@ extern "C" int fp8b_scaled_mm_multicast(const uint8_t* A, const uint8_t* B, void
                                         const void* bias, int bias_dtype,
                                         const float* scale_result, void* stream)
 {
-    MMArgs a;
-    a.A = A; a.B = B; a.C = C_multicast; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = nullptr; a.ws_bytes = 0; a.st = (cudaStream_t)stream;
-    a.store_mc = 1;
-    int rc = validate(a);
-    if (rc != FP8B_OK) return rc;
-    if (out_dtype == FP8B_OUT_E4M3FN) return FP8B_ERR_UNSUPPORTED;    // no byte output through the multicast mapping
-    if (M == 0 || N == 0) return FP8B_OK;
-    if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
-    return launch_gemm_tcgen05(a);
+    MMArgs a = mm_args(A, B, C_multicast, out_dtype, M, N, K, ldc, scale_a, scale_a_len, scale_b, scale_b_len, bias,
+                       bias_dtype, scale_result, stream);
+    a.store = Store::Multicast;
+    // no byte output through the multicast mapping
+    if (out_dtype == FP8B_OUT_E4M3FN && validate(a) == FP8B_OK) return FP8B_ERR_UNSUPPORTED;
+    return launch_exchange(a, FP8B_OK);
 }
 
 static size_t align16(size_t v) { return (v + 15) & ~(size_t)15; }
@@ -232,12 +253,9 @@ extern "C" int fp8b_linear_dynamic(const void* X, int x_dtype, const uint8_t* B,
     const bool vec_ok = K >= 16 && (K % 16) == 0 && aligned(B, 16) && aligned(X, 16);
     if (M <= 16 && !have_ws && !vec_ok) return FP8B_ERR_UNSUPPORTED;
     if (M > 16 && !have_ws) return FP8B_ERR_UNSUPPORTED;         // the GEMM path always quantises into the workspace
-    MMArgs a;
-    a.A = nullptr; a.B = B; a.C = C; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_b; a.sa_len = 1;                 // replaced below / unused by the single-kernel path
-    a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = nullptr; a.ws_bytes = 0; a.st = (cudaStream_t)stream; a.store_mc = 0;
+    // A and scale_a: set below (workspace plans) / unused (single-kernel plan)
+    MMArgs a = mm_args(nullptr, B, C, out_dtype, M, N, K, ldc, scale_b, 1, scale_b, scale_b_len, bias, bias_dtype,
+                       scale_result, stream);
 
     // Two plans.  With a workspace: quantise once (one CTA per row) and chain the GEMV behind it with
     // programmatic dependent launch -- the GEMV is resident and already streaming its first weight vectors
@@ -254,10 +272,7 @@ extern "C" int fp8b_linear_dynamic(const void* X, int x_dtype, const uint8_t* B,
         int rc = fp8b_quantize_rows(X, x_dtype, M, (size_t)K, q, inv, stream);
         if (rc != FP8B_OK) return rc;
         a.A = q; a.sa = inv; a.sa_len = M;
-        if (M > 16) {
-            const int algo = select_algo(a);
-            return algo == FP8B_MM_TCGEN05 ? launch_gemm_tcgen05(a) : algo == FP8B_MM_GEMV ? launch_gemv(a) : launch_gemm_simt(a);
-        }
+        if (M > 16) return launch_algo(a, FP8B_MM_AUTO);
         a.chain_pdl = 1;
         return launch_gemv(a);
     }
@@ -273,18 +288,10 @@ extern "C" int fp8b_scaled_mm_peers(const uint8_t* A, const uint8_t* B, void* C_
                                     const float* scale_result, void* stream)
 {
     if (world < 2 || world > 8 || !peer_deltas) return FP8B_ERR_INVALID;
-    MMArgs a;
-    a.A = A; a.B = B; a.C = C_local; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = const_cast<int64_t*>(peer_deltas); a.ws_bytes = (size_t)world * sizeof(int64_t); a.st = (cudaStream_t)stream;
-    a.store_mc = 2 | (world << 8);
-    int rc = validate(a);
-    if (rc != FP8B_OK) return rc;
-    if (M == 0 || N == 0) return FP8B_OK;
-    if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
-    if (!tcgen05_supported(a)) return FP8B_ERR_UNSUPPORTED;
-    return launch_gemm_tcgen05(a);
+    MMArgs a = mm_args(A, B, C_local, out_dtype, M, N, K, ldc, scale_a, scale_a_len, scale_b, scale_b_len, bias,
+                       bias_dtype, scale_result, stream);
+    a.store = Store::Peers; a.n_dst = world; a.peer_deltas = peer_deltas;
+    return launch_exchange(a, FP8B_OK);
 }
 
 // N-sharded linear, fused compute + exchange with TMA stores: see include/fp8_b200.h.
@@ -295,21 +302,11 @@ extern "C" int fp8b_scaled_mm_push(const uint8_t* A, const uint8_t* B, void* con
                                    const void* bias, int bias_dtype,
                                    const float* scale_result, void* stream)
 {
-    if (n_dst < 1 || n_dst > 8 || !C_dsts) return FP8B_ERR_INVALID;
-    for (int d = 0; d < n_dst; ++d)
-        if (!C_dsts[d]) return FP8B_ERR_INVALID;
-    MMArgs a;
-    a.A = A; a.B = B; a.C = C_dsts[0]; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = const_cast<void**>(C_dsts); a.ws_bytes = (size_t)n_dst * sizeof(void*); a.st = (cudaStream_t)stream;
-    a.store_mc = 3 | (n_dst << 8);
-    int rc = validate(a);
-    if (rc != FP8B_OK) return rc;
-    if (M == 0 || N == 0) return FP8B_OK;
-    if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
-    if (!tcgen05_supported(a)) return FP8B_ERR_UNSUPPORTED;
-    return launch_gemm_tcgen05(a);
+    if (!valid_dsts(C_dsts, n_dst)) return FP8B_ERR_INVALID;
+    MMArgs a = mm_args(A, B, C_dsts[0], out_dtype, M, N, K, ldc, scale_a, scale_a_len, scale_b, scale_b_len, bias,
+                       bias_dtype, scale_result, stream);
+    a.store = Store::Push; a.n_dst = n_dst; a.dsts = C_dsts;
+    return launch_exchange(a, FP8B_OK);
 }
 
 extern "C" int fp8b_scaled_mm_push_signal(const uint8_t* A, const uint8_t* B, void* const* C_dsts, int n_dst,
@@ -319,26 +316,17 @@ extern "C" int fp8b_scaled_mm_push_signal(const uint8_t* A, const uint8_t* B, vo
                                           const void* bias, int bias_dtype, const float* scale_result,
                                           uint64_t* const* signal_flags, uint32_t* cta_counter, uint64_t epoch, void* stream)
 {
-    if (n_dst < 1 || n_dst > 8 || !C_dsts || !signal_flags || !cta_counter) return FP8B_ERR_INVALID;
-    for (int d = 0; d < n_dst; ++d)
-        if (!C_dsts[d]) return FP8B_ERR_INVALID;
+    if (!valid_dsts(C_dsts, n_dst) || !signal_flags || !cta_counter) return FP8B_ERR_INVALID;
     PushSignal sig;
     for (int d = 0; d < 8; ++d) sig.flags[d] = d < n_dst ? signal_flags[d] : nullptr;
     sig.cta_counter = cta_counter;
     sig.epoch = epoch;
-    MMArgs a;
-    a.A = A; a.B = B; a.C = C_dsts[0]; a.out_dtype = out_dtype; a.M = M; a.N = N; a.K = K; a.ldc = ldc;
-    a.sa = scale_a; a.sa_len = scale_a_len; a.sb = scale_b; a.sb_len = scale_b_len;
-    a.bias = bias; a.bias_dtype = bias_dtype; a.sr = scale_result;
-    a.ws = const_cast<void**>(C_dsts); a.ws_bytes = (size_t)n_dst * sizeof(void*); a.st = (cudaStream_t)stream;
-    a.store_mc = 3 | (n_dst << 8);
+    MMArgs a = mm_args(A, B, C_dsts[0], out_dtype, M, N, K, ldc, scale_a, scale_a_len, scale_b, scale_b_len, bias,
+                       bias_dtype, scale_result, stream);
+    a.store = Store::Push; a.n_dst = n_dst; a.dsts = C_dsts;
     a.sig = &sig;
-    int rc = validate(a);
-    if (rc != FP8B_OK) return rc;
-    if (M == 0 || N == 0) return FP8B_ERR_UNSUPPORTED;        // an empty shard cannot signal: the caller uses fp8b_peer_signal
-    if (!device_info().ok) return FP8B_ERR_NO_DEVICE;
-    if (!tcgen05_supported(a)) return FP8B_ERR_UNSUPPORTED;
-    return launch_gemm_tcgen05(a);
+    // an empty shard cannot signal: the caller uses fp8b_peer_signal
+    return launch_exchange(a, FP8B_ERR_UNSUPPORTED);
 }
 
 extern "C" int fp8b_peer_wait(const uint64_t* flags, int world, int rank, uint64_t epoch, void* stream)

@@ -122,12 +122,14 @@ struct GemmParams {
     Epi epi;
     int vec_store_ok;                        // C base and ldc allow 16-byte row-chunk stores
     int col_vec_ok;                          // scale_b / bias bases allow 16-byte broadcast loads
-    int store_mc;                            // bits 0-7: 1 = C is an NVSwitch multicast address (multimem.st);
-                                             // bits 8+: number of destinations (kStPeers / kStTma)
-    long long* aux;                          // kStPeers: device table of per-rank byte deltas.  FP8B_PROFILE builds,
-                                             // FP8B_GEMM_DEBUG & 16: per-tile clock64 stamps of CTA 0
-    int debug;                               // bits 0-7: FP8B_GEMM_DEBUG profiling knob (FP8B_PROFILE builds only);
-                                             // bit 8 / bit 9: A / B operand is e5m2
+    int multicast;                           // kStDirect: C is an NVSwitch multicast address (multimem.st)
+    int n_dst;                               // kStPeers: world size; kStTma: number of destinations
+    const long long* peer_delta;             // kStPeers: device table of per-rank byte offsets from C
+    int a_fmt, b_fmt;                        // operand formats: 0 = e4m3, 1 = e5m2
+#ifdef FP8B_PROFILE
+    long long* dbg;                          // FP8B_GEMM_DEBUG & 16: per-tile clock64 stamps of CTA 0 (else null)
+    int debug;                               // FP8B_GEMM_DEBUG bits
+#endif
 };
 
 // ------------------------------------------------------------------------------ PTX wrappers
@@ -267,7 +269,7 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t smem_addr) {
 }
 
 // Instruction descriptor for kind::f8f6f4: D = f32 (bits 4-5 = 1), A format at [7,10), B format at [10,13)
-// (0 = e4m3, 1 = e5m2; OR-ed in at run time from GemmParams::debug bits 8/9), both K-major (bits 15,16 = 0),
+// (0 = e4m3, 1 = e5m2; OR-ed in at run time from GemmParams::a_fmt / b_fmt), both K-major (bits 15,16 = 0),
 // N >> 3 at [17,23), M >> 4 at [24,29).
 __host__ __device__ constexpr uint32_t make_idesc(int m, int n) {
     return (1u << 4) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
@@ -475,7 +477,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
     using Cfg = GemmCfg<BN, CG, MODE>;
     constexpr bool PEERS = MODE == kStPeers;
 #ifdef FP8B_PROFILE
-    long long* const dbg = PEERS ? nullptr : p.aux;  // (PEERS: the field carries the peer delta table instead)
+    long long* const dbg = p.dbg;
 #endif
     constexpr int kTileM = kBM * CG;                 // rows of C per tile (per CTA pair when CG == 2)
     const uint32_t cta_rank = (CG == 2) ? cluster_ctarank() : 0u;
@@ -588,7 +590,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
         // tensor pipe may have to absorb (measured: a 90-instruction body cost 15 % of MMA throughput).
         if (is_leader) {
             constexpr uint32_t idesc = make_idesc(kTileM, BN);
-            const uint32_t idesc_fmt = (((uint32_t)p.debug >> 8) & 1u) << 7 | (((uint32_t)p.debug >> 9) & 1u) << 10;
+            const uint32_t idesc_fmt = (uint32_t)p.a_fmt << 7 | (uint32_t)p.b_fmt << 10;
             const bool elected = elect_one();
             const uint64_t desc_a0 = make_smem_desc(smem_base);
             const uint64_t desc_b0 = make_smem_desc(smem_base + Cfg::kABytes);
@@ -643,7 +645,6 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
         // finished READING shared memory (the writes themselves stay in flight).
         if constexpr (MODE == kStTma) {
             const bool elected = elect_one();
-            const int n_dst = p.store_mc >> 8;
             const int esz = out_esz(p.epi.out_dtype);
             const int cols_per_box = 128 / esz;
             uint32_t seq = 0;
@@ -658,7 +659,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                     if (elected) {
                         if (m_idx < p.M) {
                             const uint32_t src = stage_base + slot * kStoreBoxBytes;
-                            for (int d = 0; d < n_dst; ++d) tma_store_2d(&smaps.m[d], src, n_box * esz, m_idx);
+                            for (int d = 0; d < p.n_dst; ++d) tma_store_2d(&smaps.m[d], src, n_box * esz, m_idx);
                         }
                         bulk_commit_group();
                         bulk_wait_group_read<kStoreInflight>();
@@ -683,6 +684,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
             const int q = warp & 3;
             const int row_in_tile = q * 32 + lane;
             const Epi& e = p.epi;
+            const int a_fmt = p.a_fmt, b_fmt = p.b_fmt;
             const float sr = e.sr ? *e.sr : 1.0f;
             const float sb0 = e.sb[0];
             const int esz = out_esz(e.out_dtype);
@@ -748,7 +750,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
 #pragma unroll
                                 for (int j = 0; j < 32; ++j) t[j] = r[j];
                                 if (m_ok) fix_nan_chunk(t, p.A + (size_t)m * p.K, p.B + (size_t)n0 * p.K, p.K, p.N - n0,
-                                                        (p.debug >> 8) & 1, (p.debug >> 9) & 1);
+                                                        a_fmt, b_fmt);
 #pragma unroll
                                 for (int j = 0; j < 32; ++j) r[j] = t[j];
                             }
@@ -815,10 +817,10 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
         const float sr = e.sr ? *e.sr : 1.0f;
         const float sb0 = e.sb[0];
         long long peer_delta[8];                     // PEERS: byte offset of every rank's buffer from the local one (0 = self)
-        const int peer_world = PEERS ? (p.store_mc >> 8) : 0;
+        const int peer_world = PEERS ? p.n_dst : 0;
         if (PEERS) {
 #pragma unroll
-            for (int r = 0; r < 8; ++r) peer_delta[r] = r < peer_world ? p.aux[r] : 0;
+            for (int r = 0; r < 8; ++r) peer_delta[r] = r < peer_world ? p.peer_delta[r] : 0;
         }
         auto store16 = [&](void* ptr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
             if (PEERS) {
@@ -826,7 +828,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                 for (int r = 0; r < 8; ++r)
                     if (r < peer_world) stg_v4(reinterpret_cast<uint8_t*>(ptr) + peer_delta[r], a, b, c, d, 0);
             } else {
-                stg_v4(ptr, a, b, c, d, p.store_mc & 1);
+                stg_v4(ptr, a, b, c, d, p.multicast);
             }
         };
         int acc = 0; uint32_t acc_phase = 0;
@@ -876,7 +878,7 @@ fp8_gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a,
                         const float a = __uint_as_float(r[j]);
                         if (a != a && m_ok && n0 + j < p.N)
                             r[j] = __float_as_uint(slow_dot_fmt(p.A + (size_t)m * p.K, p.B + (size_t)(n0 + j) * p.K, p.K,
-                                                                (p.debug >> 8) & 1, (p.debug >> 9) & 1));
+                                                                p.a_fmt, p.b_fmt));
                     }
                 }
                 if (full_chunk && p.vec_store_ok) {
@@ -1361,7 +1363,7 @@ static bool tma_store_ok(const MMArgs& a, void* const* dsts, int n_dst)
     // store would write past column N (seen: three columns of a neighbour's shard zeroed)
     if (((size_t)a.N * esz) % 16 != 0) return false;
     for (int d = 0; d < n_dst; ++d)
-        if (!dsts[d] || !aligned(dsts[d], 16)) return false;
+        if (!aligned(dsts[d], 16)) return false;
     return true;
 }
 
@@ -1370,7 +1372,7 @@ static void fill_signal(StoreMaps& sm, const MMArgs& a)
     sm.n_sig = 0; sm.cta_counter = nullptr; sm.epoch = 0;
     for (int d = 0; d < kMaxDst; ++d) sm.sig[d] = nullptr;
     if (!a.sig) return;
-    sm.n_sig = a.store_mc >> 8;
+    sm.n_sig = a.n_dst;
     for (int d = 0; d < sm.n_sig; ++d) sm.sig[d] = reinterpret_cast<unsigned long long*>(a.sig->flags[d]);
     sm.cta_counter = a.sig->cta_counter;
     sm.epoch = a.sig->epoch;
@@ -1433,74 +1435,48 @@ static int launch_tcgen05_cfg(const MMArgs& a)
     p.epi = make_epi(a);
     p.vec_store_ok = aligned(a.C, 16) && ((a.ldc * esz) % 16 == 0);
     p.col_vec_ok = (a.sb_len == 1 || aligned(a.sb, 16)) && (!a.bias || aligned(a.bias, 16));
-    p.debug = (a.a_fmt ? 0x100 : 0) | (a.b_fmt ? 0x200 : 0);
-    p.store_mc = a.store_mc;
-    p.aux = nullptr;
+    p.multicast = a.store == Store::Multicast;
+    p.n_dst = a.n_dst;
+    p.peer_delta = reinterpret_cast<const long long*>(a.peer_deltas);
+    p.a_fmt = a.a_fmt; p.b_fmt = a.b_fmt;
     p.stage_tx = a_box_rows * kBK + Cfg::kBBytes;
     typename StoreMapsOf<MODE>::type smaps;
-    if constexpr (MODE == kStPeers) {        // store_mc = 2 | world << 8; a.ws = device table of world byte deltas
-        p.aux = static_cast<long long*>(a.ws);
-    } else if constexpr (MODE == kStTma) {   // store_mc = 3 | n_dst << 8; a.ws = HOST array of n_dst destination pointers
-        const int n_dst = a.store_mc >> 8;
-        void* const* dsts = static_cast<void* const*>(a.ws);
-        void* self[1] = {a.C};
-        if (!dsts) dsts = self;
+    if constexpr (MODE == kStTma) {
         // (BN * esz) % 128: a tile must be whole 128-byte boxes, or a box store would cover the next tile's columns
-        if (n_dst < 1 || n_dst > kMaxDst || !tma_store_ok(a, dsts, n_dst) || (BN * esz) % 128 != 0) return FP8B_ERR_UNSUPPORTED;
-        for (int d = 0; d < n_dst; ++d)
-            if (!get_tensor_map(&smaps.m[d], dsts[d], (uint64_t)a.M, (uint64_t)a.N * esz, (uint64_t)a.ldc * esz, 128, 128))
+        if (!tma_store_ok(a, a.dsts, a.n_dst) || (BN * esz) % 128 != 0) return FP8B_ERR_UNSUPPORTED;
+        for (int d = 0; d < a.n_dst; ++d)
+            if (!get_tensor_map(&smaps.m[d], a.dsts[d], (uint64_t)a.M, (uint64_t)a.N * esz, (uint64_t)a.ldc * esz, 128, 128))
                 return FP8B_ERR_CUDA;
-        for (int d = n_dst; d < kMaxDst; ++d) smaps.m[d] = smaps.m[0];
+        for (int d = a.n_dst; d < kMaxDst; ++d) smaps.m[d] = smaps.m[0];
         fill_signal(smaps, a);
     } else {
         smaps.unused = 0;
     }
 #ifdef FP8B_PROFILE
-    if constexpr (MODE != kStPeers) {
-        p.debug |= tune_int("FP8B_GEMM_DEBUG", 0) & 0xFF;
-        if (p.debug & 16) {                  // profiling only: allocates and synchronises
-            static long long* dbuf = nullptr;
-            if (!dbuf) cudaMalloc(&dbuf, 64 * 8 * sizeof(long long));
-            cudaMemset(dbuf, 0, 64 * 8 * sizeof(long long));
-            p.aux = dbuf;
-        }
+    p.debug = tune_int("FP8B_GEMM_DEBUG", 0);
+    p.dbg = nullptr;
+    if (p.debug & 16) {                      // profiling only: allocates and synchronises
+        static long long* dbuf = nullptr;
+        if (!dbuf) cudaMalloc(&dbuf, 64 * 8 * sizeof(long long));
+        cudaMemset(dbuf, 0, 64 * 8 * sizeof(long long));
+        p.dbg = dbuf;
     }
 #endif
     // multimem.st / peer stores have no sub-word form: both modes need every chunk on the 16-byte path
-    if (!is_push<MODE>() && a.store_mc && !(p.vec_store_ok && p.col_vec_ok && a.N % 32 == 0)) return FP8B_ERR_UNSUPPORTED;
+    if (!is_push<MODE>() && a.store != Store::Local && !(p.vec_store_ok && p.col_vec_ok && a.N % 32 == 0))
+        return FP8B_ERR_UNSUPPORTED;
 
-    const int tiles = p.num_work;
-    const int workers_max = workers_cap;                            // one CTA (or CTA pair) per SM (pair)
-    const int workers = tiles < workers_max ? tiles : workers_max;
-
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(workers * CG, 1, 1);
-    cfg.blockDim = dim3(gemm_threads<MODE>(), 1, 1);
-    cfg.dynamicSmemBytes = Cfg::kSmemBytes;
-    cfg.stream = a.st;
-    cudaLaunchAttribute attr[3];
-    int nattr = 0;
-    if (CG > 1) {
-        attr[nattr].id = cudaLaunchAttributeClusterDimension;
-        attr[nattr].val.clusterDim.x = CG; attr[nattr].val.clusterDim.y = 1; attr[nattr].val.clusterDim.z = 1;
-        ++nattr;
-    }
+    const int workers = p.num_work < workers_cap ? p.num_work : workers_cap;      // one CTA (or CTA pair) per SM (pair)
     // Programmatic dependent launch (FP8B_OPT_PDL): the prologue overlaps the predecessor's tail.  Worth nothing on C4
     // (104.17 vs 104.12 us back to back: power-limited, idle gaps only buy clock) but a fixed ~2 us on small problems.
-    if (g_opt_pdl.load(std::memory_order_relaxed)) {
-        attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[nattr].val.programmaticStreamSerializationAllowed = 1;
-        ++nattr;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = nattr;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, fp8_gemm_tcgen05_kernel<BN, CG, MODE>, tmap_a, tmap_b, smaps, p);
-    if (e != cudaSuccess) return cuda_fail(e);
+    const int rc = launch_ex(fp8_gemm_tcgen05_kernel<BN, CG, MODE>, dim3(workers * CG), dim3(gemm_threads<MODE>()),
+                             Cfg::kSmemBytes, a.st, CG, 1, g_opt_pdl.load(std::memory_order_relaxed) != 0,
+                             tmap_a, tmap_b, smaps, p);
 #ifdef FP8B_PROFILE
-    if (MODE != kStPeers && p.aux) {
+    if (rc == FP8B_OK && p.dbg) {
         long long h[64 * 8];
         cudaDeviceSynchronize();
-        cudaMemcpy(h, p.aux, sizeof(h), cudaMemcpyDeviceToHost);
+        cudaMemcpy(h, p.dbg, sizeof(h), cudaMemcpyDeviceToHost);
         printf("CTA 0: kernel entry -> first MMA wait %lld cycles; last epilogue end -> stores complete %lld; -> CTA end %lld\n",
                h[0] - h[7], h[15] ? h[15] - h[23] : 0, h[31] - (h[15] ? h[15] : h[23]));
         printf("tile | mma: wait_tempty  issue+run (of which waiting for TMA) | epi: wait_tfull  drain+store | epi_end - mma_end\n");
@@ -1510,7 +1486,7 @@ static int launch_tcgen05_cfg(const MMArgs& a)
                    h[t * 8 + 6] - h[t * 8 + 2], h[t * 8 + 0] - h[0]);
     }
 #endif
-    return after_launch();
+    return rc;
 }
 
 // Split-K plan (fp8_gemm_splitk_kernel): clusters of S CTAs, one 128 x 128 tile each.
@@ -1545,27 +1521,10 @@ static int launch_splitk(const MMArgs& a)
 #endif
     const long tiles = (long)((a.M + kBM - 1) / kBM) * p.num_n_blocks;
     if (p.num_k_blocks < S || tiles * S > 65535L * 16) return FP8B_ERR_UNSUPPORTED;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(tiles * S), 1, 1);
-    cfg.blockDim = dim3(kSkThreads, 1, 1);
-    cfg.dynamicSmemBytes = kSkSmemBytes;
-    cfg.stream = a.st;
-    cudaLaunchAttribute attr[2];
-    int nattr = 0;
-    attr[nattr].id = cudaLaunchAttributeClusterDimension;
-    attr[nattr].val.clusterDim.x = S; attr[nattr].val.clusterDim.y = 1; attr[nattr].val.clusterDim.z = 1;
-    ++nattr;
-    if (g_opt_pdl.load(std::memory_order_relaxed)) {
-        attr[nattr].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[nattr].val.programmaticStreamSerializationAllowed = 1;
-        ++nattr;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = nattr;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, fp8_gemm_splitk_kernel<S>, tmap_a, tmap_b, p);
-    if (e != cudaSuccess) return cuda_fail(e);
+    const int rc = launch_ex(fp8_gemm_splitk_kernel<S>, dim3((unsigned)(tiles * S)), dim3(kSkThreads), kSkSmemBytes, a.st, S, 1,
+                             g_opt_pdl.load(std::memory_order_relaxed) != 0, tmap_a, tmap_b, p);
 #ifdef FP8B_PROFILE
-    if (p.dbg) {
+    if (rc == FP8B_OK && p.dbg) {
         long long h[8];
         cudaDeviceSynchronize();
         cudaMemcpy(h, p.dbg, sizeof(h), cudaMemcpyDeviceToHost);
@@ -1574,7 +1533,7 @@ static int launch_splitk(const MMArgs& a)
                h[6] - h[5]);
     }
 #endif
-    return after_launch();
+    return rc;
 }
 
 // How many CTAs should share one tile (0 = the ordinary plans).  Split K when all clusters fit on the GPU at once and K
@@ -1606,10 +1565,10 @@ static bool tile_whole_boxes(int cfg, int out_dtype)
     return (width * dtype_size(out_dtype)) % 128 == 0;
 }
 
-// no_192: leave 256x192 out of the choice (a TMA-store epilogue that cannot take it)
-static int pick_tile_cfg(const MMArgs& a, bool pairs_only = false, bool no_192 = false)
+static int pick_tile_cfg(const MMArgs& a)
 {
     const int sms = device_info().sm_count;
+    const bool pairs_only = a.store == Store::Peers;         // the peer-store plan exists for CTA pairs only
     // Small problems (one round of 128 x 128 tiles, or two short ones): one-CTA tiles.  A CTA pair spends ~1 300 more cycles
     // in its prologue (cluster barrier) and its larger tile leaves a longer exposed epilogue; measured (us, chosen pair
     // config -> 128 x 128): 512^3 4.9 -> 4.4, 1024^3 6.2 -> 5.7, 2048 x 512 x 2048 8.5 -> 7.2, M=333 K=N=4096 13.1 -> 12.1;
@@ -1621,6 +1580,12 @@ static int pick_tile_cfg(const MMArgs& a, bool pairs_only = false, bool no_192 =
         // hand-over, pipeline fill) plus a part proportional to K that was measured at K = 3072 as 10.5 / 9.3 / 8.65 us
         // per tile for widths 256 / 192 / 128 (L2->SM traffic of the operands, not MMA time, dominates, so narrow
         // tiles are barely cheaper).  Only the ratios matter.
+        // Pushing to peers the kernel is bound by NVLink, not by the tensor pipe, and the link idles until the first tiles
+        // are complete: narrower tiles (256 x 128) halve that ramp at no cost in exchange time (measured at w = 2:
+        // 103.4 us against 106.4 us with 256 x 256 tiles; profiles/r2_scaling.md).
+        if (a.store == Store::Push && a.n_dst > 1) return 4;
+        // a push whose TMA-store boxes do not tile 256x192 leaves that configuration out
+        const bool no_192 = a.store == Store::Push && !tile_whole_boxes(5, a.out_dtype);
         const long mt = (a.M + 255) / 256;
         const int pairs = sms / 2;
         const double kf = (double)a.K / 3072.0;
@@ -1639,6 +1604,19 @@ static int pick_tile_cfg(const MMArgs& a, bool pairs_only = false, bool no_192 =
     return (a.N > 128 && t_256 >= 2L * sms) ? 1 : 2;
 }
 
+// Tile configuration -> kernel instantiation.  The peer-store epilogue is built for the CTA-pair configurations only.
+template <int MODE>
+static int launch_cfg(int cfg, const MMArgs& a)
+{
+    switch (cfg) {
+        case 3: return launch_tcgen05_cfg<256, 2, MODE>(a);
+        case 4: return launch_tcgen05_cfg<128, 2, MODE>(a);
+        case 5: return launch_tcgen05_cfg<192, 2, MODE>(a);
+    }
+    if constexpr (MODE == kStPeers) return FP8B_ERR_UNSUPPORTED;
+    else return cfg == 1 ? launch_tcgen05_cfg<256, 1, MODE>(a) : launch_tcgen05_cfg<128, 1, MODE>(a);
+}
+
 int launch_gemm_tcgen05(const MMArgs& a)
 {
     if (!tcgen05_supported(a)) return FP8B_ERR_UNSUPPORTED;
@@ -1646,58 +1624,25 @@ int launch_gemm_tcgen05(const MMArgs& a)
     // 256-wide when that still leaves >= ~2 waves of tiles, else 128-wide (finer tail).
     // fp8b_set_option(FP8B_OPT_TUNE_GEMM_CFG) -- a result-neutral tuning knob -- forces one.
     const int forced = tune(kTuneGemmCfg, 0);
-    const int mode = a.store_mc & 0xFF;
-    int cfg = forced ? forced : pick_tile_cfg(a, /*pairs_only=*/mode == 2,      // (the round-1 peer-store plan exists for CTA pairs only)
-                                              /*no_192=*/mode == 3 && !tile_whole_boxes(5, a.out_dtype));
-    if (mode == 0 && !forced) {               // plain call: few tiles and a long K -> several CTAs per tile
+    const int cfg = forced ? forced : pick_tile_cfg(a);
+    switch (a.store) {
+        case Store::Multicast: return launch_cfg<kStDirect>(cfg, a);
+        case Store::Peers: return launch_cfg<kStPeers>(cfg, a);
+        case Store::Push: return launch_cfg<kStTma>(cfg, a);      // store-ring epilogue, 1..8 destinations
+        case Store::Local: break;
+    }
+    if (!forced) {                            // few tiles and a long K -> several CTAs per tile
         const int split = pick_split_k(a);
         if (split == 4) return launch_splitk<4>(a);
         if (split == 2) return launch_splitk<2>(a);
     }
-    // Pushing to peers the kernel is bound by NVLink, not by the tensor pipe, and the link idles until the first tiles
-    // are complete: narrower tiles (256 x 128) halve that ramp at no cost in exchange time (measured at w = 2:
-    // 103.4 us against 106.4 us with 256 x 256 tiles; profiles/r2_scaling.md).
-    if (!forced && mode == 3 && (a.store_mc >> 8) > 1 && (cfg == 3 || cfg == 5)) cfg = 4;
-    if (mode == 2) {          // peer stores with st.global (round-1 plan): the CTA-pair configurations only
-        if ((a.store_mc >> 8) < 2 || (a.store_mc >> 8) > 8 || !a.ws) return FP8B_ERR_INVALID;
-        switch (cfg) {
-            case 3: return launch_tcgen05_cfg<256, 2, kStPeers>(a);
-            case 4: return launch_tcgen05_cfg<128, 2, kStPeers>(a);
-            case 5: return launch_tcgen05_cfg<192, 2, kStPeers>(a);
-            default: return FP8B_ERR_UNSUPPORTED;
-        }
+    // TMA-store epilogue to the one output, else the st.global epilogue (same bits)
+    if (tune(kTuneGemmStore, kDefaultGemmStore) == 2 && tma_store_ok(a, &a.C, 1) && tile_whole_boxes(cfg, a.out_dtype)) {
+        MMArgs t = a;
+        t.store = Store::Push; t.n_dst = 1; t.dsts = &a.C;
+        return launch_cfg<kStTma>(cfg, t);
     }
-    if (mode == 3) {          // store-ring epilogue, 1..8 destinations
-        switch (cfg) {
-            case 1: return launch_tcgen05_cfg<256, 1, kStTma>(a);
-            case 3: return launch_tcgen05_cfg<256, 2, kStTma>(a);
-            case 4: return launch_tcgen05_cfg<128, 2, kStTma>(a);
-            case 5: return launch_tcgen05_cfg<192, 2, kStTma>(a);
-            default: return launch_tcgen05_cfg<128, 1, kStTma>(a);
-        }
-    }
-    if (mode == 0 && tune(kTuneGemmStore, kDefaultGemmStore) == 2) {      // plain call, TMA-store epilogue to the one output
-        void* self[1] = {a.C};
-        if (tma_store_ok(a, self, 1) && tile_whole_boxes(cfg, a.out_dtype)) {      // else the st.global epilogue (same bits)
-            MMArgs t = a;
-            t.store_mc = 3 | (1 << 8);
-            t.ws = nullptr;
-            switch (cfg) {
-                case 1: return launch_tcgen05_cfg<256, 1, kStTma>(t);
-                case 3: return launch_tcgen05_cfg<256, 2, kStTma>(t);
-                case 4: return launch_tcgen05_cfg<128, 2, kStTma>(t);
-                case 5: return launch_tcgen05_cfg<192, 2, kStTma>(t);
-                default: return launch_tcgen05_cfg<128, 1, kStTma>(t);
-            }
-        }
-    }
-    switch (cfg) {
-        case 1: return launch_tcgen05_cfg<256, 1>(a);
-        case 3: return launch_tcgen05_cfg<256, 2>(a);
-        case 4: return launch_tcgen05_cfg<128, 2>(a);
-        case 5: return launch_tcgen05_cfg<192, 2>(a);
-        default: return launch_tcgen05_cfg<128, 1>(a);
-    }
+    return launch_cfg<kStDirect>(cfg, a);
 }
 
 }  // namespace fp8b

@@ -15,6 +15,14 @@ struct PushSignal {
     uint64_t epoch;
 };
 
+// Where the tcgen05 GEMM stores the tile; every other kernel stores to C only (Local).
+enum class Store {
+    Local,        // C
+    Multicast,    // C is an NVSwitch multicast address (multimem.st)
+    Peers,        // C and, at C + peer_deltas[r], every rank's buffer (st.global)
+    Push          // TMA stores to the n_dst buffers dsts[]
+};
+
 struct MMArgs {
     const uint8_t* A;      // (M,K) row-major
     const uint8_t* B;      // (N,K) row-major
@@ -26,10 +34,12 @@ struct MMArgs {
     const float* sb; int sb_len;
     const void* bias; int bias_dtype;
     const float* sr;
-    void* ws; size_t ws_bytes;
-    int store_mc;          // tcgen05 kernel only: C is a multicast address (multimem.st)
     cudaStream_t st;
     int a_fmt = 0, b_fmt = 0;   // operand formats (FP8B_E4M3FN / FP8B_E5M2); host-side routing only
+    Store store = Store::Local;
+    int n_dst = 1;                          // Peers: world size; Push: number of destinations
+    const int64_t* peer_deltas = nullptr;   // Peers: DEVICE table of n_dst byte offsets from C (0 for this rank)
+    void* const* dsts = nullptr;            // Push: HOST array of n_dst destination buffers
     const PushSignal* sig = nullptr;   // push kernel only
     int chain_pdl = 0;     // GEMV only: the predecessor on the stream is our own quantise kernel (never writes B),
                            // so launch with PDL and prefetch B before griddepcontrol.wait
