@@ -60,9 +60,103 @@ void* current_stream() { return static_cast<void*>(at::cuda::getCurrentCUDAStrea
 
 const uint8_t* u8_ptr(const torch::Tensor& t) { return static_cast<const uint8_t*>(t.data_ptr()); }
 
-torch::Tensor as_device_f32(const torch::Tensor& t, const torch::Device& dev)
+// ---- argument preparation shared by the bindings ----------------------------------------------
+// Each rule below exists once; the bindings only name which ones apply to them.
+
+// A float tensor as the kernels read it: contiguous, float32/float16/bfloat16 as they are, anything else widened to
+// float32 (fp8_mps_native.py:142).  Inputs of the casts and biases of the matmuls follow the same rule.
+torch::Tensor float_input(const torch::Tensor& t)
 {
-    return t.to(dev, torch::kFloat32).contiguous().reshape({-1});
+    torch::Tensor in = t.contiguous();
+    const auto st = in.scalar_type();
+    return (st == at::kFloat || st == at::kHalf || st == at::kBFloat16) ? in : in.to(torch::kFloat32);
+}
+
+// FP8-encoded matmul operand: uint8, on the GPU, row-major.
+void check_fp8_operand(const torch::Tensor& t, const char* name)
+{
+    TORCH_CHECK(t.dtype() == torch::kUInt8, name, " must be uint8 (FP8 encoded)");
+    TORCH_CHECK(t.is_cuda(), name, " must be a CUDA tensor");
+    TORCH_CHECK(t.is_contiguous(), name, " must be contiguous");
+}
+
+// A (M,K) and B (N,K) of one matmul.
+void check_fp8_pair(const torch::Tensor& A, const torch::Tensor& B)
+{
+    check_fp8_operand(A, "A");
+    check_fp8_operand(B, "B");
+    TORCH_CHECK(A.dim() == 2 && B.dim() == 2, "A must be (M,K) and B must be (N,K)");
+    TORCH_CHECK(B.size(1) == A.size(1), "K dimension mismatch between A and B");
+    TORCH_CHECK(A.device() == B.device(), "A and B must be on the same device");
+    TORCH_CHECK(A.size(0) < (1LL << 31) && B.size(0) < (1LL << 31) && A.size(1) < (1LL << 31), "extent too large");
+}
+
+struct Scale {
+    torch::Tensor keep;                 // holds a converted scale alive until the call
+    const float* ptr = nullptr;
+    int len = 0;
+};
+
+// A scale as a float32 device pointer of 1 or n elements (`msg` when it has neither).  A tensor that already is one is
+// used as it is, any other is converted; None is the default scale 1.0 (fp8_mps_patch.py:87-90), one cached tensor per
+// device instead of an allocation and a fill kernel on every call.
+Scale scale_arg(const c10::optional<torch::Tensor>& s, const torch::Device& dev, int64_t n, const char* msg)
+{
+    Scale r;
+    if (!s.has_value() || !s->defined()) {
+        static std::mutex mu;
+        static torch::Tensor ones[64];
+        const int idx = dev.has_index() ? dev.index() : 0;
+        std::lock_guard<std::mutex> lock(mu);
+        if (idx < 0 || idx >= 64) r.keep = torch::ones({1}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
+        else {
+            if (!ones[idx].defined()) ones[idx] = torch::ones({1}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
+            r.keep = ones[idx];
+        }
+    } else if (s->device() == dev && s->scalar_type() == at::kFloat && s->is_contiguous()) {
+        r.keep = *s;
+    } else {
+        r.keep = s->to(dev, torch::kFloat32).contiguous();
+    }
+    const int64_t len = r.keep.numel();
+    TORCH_CHECK(len == 1 || len == n, msg);
+    r.ptr = r.keep.data_ptr<float>();
+    r.len = (int)len;
+    return r;
+}
+
+// scale_result: nullptr when absent, else one element.
+Scale scale_result_arg(const c10::optional<torch::Tensor>& s, const torch::Device& dev)
+{
+    if (!s.has_value() || !s->defined()) return Scale();
+    return scale_arg(s, dev, 1, "scale_result must have 1 element");
+}
+
+struct Bias {
+    torch::Tensor keep;
+    const void* ptr = nullptr;
+    int dtype = FP8B_F32;
+};
+
+// An N-element bias on `dev` as (pointer, FP8B dtype); none when undefined.  A contiguous tensor on `dev` in a bias
+// dtype is passed as it is.
+Bias bias_arg(const c10::optional<torch::Tensor>& bias, const torch::Device& dev, int64_t N)
+{
+    Bias r;
+    if (!bias.has_value() || !bias->defined()) return r;
+    r.keep = float_input(bias->device() == dev ? *bias : bias->to(dev));
+    TORCH_CHECK(r.keep.numel() == N, "bias must have N elements");
+    r.ptr = r.keep.data_ptr();
+    r.dtype = to_fp8b_dtype(r.keep.scalar_type());
+    return r;
+}
+
+// Exchange bindings: the N-column block at n0 of a row-major (M, full_N) buffer at `base` must lie inside it; returns
+// the address of its first element.
+void* column_block(uintptr_t base, int64_t n0, int64_t N, int64_t full_N, size_t elem_size)
+{
+    TORCH_CHECK(n0 >= 0 && n0 + N <= full_N, "column block outside the full matrix");
+    return reinterpret_cast<void*>(base + static_cast<uintptr_t>(n0) * elem_size);
 }
 
 // ---- fused scaled matmul: everything torch._scaled_mm can ask for, in one kernel -------------
@@ -71,66 +165,34 @@ torch::Tensor fp8_scaled_mm_fused(torch::Tensor A, torch::Tensor B, torch::Tenso
                                   c10::optional<at::ScalarType> out_dtype, int64_t algo,
                                   c10::optional<torch::Tensor> out, int64_t a_format, int64_t b_format)
 {
-    TORCH_CHECK(A.dtype() == torch::kUInt8, "A must be uint8 (FP8 encoded)");
-    TORCH_CHECK(B.dtype() == torch::kUInt8, "B must be uint8 (FP8 encoded)");
-    TORCH_CHECK(A.is_cuda() && B.is_cuda(), "A and B must be CUDA tensors");
-    TORCH_CHECK(A.dim() == 2 && B.dim() == 2, "A must be (M,K) and B must be (N,K)");
-    TORCH_CHECK(A.is_contiguous(), "A must be contiguous");
-    TORCH_CHECK(B.is_contiguous(), "B must be contiguous");
-    TORCH_CHECK(B.size(1) == A.size(1), "K dimension mismatch between A and B");
-    TORCH_CHECK(A.device() == B.device(), "A and B must be on the same device");
+    check_fp8_pair(A, B);
     const int64_t M = A.size(0), K = A.size(1), N = B.size(0);
-    TORCH_CHECK(M < (1LL << 31) && N < (1LL << 31) && K < (1LL << 31), "extent too large");
-
-    c10::cuda::CUDAGuard guard(A.device());
-    torch::Tensor sa = as_device_f32(scale_a, A.device());
-    torch::Tensor sb = as_device_f32(scale_b, A.device());
-    TORCH_CHECK(sa.numel() == 1 || sa.numel() == M, "scale_a must have 1 or M elements");
-    TORCH_CHECK(sb.numel() == 1 || sb.numel() == N, "scale_b must have 1 or N elements");
+    const auto dev = A.device();
+    c10::cuda::CUDAGuard guard(dev);
+    const Scale sa = scale_arg(scale_a, dev, M, "scale_a must have 1 or M elements");
+    const Scale sb = scale_arg(scale_b, dev, N, "scale_b must have 1 or N elements");
 
     const at::ScalarType odt = out_dtype.value_or(at::kFloat);          // out_dtype=None -> fp32 (fp8_mps_patch.py:103)
     torch::Tensor C;
     int64_t ldc = N;
     if (out.has_value()) {
         C = *out;
-        TORCH_CHECK(C.is_cuda() && C.device() == A.device() && C.dim() == 2 && C.size(0) == M && C.size(1) == N,
+        TORCH_CHECK(C.is_cuda() && C.device() == dev && C.dim() == 2 && C.size(0) == M && C.size(1) == N,
                     "out must be a (M,N) CUDA tensor on A's device");
         TORCH_CHECK(C.scalar_type() == odt, "out dtype mismatch");
         TORCH_CHECK(C.stride(1) == 1 && C.stride(0) >= N, "out must be row-major with unit column stride");
         ldc = C.stride(0);
     } else {
-        C = torch::empty({M, N}, torch::TensorOptions().dtype(odt).device(A.device()));
+        C = torch::empty({M, N}, torch::TensorOptions().dtype(odt).device(dev));
     }
-
-    torch::Tensor bias_t, sr_t;
-    const void* bias_ptr = nullptr;
-    int bias_dt = FP8B_F32;
-    if (bias.has_value() && bias->defined()) {
-        bias_t = bias->to(A.device()).contiguous().reshape({-1});
-        if (bias_t.scalar_type() != at::kFloat && bias_t.scalar_type() != at::kHalf && bias_t.scalar_type() != at::kBFloat16)
-            bias_t = bias_t.to(torch::kFloat32);
-        TORCH_CHECK(bias_t.numel() == N, "bias must have N elements");
-        bias_ptr = bias_t.data_ptr();
-        bias_dt = to_fp8b_dtype(bias_t.scalar_type());
-    }
-    const float* sr_ptr = nullptr;
-    if (scale_result.has_value() && scale_result->defined()) {
-        sr_t = as_device_f32(*scale_result, A.device());
-        TORCH_CHECK(sr_t.numel() == 1, "scale_result must have 1 element");
-        sr_ptr = sr_t.data_ptr<float>();
-    }
+    const Bias b = bias_arg(bias, dev, N);
+    const Scale sr = scale_result_arg(scale_result, dev);
 
     if (M == 0 || N == 0) return C;
-    int rc;
-    if (a_format != FP8B_E4M3FN || b_format != FP8B_E4M3FN)
-        rc = fp8b_scaled_mm_fmt(u8_ptr(A), (int)a_format, u8_ptr(B), (int)b_format, C.data_ptr(), to_fp8b_out_dtype(odt),
-                                (int)M, (int)N, (int)K, ldc, sa.data_ptr<float>(), (int)sa.numel(), sb.data_ptr<float>(),
-                                (int)sb.numel(), bias_ptr, bias_dt, sr_ptr, (int)algo, current_stream());
-    else
-        rc = fp8b_scaled_mm(u8_ptr(A), u8_ptr(B), C.data_ptr(), to_fp8b_out_dtype(odt), (int)M, (int)N, (int)K, ldc,
-                                sa.data_ptr<float>(), (int)sa.numel(), sb.data_ptr<float>(), (int)sb.numel(),
-                                bias_ptr, bias_dt, sr_ptr, nullptr, 0, (int)algo, current_stream());
-    check_status(rc, "fp8b_scaled_mm");
+    check_status(fp8b_scaled_mm_fmt(u8_ptr(A), (int)a_format, u8_ptr(B), (int)b_format, C.data_ptr(), to_fp8b_out_dtype(odt),
+                                    (int)M, (int)N, (int)K, ldc, sa.ptr, sa.len, sb.ptr, sb.len, b.ptr, b.dtype, sr.ptr,
+                                    (int)algo, current_stream()),
+                 "fp8b_scaled_mm");
     return C;
 }
 
@@ -139,8 +201,6 @@ torch::Tensor fp8_scaled_mm_fused(torch::Tensor A, torch::Tensor B, torch::Tenso
 // separate Python-level tensor ops (~6 us of host time per call, more than a decode GEMV's kernel time); this does
 // the same on raw strides and pointers.  input: (M,K) uint8 / float8_e4m3fn / float8_e5m2; other: (K,N), normally
 // column-major so that its memory IS the (N,K) row-major weight (fp8_mps_patch.py:82-84).
-namespace {
-
 int format_of(const torch::Tensor& t)
 {
     return t.scalar_type() == at::kFloat8_e5m2 ? FP8B_E5M2 : FP8B_E4M3FN;     // uint8 is taken as e4m3fn (reference)
@@ -151,32 +211,6 @@ bool is_fp8_like(const torch::Tensor& t)
     const auto st = t.scalar_type();
     return st == at::kByte || st == at::kFloat8_e4m3fn || st == at::kFloat8_e5m2;
 }
-
-// float32 device pointer for a scale tensor without touching it when it already is one
-const float* scale_ptr(const c10::optional<torch::Tensor>& s, const torch::Device& dev, torch::Tensor& keep, int64_t& len)
-{
-    if (!s.has_value() || !s->defined()) {
-        // default scale 1.0 (fp8_mps_patch.py:87-90): one cached tensor per device instead of an allocation and a fill
-        // kernel on every call
-        static std::mutex mu;
-        static torch::Tensor ones[64];
-        const int idx = dev.has_index() ? dev.index() : 0;
-        std::lock_guard<std::mutex> lock(mu);
-        if (idx < 0 || idx >= 64) keep = torch::ones({1}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
-        else {
-            if (!ones[idx].defined()) ones[idx] = torch::ones({1}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
-            keep = ones[idx];
-        }
-    } else if (s->device() == dev && s->scalar_type() == at::kFloat && s->is_contiguous()) {
-        keep = *s;
-    } else {
-        keep = as_device_f32(*s, dev);
-    }
-    len = keep.numel();
-    return keep.data_ptr<float>();
-}
-
-}  // namespace
 
 torch::Tensor scaled_mm_patch(torch::Tensor input, torch::Tensor other, c10::optional<torch::Tensor> scale_a,
                               c10::optional<torch::Tensor> scale_b, c10::optional<torch::Tensor> bias,
@@ -194,36 +228,17 @@ torch::Tensor scaled_mm_patch(torch::Tensor input, torch::Tensor other, c10::opt
     // (N,K) row-major view of `other`: free when other is column-major, one copy otherwise (fp8_mps_patch.py:84)
     torch::Tensor b = (other.stride(0) == 1 && (other.stride(1) == K || N == 1)) ? other : other.t().contiguous();
 
-    torch::Tensor sa_t, sb_t, sr_t, bias_t;
-    int64_t sa_len = 0, sb_len = 0;
-    const float* sa = scale_ptr(scale_a, dev, sa_t, sa_len);
-    const float* sb = scale_ptr(scale_b, dev, sb_t, sb_len);
-    TORCH_CHECK(sa_len == 1 || sa_len == M, "scale_a must have 1 or M elements");
-    TORCH_CHECK(sb_len == 1 || sb_len == N, "scale_b must have 1 or N elements");
-    const void* bias_ptr = nullptr;
-    int bias_dt = FP8B_F32;
-    if (bias.has_value() && bias->defined()) {
-        bias_t = (bias->device() == dev && bias->is_contiguous()) ? *bias : bias->to(dev).contiguous();
-        if (bias_t.scalar_type() != at::kFloat && bias_t.scalar_type() != at::kHalf && bias_t.scalar_type() != at::kBFloat16)
-            bias_t = bias_t.to(torch::kFloat32);
-        TORCH_CHECK(bias_t.numel() == N, "bias must have N elements");
-        bias_ptr = bias_t.data_ptr();
-        bias_dt = to_fp8b_dtype(bias_t.scalar_type());
-    }
-    const float* sr = nullptr;
-    if (scale_result.has_value() && scale_result->defined()) {
-        int64_t sr_len = 0;
-        sr = scale_ptr(scale_result, dev, sr_t, sr_len);
-        TORCH_CHECK(sr_len == 1, "scale_result must have 1 element");
-    }
+    const Scale sa = scale_arg(scale_a, dev, M, "scale_a must have 1 or M elements");
+    const Scale sb = scale_arg(scale_b, dev, N, "scale_b must have 1 or N elements");
+    const Bias bi = bias_arg(bias, dev, N);
+    const Scale sr = scale_result_arg(scale_result, dev);
     const at::ScalarType odt = out_dtype.value_or(at::kFloat);          // out_dtype=None -> fp32 (fp8_mps_patch.py:103)
     torch::Tensor C = torch::empty({M, N}, torch::TensorOptions().dtype(odt).device(dev));
     if (M == 0 || N == 0) return C;
-    const int rc = fp8b_scaled_mm_fmt(static_cast<const uint8_t*>(a.data_ptr()), format_of(input),
-                                      static_cast<const uint8_t*>(b.data_ptr()), format_of(other), C.data_ptr(),
-                                      to_fp8b_out_dtype(odt), (int)M, (int)N, (int)K, N, sa, (int)sa_len, sb, (int)sb_len,
-                                      bias_ptr, bias_dt, sr, FP8B_MM_AUTO, current_stream());
-    check_status(rc, "fp8b_scaled_mm");
+    check_status(fp8b_scaled_mm_fmt(u8_ptr(a), format_of(input), u8_ptr(b), format_of(other), C.data_ptr(),
+                                    to_fp8b_out_dtype(odt), (int)M, (int)N, (int)K, N, sa.ptr, sa.len, sb.ptr, sb.len,
+                                    bi.ptr, bi.dtype, sr.ptr, FP8B_MM_AUTO, current_stream()),
+                 "fp8b_scaled_mm");
     return C;
 }
 
@@ -240,10 +255,9 @@ torch::Tensor fp8_dequantize(torch::Tensor input, torch::Tensor scale)
     TORCH_CHECK(input.is_cuda(), "input must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(input.device());
     torch::Tensor in = input.contiguous();
-    torch::Tensor sc = as_device_f32(scale, input.device());
-    TORCH_CHECK(sc.numel() == 1, "scale must be a scalar tensor");
+    const Scale sc = scale_arg(scale, input.device(), 1, "scale must be a scalar tensor");
     torch::Tensor out = torch::empty(in.sizes(), torch::TensorOptions().dtype(torch::kFloat16).device(in.device()));
-    check_status(fp8b_dequant_f16(u8_ptr(in), out.data_ptr(), (size_t)in.numel(), sc.data_ptr<float>(), current_stream()),
+    check_status(fp8b_dequant_f16(u8_ptr(in), out.data_ptr(), (size_t)in.numel(), sc.ptr, current_stream()),
                  "fp8b_dequant_f16");
     return out;
 }
@@ -267,9 +281,7 @@ torch::Tensor fp8_encode(torch::Tensor input)
 {
     TORCH_CHECK(input.is_cuda(), "input must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(input.device());
-    torch::Tensor in = input.contiguous();
-    if (in.scalar_type() != at::kFloat && in.scalar_type() != at::kHalf && in.scalar_type() != at::kBFloat16)
-        in = in.to(torch::kFloat32);                                   // fp8_mps_native.py:142
+    torch::Tensor in = float_input(input);
     torch::Tensor out = torch::empty(in.sizes(), torch::TensorOptions().dtype(torch::kUInt8).device(in.device()));
     check_status(fp8b_encode(in.data_ptr(), to_fp8b_dtype(in.scalar_type()), static_cast<uint8_t*>(out.data_ptr()),
                              (size_t)in.numel(), nullptr, current_stream()),
@@ -287,11 +299,8 @@ std::vector<torch::Tensor> fp8_encode_many(std::vector<torch::Tensor> inputs)
     c10::cuda::CUDAGuard guard(dev);
     for (size_t i = 0; i < inputs.size(); ++i) {
         TORCH_CHECK(inputs[i].device() == dev, "all inputs must be on one device");
-        torch::Tensor in = inputs[i].contiguous();
-        if (in.scalar_type() != at::kFloat && in.scalar_type() != at::kHalf && in.scalar_type() != at::kBFloat16)
-            in = in.to(torch::kFloat32);
-        ins[i] = in;
-        outs[i] = torch::empty(in.sizes(), torch::TensorOptions().dtype(torch::kUInt8).device(dev));
+        ins[i] = float_input(inputs[i]);
+        outs[i] = torch::empty(ins[i].sizes(), torch::TensorOptions().dtype(torch::kUInt8).device(dev));
     }
     for (at::ScalarType dt : {at::kFloat, at::kHalf, at::kBFloat16}) {
         std::vector<fp8b_span> spans;
@@ -328,9 +337,7 @@ std::tuple<torch::Tensor, torch::Tensor> fp8_quantize(torch::Tensor input)
 {
     TORCH_CHECK(input.is_cuda(), "input must be a CUDA tensor");
     c10::cuda::CUDAGuard guard(input.device());
-    torch::Tensor in = input.contiguous();
-    if (in.scalar_type() != at::kFloat && in.scalar_type() != at::kHalf && in.scalar_type() != at::kBFloat16)
-        in = in.to(torch::kFloat32);
+    torch::Tensor in = float_input(input);
     auto f32 = torch::TensorOptions().dtype(torch::kFloat32).device(in.device());
     torch::Tensor scales = torch::empty({2}, f32);                    // [scale, inv_scale]
     torch::Tensor scratch = torch::empty({1}, torch::TensorOptions().dtype(torch::kInt32).device(in.device()));
@@ -353,32 +360,18 @@ void fp8_scaled_mm_multicast(torch::Tensor A, torch::Tensor B, torch::Tensor sca
                              c10::optional<torch::Tensor> bias, at::ScalarType out_dtype,
                              int64_t mc_ptr, int64_t full_N, int64_t n0)
 {
-    TORCH_CHECK(A.dtype() == torch::kUInt8 && B.dtype() == torch::kUInt8, "A and B must be uint8 (FP8 encoded)");
-    TORCH_CHECK(A.is_cuda() && B.is_cuda() && A.is_contiguous() && B.is_contiguous(), "A, B must be contiguous CUDA tensors");
-    TORCH_CHECK(A.dim() == 2 && B.dim() == 2 && A.size(1) == B.size(1), "K dimension mismatch between A and B");
+    check_fp8_pair(A, B);
     const int64_t M = A.size(0), K = A.size(1), N = B.size(0);
-    TORCH_CHECK(n0 >= 0 && n0 + N <= full_N, "column block outside the full matrix");
-    c10::cuda::CUDAGuard guard(A.device());
-    torch::Tensor sa = as_device_f32(scale_a, A.device());
-    torch::Tensor sb = as_device_f32(scale_b, A.device());
-    torch::Tensor bias_t;
-    const void* bias_ptr = nullptr;
-    int bias_dt = FP8B_F32;
-    if (bias.has_value() && bias->defined()) {
-        bias_t = bias->to(A.device()).contiguous().reshape({-1});
-        if (bias_t.scalar_type() != at::kFloat && bias_t.scalar_type() != at::kHalf && bias_t.scalar_type() != at::kBFloat16)
-            bias_t = bias_t.to(torch::kFloat32);
-        TORCH_CHECK(bias_t.numel() == N, "bias must have N elements");
-        bias_ptr = bias_t.data_ptr();
-        bias_dt = to_fp8b_dtype(bias_t.scalar_type());
-    }
-    const int odt = to_fp8b_dtype(out_dtype);
-    const int64_t esz = odt == FP8B_F32 ? 4 : 2;
-    void* c_mc = reinterpret_cast<void*>(static_cast<uintptr_t>(mc_ptr) + static_cast<uintptr_t>(n0 * esz));
-    int rc = fp8b_scaled_mm_multicast(u8_ptr(A), u8_ptr(B), c_mc, odt, (int)M, (int)N, (int)K, full_N,
-                                      sa.data_ptr<float>(), (int)sa.numel(), sb.data_ptr<float>(), (int)sb.numel(),
-                                      bias_ptr, bias_dt, nullptr, current_stream());
-    check_status(rc, "fp8b_scaled_mm_multicast");
+    const int odt = to_fp8b_dtype(out_dtype);                 // no float8_e4m3fn output through the multicast mapping
+    void* c_mc = column_block(static_cast<uintptr_t>(mc_ptr), n0, N, full_N, c10::elementSize(out_dtype));
+    const auto dev = A.device();
+    c10::cuda::CUDAGuard guard(dev);
+    const Scale sa = scale_arg(scale_a, dev, M, "scale_a must have 1 or M elements");
+    const Scale sb = scale_arg(scale_b, dev, N, "scale_b must have 1 or N elements");
+    const Bias b = bias_arg(bias, dev, N);
+    check_status(fp8b_scaled_mm_multicast(u8_ptr(A), u8_ptr(B), c_mc, odt, (int)M, (int)N, (int)K, full_N, sa.ptr, sa.len,
+                                          sb.ptr, sb.len, b.ptr, b.dtype, nullptr, current_stream()),
+                 "fp8b_scaled_mm_multicast");
 }
 
 // Several independent M = 1 GEMVs (same K, same out dtype) in one launch: fp8b_gemv_batch.
@@ -404,31 +397,26 @@ std::vector<torch::Tensor> fp8_scaled_mm_many(std::vector<torch::Tensor> xs, std
     for (size_t i = 0; i < n; ++i) {
         const torch::Tensor& x = xs[i];
         const torch::Tensor& W = Ws[i];
-        TORCH_CHECK(x.dtype() == torch::kUInt8 && W.dtype() == torch::kUInt8, "x and W must be uint8 (FP8 encoded)");
+        check_fp8_operand(x, "x");
+        check_fp8_operand(W, "W");
         TORCH_CHECK(x.device() == dev && W.device() == dev, "all operands must be on one device");
-        TORCH_CHECK(x.is_contiguous() && W.is_contiguous(), "x and W must be contiguous");
         TORCH_CHECK(W.dim() == 2 && W.size(1) == K && x.numel() == K, "every problem must have M = 1 and the same K");
         const int64_t N = W.size(0);
-        torch::Tensor sx = as_device_f32(scale_xs[i], dev), sw = as_device_f32(scale_ws[i], dev);
-        TORCH_CHECK(sx.numel() == 1, "scale_x must have 1 element");
-        TORCH_CHECK(sw.numel() == 1 || sw.numel() == N, "scale_w must have 1 or N elements");
-        keep.push_back(sx); keep.push_back(sw);
+        const Scale sx = scale_arg(scale_xs[i], dev, 1, "scale_x must have 1 element");
+        const Scale sw = scale_arg(scale_ws[i], dev, N, "scale_w must have 1 or N elements");
+        // fp8_mps_native passes an empty tensor for a problem without bias
+        const bool has_bias = biases.has_value() && (*biases)[i].defined() && (*biases)[i].numel() > 0;
+        const Bias b = bias_arg(has_bias ? c10::optional<torch::Tensor>((*biases)[i]) : c10::nullopt, dev, N);
+        if (b.ptr) {
+            TORCH_CHECK(!bias_seen || b.dtype == bias_dt, "all biases must share one dtype");
+            bias_dt = b.dtype; bias_seen = true;
+        }
+        keep.insert(keep.end(), {sx.keep, sw.keep, b.keep});
         outs[i] = torch::empty({1, N}, torch::TensorOptions().dtype(odt).device(dev));
         fp8b_gemv_item& q = items[i];
         q.x = u8_ptr(x); q.W = u8_ptr(W); q.y = outs[i].data_ptr(); q.N = (int)N;
-        q.scale_x = sx.data_ptr<float>(); q.scale_w = sw.data_ptr<float>(); q.scale_w_len = (int)sw.numel();
-        q.bias = nullptr;
-        if (biases.has_value() && (*biases)[i].defined() && (*biases)[i].numel() > 0) {
-            torch::Tensor bt = (*biases)[i].to(dev).contiguous().reshape({-1});
-            if (bt.scalar_type() != at::kFloat && bt.scalar_type() != at::kHalf && bt.scalar_type() != at::kBFloat16)
-                bt = bt.to(torch::kFloat32);
-            TORCH_CHECK(bt.numel() == N, "bias must have N elements");
-            const int dt = to_fp8b_dtype(bt.scalar_type());
-            TORCH_CHECK(!bias_seen || dt == bias_dt, "all biases must share one dtype");
-            bias_dt = dt; bias_seen = true;
-            keep.push_back(bt);
-            q.bias = bt.data_ptr();
-        }
+        q.scale_x = sx.ptr; q.scale_w = sw.ptr; q.scale_w_len = sw.len;
+        q.bias = b.ptr;
     }
     check_status(fp8b_gemv_batch(items.data(), (int)n, (int)K, to_fp8b_out_dtype(odt), bias_dt, current_stream()), "fp8b_gemv_batch");
     return outs;
@@ -439,34 +427,21 @@ std::vector<torch::Tensor> fp8_scaled_mm_many(std::vector<torch::Tensor> xs, std
 void fp8_scaled_mm_peers(torch::Tensor A, torch::Tensor B, torch::Tensor scale_a, torch::Tensor scale_b,
                          c10::optional<torch::Tensor> bias, torch::Tensor out, torch::Tensor peer_deltas, int64_t n0)
 {
-    TORCH_CHECK(A.dtype() == torch::kUInt8 && B.dtype() == torch::kUInt8, "A and B must be uint8 (FP8 encoded)");
-    TORCH_CHECK(A.is_cuda() && B.is_cuda() && A.is_contiguous() && B.is_contiguous(), "A, B must be contiguous CUDA tensors");
-    TORCH_CHECK(A.dim() == 2 && B.dim() == 2 && A.size(1) == B.size(1), "K dimension mismatch between A and B");
+    check_fp8_pair(A, B);
     TORCH_CHECK(out.is_cuda() && out.dim() == 2 && out.is_contiguous() && out.size(0) == A.size(0), "out must be (M, full_N) contiguous");
     TORCH_CHECK(peer_deltas.is_cuda() && peer_deltas.scalar_type() == at::kLong && peer_deltas.is_contiguous(),
                 "peer_deltas must be a contiguous CUDA int64 tensor");
     const int64_t M = A.size(0), K = A.size(1), N = B.size(0), full_N = out.size(1);
-    TORCH_CHECK(n0 >= 0 && n0 + N <= full_N, "column block outside the full matrix");
-    c10::cuda::CUDAGuard guard(A.device());
-    torch::Tensor sa = as_device_f32(scale_a, A.device());
-    torch::Tensor sb = as_device_f32(scale_b, A.device());
-    torch::Tensor bias_t;
-    const void* bias_ptr = nullptr;
-    int bias_dt = FP8B_F32;
-    if (bias.has_value() && bias->defined()) {
-        bias_t = bias->to(A.device()).contiguous().reshape({-1});
-        if (bias_t.scalar_type() != at::kFloat && bias_t.scalar_type() != at::kHalf && bias_t.scalar_type() != at::kBFloat16)
-            bias_t = bias_t.to(torch::kFloat32);
-        TORCH_CHECK(bias_t.numel() == N, "bias must have N elements");
-        bias_ptr = bias_t.data_ptr();
-        bias_dt = to_fp8b_dtype(bias_t.scalar_type());
-    }
-    const int odt = to_fp8b_out_dtype(out.scalar_type());
-    void* c_local = static_cast<uint8_t*>(out.data_ptr()) + n0 * out.element_size();
-    int rc = fp8b_scaled_mm_peers(u8_ptr(A), u8_ptr(B), c_local, peer_deltas.data_ptr<int64_t>(), (int)peer_deltas.numel(), odt,
-                                  (int)M, (int)N, (int)K, full_N, sa.data_ptr<float>(), (int)sa.numel(),
-                                  sb.data_ptr<float>(), (int)sb.numel(), bias_ptr, bias_dt, nullptr, current_stream());
-    check_status(rc, "fp8b_scaled_mm_peers");
+    void* c_local = column_block(reinterpret_cast<uintptr_t>(out.data_ptr()), n0, N, full_N, out.element_size());
+    const auto dev = A.device();
+    c10::cuda::CUDAGuard guard(dev);
+    const Scale sa = scale_arg(scale_a, dev, M, "scale_a must have 1 or M elements");
+    const Scale sb = scale_arg(scale_b, dev, N, "scale_b must have 1 or N elements");
+    const Bias b = bias_arg(bias, dev, N);
+    check_status(fp8b_scaled_mm_peers(u8_ptr(A), u8_ptr(B), c_local, peer_deltas.data_ptr<int64_t>(), (int)peer_deltas.numel(),
+                                      to_fp8b_out_dtype(out.scalar_type()), (int)M, (int)N, (int)K, full_N, sa.ptr, sa.len,
+                                      sb.ptr, sb.len, b.ptr, b.dtype, nullptr, current_stream()),
+                 "fp8b_scaled_mm_peers");
 }
 
 // N-sharded linear, fused compute + exchange with TMA stores (fp8b_scaled_mm_push).  `out` is this rank's (M, full_N)
@@ -478,36 +453,23 @@ void fp8_scaled_mm_push(torch::Tensor A, torch::Tensor B, torch::Tensor scale_a,
                         std::vector<int64_t> signal_ptrs, c10::optional<torch::Tensor> cta_counter, int64_t epoch,
                         c10::optional<torch::Tensor> wait_flags, int64_t rank)
 {
-    TORCH_CHECK(A.dtype() == torch::kUInt8 && B.dtype() == torch::kUInt8, "A and B must be uint8 (FP8 encoded)");
-    TORCH_CHECK(A.is_cuda() && B.is_cuda() && A.is_contiguous() && B.is_contiguous(), "A, B must be contiguous CUDA tensors");
-    TORCH_CHECK(A.dim() == 2 && B.dim() == 2 && A.size(1) == B.size(1), "K dimension mismatch between A and B");
+    check_fp8_pair(A, B);
     TORCH_CHECK(out.is_cuda() && out.dim() == 2 && out.is_contiguous() && out.size(0) == A.size(0), "out must be (M, full_N) contiguous");
     TORCH_CHECK(!dst_ptrs.empty() && dst_ptrs.size() <= 8, "need 1..8 destination buffers");
     const int64_t M = A.size(0), K = A.size(1), N = B.size(0), full_N = out.size(1);
-    TORCH_CHECK(n0 >= 0 && n0 + N <= full_N, "column block outside the full matrix");
-    c10::cuda::CUDAGuard guard(A.device());
-    torch::Tensor sa_t, sb_t, bias_t;
-    int64_t sa_len = 0, sb_len = 0;
-    const float* sa = scale_ptr(scale_a, A.device(), sa_t, sa_len);
-    const float* sb = scale_ptr(scale_b, A.device(), sb_t, sb_len);
-    const void* bias_ptr = nullptr;
-    int bias_dt = FP8B_F32;
-    if (bias.has_value() && bias->defined()) {
-        bias_t = bias->to(A.device()).contiguous().reshape({-1});
-        if (bias_t.scalar_type() != at::kFloat && bias_t.scalar_type() != at::kHalf && bias_t.scalar_type() != at::kBFloat16)
-            bias_t = bias_t.to(torch::kFloat32);
-        TORCH_CHECK(bias_t.numel() == N, "bias must have N elements");
-        bias_ptr = bias_t.data_ptr();
-        bias_dt = to_fp8b_dtype(bias_t.scalar_type());
-    }
     void* dsts[8];
     for (size_t d = 0; d < dst_ptrs.size(); ++d)
-        dsts[d] = reinterpret_cast<uint8_t*>(static_cast<uintptr_t>(dst_ptrs[d])) + n0 * out.element_size();
+        dsts[d] = column_block(static_cast<uintptr_t>(dst_ptrs[d]), n0, N, full_N, out.element_size());
+    const auto dev = A.device();
+    c10::cuda::CUDAGuard guard(dev);
+    const Scale sa = scale_arg(scale_a, dev, M, "scale_a must have 1 or M elements");
+    const Scale sb = scale_arg(scale_b, dev, N, "scale_b must have 1 or N elements");
+    const Bias b = bias_arg(bias, dev, N);
     const int n_dst = (int)dst_ptrs.size();
     const int odt = to_fp8b_out_dtype(out.scalar_type());
     if (signal_ptrs.empty()) {
-        check_status(fp8b_scaled_mm_push(u8_ptr(A), u8_ptr(B), dsts, n_dst, odt, (int)M, (int)N, (int)K, full_N, sa, (int)sa_len,
-                                         sb, (int)sb_len, bias_ptr, bias_dt, nullptr, current_stream()),
+        check_status(fp8b_scaled_mm_push(u8_ptr(A), u8_ptr(B), dsts, n_dst, odt, (int)M, (int)N, (int)K, full_N, sa.ptr, sa.len,
+                                         sb.ptr, sb.len, b.ptr, b.dtype, nullptr, current_stream()),
                      "fp8b_scaled_mm_push");
         return;
     }
@@ -517,8 +479,8 @@ void fp8_scaled_mm_push(torch::Tensor A, torch::Tensor B, torch::Tensor scale_a,
     TORCH_CHECK(wait_flags.has_value() && wait_flags->is_cuda() && wait_flags->scalar_type() == at::kLong, "wait_flags: CUDA int64");
     uint64_t* sig[8];
     for (int d = 0; d < n_dst; ++d) sig[d] = reinterpret_cast<uint64_t*>(static_cast<uintptr_t>(signal_ptrs[d]));
-    check_status(fp8b_scaled_mm_push_signal(u8_ptr(A), u8_ptr(B), dsts, n_dst, odt, (int)M, (int)N, (int)K, full_N, sa, (int)sa_len,
-                                            sb, (int)sb_len, bias_ptr, bias_dt, nullptr, sig,
+    check_status(fp8b_scaled_mm_push_signal(u8_ptr(A), u8_ptr(B), dsts, n_dst, odt, (int)M, (int)N, (int)K, full_N, sa.ptr, sa.len,
+                                            sb.ptr, sb.len, b.ptr, b.dtype, nullptr, sig,
                                             reinterpret_cast<uint32_t*>(cta_counter->data_ptr()), (uint64_t)epoch, current_stream()),
                  "fp8b_scaled_mm_push_signal");
     check_status(fp8b_peer_wait(reinterpret_cast<const uint64_t*>(wait_flags->data_ptr()), n_dst, (int)rank, (uint64_t)epoch,
@@ -532,9 +494,7 @@ std::tuple<torch::Tensor, torch::Tensor> fp8_quantize_rowwise(torch::Tensor inpu
     TORCH_CHECK(input.is_cuda(), "input must be a CUDA tensor");
     TORCH_CHECK(input.dim() == 2, "input must be 2-D (rows, cols)");
     c10::cuda::CUDAGuard guard(input.device());
-    torch::Tensor in = input.contiguous();
-    if (in.scalar_type() != at::kFloat && in.scalar_type() != at::kHalf && in.scalar_type() != at::kBFloat16)
-        in = in.to(torch::kFloat32);
+    torch::Tensor in = float_input(input);
     torch::Tensor out = torch::empty(in.sizes(), torch::TensorOptions().dtype(torch::kUInt8).device(in.device()));
     torch::Tensor inv = torch::empty({in.size(0)}, torch::TensorOptions().dtype(torch::kFloat32).device(in.device()));
     check_status(fp8b_quantize_rows(in.data_ptr(), to_fp8b_dtype(in.scalar_type()), (int)in.size(0), (size_t)in.size(1),
@@ -549,42 +509,29 @@ std::tuple<torch::Tensor, torch::Tensor> fp8_linear_dynamic(torch::Tensor x, tor
                                                             c10::optional<torch::Tensor> bias,
                                                             c10::optional<at::ScalarType> out_dtype, bool single_kernel)
 {
-    TORCH_CHECK(B.dtype() == torch::kUInt8, "B must be uint8 (FP8 encoded)");
-    TORCH_CHECK(x.is_cuda() && B.is_cuda() && x.device() == B.device(), "x and B must be CUDA tensors on one device");
+    check_fp8_operand(B, "B");
+    TORCH_CHECK(x.is_cuda() && x.device() == B.device(), "x and B must be CUDA tensors on one device");
     TORCH_CHECK(x.dim() == 2 && B.dim() == 2 && x.size(1) == B.size(1), "K dimension mismatch between x and B");
-    TORCH_CHECK(B.is_contiguous(), "B must be contiguous");
-    c10::cuda::CUDAGuard guard(x.device());
-    torch::Tensor xin = x.contiguous();
-    if (xin.scalar_type() != at::kFloat && xin.scalar_type() != at::kHalf && xin.scalar_type() != at::kBFloat16)
-        xin = xin.to(torch::kFloat32);
+    const auto dev = x.device();
+    c10::cuda::CUDAGuard guard(dev);
+    torch::Tensor xin = float_input(x);
     const int64_t M = xin.size(0), K = xin.size(1), N = B.size(0);
-    torch::Tensor sb = as_device_f32(scale_b, x.device());
-    TORCH_CHECK(sb.numel() == 1 || sb.numel() == N, "scale_b must have 1 or N elements");
-    torch::Tensor bias_t;
-    const void* bias_ptr = nullptr;
-    int bias_dt = FP8B_F32;
-    if (bias.has_value() && bias->defined()) {
-        bias_t = bias->to(x.device()).contiguous().reshape({-1});
-        if (bias_t.scalar_type() != at::kFloat && bias_t.scalar_type() != at::kHalf && bias_t.scalar_type() != at::kBFloat16)
-            bias_t = bias_t.to(torch::kFloat32);
-        TORCH_CHECK(bias_t.numel() == N, "bias must have N elements");
-        bias_ptr = bias_t.data_ptr();
-        bias_dt = to_fp8b_dtype(bias_t.scalar_type());
-    }
+    const Scale sb = scale_arg(scale_b, dev, N, "scale_b must have 1 or N elements");
+    const Bias b = bias_arg(bias, dev, N);
     const at::ScalarType odt = out_dtype.value_or(at::kFloat);
-    torch::Tensor C = torch::empty({M, N}, torch::TensorOptions().dtype(odt).device(x.device()));
-    torch::Tensor inv = torch::empty({M}, torch::TensorOptions().dtype(torch::kFloat32).device(x.device()));
+    torch::Tensor C = torch::empty({M, N}, torch::TensorOptions().dtype(odt).device(dev));
+    torch::Tensor inv = torch::empty({M}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
     if (M == 0 || N == 0) return std::make_tuple(C, inv);
     torch::Tensor ws;
     void* ws_ptr = nullptr;
     size_t workspace_bytes = 0;
     if (!single_kernel) {
         workspace_bytes = fp8b_linear_dynamic_workspace_bytes((int)M, (int)K);
-        ws = torch::empty({(int64_t)workspace_bytes}, torch::TensorOptions().dtype(torch::kUInt8).device(x.device()));
+        ws = torch::empty({(int64_t)workspace_bytes}, torch::TensorOptions().dtype(torch::kUInt8).device(dev));
         ws_ptr = ws.data_ptr();
     }
     int rc = fp8b_linear_dynamic(xin.data_ptr(), to_fp8b_dtype(xin.scalar_type()), u8_ptr(B), C.data_ptr(), to_fp8b_out_dtype(odt),
-                               (int)M, (int)N, (int)K, N, sb.data_ptr<float>(), (int)sb.numel(), bias_ptr, bias_dt, nullptr,
+                               (int)M, (int)N, (int)K, N, sb.ptr, sb.len, b.ptr, b.dtype, nullptr,
                                inv.data_ptr<float>(), ws_ptr, workspace_bytes, current_stream());
     check_status(rc, "fp8b_linear_dynamic");
     return std::make_tuple(C, inv);
