@@ -97,22 +97,45 @@ struct Scale {
     int len = 0;
 };
 
+// The default scale 1.0 of one device: a float of its own cudaMalloc memory, written once and kept for the life of the
+// process, so that no call allocates or launches anything for it.  It is written by a blocking copy on a private stream,
+// never on the caller's stream: a first call inside a graph capture would otherwise capture the fill instead of running
+// it (every eager call before the first replay would read unwritten memory), and a first call on a busy stream would
+// let a call on another stream read the scale before the fill had run.  Relaxed capture mode lets the allocation and
+// the blocking copy run while this or another thread is capturing.
+const float* default_scale(int device)
+{
+    static std::mutex mu;
+    static float* ones[64] = {};
+    TORCH_CHECK(device >= 0 && device < 64, "fp8_metal: device ordinal out of range");
+    std::lock_guard<std::mutex> lock(mu);
+    if (ones[device]) return ones[device];
+    static const float one = 1.0f;
+    cudaStreamCaptureMode mode = cudaStreamCaptureModeRelaxed;
+    cudaThreadExchangeStreamCaptureMode(&mode);
+    float* ptr = nullptr;
+    cudaStream_t st = nullptr;
+    cudaError_t e = cudaMalloc(&ptr, sizeof(float));
+    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ptr, &one, sizeof(float), cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (st) cudaStreamDestroy(st);
+    if (e != cudaSuccess && ptr) cudaFree(ptr);
+    cudaThreadExchangeStreamCaptureMode(&mode);
+    TORCH_CHECK(e == cudaSuccess, "fp8_metal: could not set up the default scale: ", cudaGetErrorString(e));
+    ones[device] = ptr;
+    return ptr;
+}
+
 // A scale as a float32 device pointer of 1 or n elements (`msg` when it has neither).  A tensor that already is one is
-// used as it is, any other is converted; None is the default scale 1.0 (fp8_mps_patch.py:87-90), one cached tensor per
-// device instead of an allocation and a fill kernel on every call.
+// used as it is, any other is converted; None is the default scale 1.0 (fp8_mps_patch.py:87-90).
 Scale scale_arg(const c10::optional<torch::Tensor>& s, const torch::Device& dev, int64_t n, const char* msg)
 {
     Scale r;
     if (!s.has_value() || !s->defined()) {
-        static std::mutex mu;
-        static torch::Tensor ones[64];
-        const int idx = dev.has_index() ? dev.index() : 0;
-        std::lock_guard<std::mutex> lock(mu);
-        if (idx < 0 || idx >= 64) r.keep = torch::ones({1}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
-        else {
-            if (!ones[idx].defined()) ones[idx] = torch::ones({1}, torch::TensorOptions().dtype(torch::kFloat32).device(dev));
-            r.keep = ones[idx];
-        }
+        r.ptr = default_scale(dev.has_index() ? dev.index() : c10::cuda::current_device());
+        r.len = 1;
+        return r;
     } else if (s->device() == dev && s->scalar_type() == at::kFloat && s->is_contiguous()) {
         r.keep = *s;
     } else {

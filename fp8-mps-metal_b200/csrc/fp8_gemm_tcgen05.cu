@@ -1288,18 +1288,39 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+typedef CUresult (*PFN_ctxGetCurrent)(CUcontext*);
+
+static void* driver_fn(const char* name)
+{
+    void* p = nullptr;
+    cudaDriverEntryPointQueryResult qres;
+    return cudaGetDriverEntryPoint(name, &p, cudaEnableDefault, &qres) == cudaSuccess && qres == cudaDriverEntryPointSuccess ? p
+                                                                                                                             : nullptr;
+}
+
 static PFN_encodeTiled get_encode_fn()
 {
     static PFN_encodeTiled fn = nullptr;
     static std::once_flag once;
-    std::call_once(once, [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_encodeTiled>(p);
-    });
+    std::call_once(once, [] { fn = reinterpret_cast<PFN_encodeTiled>(driver_fn("cuTensorMapEncodeTiled")); });
     return fn;
+}
+
+// The encoder is a driver call and needs a current context.  A host thread whose first call into the library finds its
+// kernel attribute already set (by another thread) has made no runtime call that binds one -- cudaGetDevice does not --
+// and the encode then fails with CUDA_ERROR_INVALID_CONTEXT (seen on a B200 with six threads starting together).  A
+// thread without a current context gets the current device's primary context, as the runtime's own calls would give
+// it; a context the caller made current is left alone.
+static cudaError_t ensure_current_context()
+{
+    static PFN_ctxGetCurrent get_current = nullptr;
+    static std::once_flag once;
+    std::call_once(once, [] { get_current = reinterpret_cast<PFN_ctxGetCurrent>(driver_fn("cuCtxGetCurrent")); });
+    CUcontext ctx = nullptr;
+    if (get_current && get_current(&ctx) == CUDA_SUCCESS && ctx) return cudaSuccess;
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    return e == cudaSuccess ? cudaSetDevice(dev) : e;        // cudaSetDevice makes the primary context current
 }
 
 // A tensor map is a pure function of (base, rows, row bytes, pitch, box): a serving loop calls the same few
@@ -1328,7 +1349,8 @@ static bool get_tensor_map(CUtensorMap* out, const void* base, uint64_t rows, ui
     MapSlot& s = cache[h % kMapCacheSlots];
     if (s.valid && s.key == key) { *out = s.map; return true; }
     PFN_encodeTiled enc = get_encode_fn();
-    if (!enc) return false;
+    if (!enc) { t_last_cuda_error = (int)cudaErrorSymbolNotFound; return false; }
+    if (cudaError_t e = ensure_current_context()) { t_last_cuda_error = (int)e; return false; }
     cuuint64_t dims[2] = {(cuuint64_t)row_bytes, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)pitch};
     cuuint32_t box[2] = {(cuuint32_t)box_bytes, (cuuint32_t)box_rows};
@@ -1337,7 +1359,7 @@ static bool get_tensor_map(CUtensorMap* out, const void* base, uint64_t rows, ui
                      dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return false;
+    if (r != CUDA_SUCCESS) { t_last_cuda_error = (int)r; return false; }       // a CUresult (fp8b_last_cuda_error)
     s.key = key; s.map = *out; s.valid = true;
     return true;
 }

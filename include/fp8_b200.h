@@ -11,7 +11,11 @@
  *   - plain C: raw DEVICE pointers, extents, dtype enums, a CUDA stream handle (cudaStream_t
  *     passed as void*; NULL = legacy default stream).  No torch types.
  *   - no allocation, no host synchronisation, no ownership transfer.  The call enqueues work on
- *     `stream` and returns.  Re-entrant; thread-safe for distinct streams.
+ *     `stream` and returns.  Re-entrant and thread-safe: any host thread may call any entry point on
+ *     any stream, including its first call of the process or of the thread (a thread without a current
+ *     CUDA context is given the current device's primary context).  Every entry point may be called
+ *     while the stream is being captured into a CUDA graph, global capture mode included, first call
+ *     included; a replay runs the captured kernels only.
  *   - optional arguments are NULL pointers (absent), never sentinel values.
  *   - return value: FP8B_OK (0) or a negative fp8b_status.  There is NO silent fallback: an
  *     unsupported shape/alignment returns FP8B_ERR_UNSUPPORTED and does nothing; there is no CPU
@@ -70,7 +74,8 @@ typedef enum fp8b_mm_algo {
 
 FP8B_API int fp8b_version(void);
 FP8B_API const char* fp8b_status_string(int status);
-/* cudaError_t of the most recent failing CUDA call on this thread (0 if none). */
+/* cudaError_t of the most recent failing CUDA call on this thread, or the CUresult of a failing tensor-map encode
+ * (0 if none). */
 FP8B_API int fp8b_last_cuda_error(void);
 /* Number of kernel launches this library has enqueued since load (all threads).  bench.py
  * reads it before/after the timed region to report `gpu_launches`. */
